@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the B200 DSP hot path (contract: see the task's "Measurement" section).
 
     python bench.py --gpus N --steps K --warmup W [--workload NAME] [--tuners T] [--impl reference] [--no-extra]
+                    [--dump-outputs DIR]
 
 Headline workload (default, `c4fm_20m`) = BASELINE.json configs[4]: 20 MS/s tuners -> polyphase channelizer (M = 800)
 -> per channel 72-tap FIR -> block AGC -> DQPSK decision-directed timing recovery (P25 Phase 1 C4FM) on all 800 bins,
@@ -373,6 +374,35 @@ def dibit_match(decoded, truth, skip=300):
             best = max(best, float(np.mean(decoded[lag + skip:lag + n] == truth[skip:n])))
     return best
 
+
+def valid_prefix(buf, counts):
+    """rows of `buf` with everything past each row's count zeroed: a caller reads only the first count values, so what
+    a step leaves behind them is not part of its output"""
+    out = buf.copy()
+    out[np.arange(buf.shape[1])[None, :] >= counts[:, None]] = 0
+    return out
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """writes every array as DIR/<name>.npy in float32.  Arrays of up to 1 MB are written whole; the larger ones share
+    the rest of DUMP_LIMIT_BYTES and keep a fixed, seeded sample of their rows when they do not fit, listed in
+    DIR/<name>_rows.npy (the same rows on every run, so that the dumps of two builds compare value for value)."""
+    os.makedirs(directory, exist_ok=True)
+    small = {k for k, a in arrays.items() if a.size * 4 <= 1 << 20}
+    room = DUMP_LIMIT_BYTES - sum(arrays[k].size * 4 for k in small) - (1 << 20)   # 1 MB for row lists and headers
+    large = sum(a.size * 4 for k, a in arrays.items() if k not in small)
+    for name, a in sorted(arrays.items()):
+        if name not in small and large > room:
+            keep = max(1, int(a.shape[0] * room / large))
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))
+            np.save(os.path.join(directory, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def synth_dqpsk_channels(torch, dev, n_channels, n, seed, symbol_rate=6000.0, fs=50000.0, beta=0.35, noise=0.03):
     """SURVEY.md 8d config 4: channel-domain pi/4-DQPSK streams (raised-cosine shaped impulse train evaluated at the
     non-integer 8.33 samples per symbol), carrier offset U(-200, 200) Hz and timing phase per channel, + AWGN."""
@@ -621,6 +651,14 @@ class TunerWorkload:
             self.native.check(self.L.sdrgpu_pipeline_wait(self.pipeline._h))
             self._stream_inflight -= 1
 
+    def outputs(self):
+        """what the last device-resident step handed its caller: the dibits of every channel row (zero past the row's
+        count) and the counts, or the channelizer's [channel][time] streams"""
+        if self.pipeline is None:
+            return {"channels": self.out_dev.cpu().numpy()}
+        cnt = self.cnt_dev.cpu().numpy()
+        return {"dibits": valid_prefix(self.sym_dev.cpu().numpy(), cnt), "dibit_counts": cnt}
+
     def sanity(self):
         """decoded-vs-transmitted dibits of a few rows (first pass over the streams, from the reset state; a plausibility
         figure for the timed workload -- parity itself is tests/)"""
@@ -674,8 +712,9 @@ class TunerWorkload:
             ch.dispose()
 
 
-def measure_tuner(w, args, world, timed, full=True):
-    """device-resident and host-buffer throughput of one TunerWorkload; `full` adds the secondary variants"""
+def measure_tuner(w, args, world, timed, full=True, capture=False):
+    """device-resident and host-buffer throughput of one TunerWorkload; `full` adds the secondary variants, `capture`
+    keeps the outputs of the last timed device-resident step (res["outputs"])"""
     L = w.L
     steps = args.steps
     sanity = w.sanity() if (full and not args.device_only) else None
@@ -686,6 +725,8 @@ def measure_tuner(w, args, world, timed, full=True):
     total = w.total_complex * world
     res = {"ms_per_step": ms_dev / steps, "value": total / (ms_dev / steps * 1e-3) / 1e6, "launches": launches,
            "sanity": sanity}
+    if capture:
+        res["outputs"] = w.outputs()        # before the legs below run the same buffers again
 
     def e2e_leg(fmt, note):
         w.set_format(fmt)
@@ -911,6 +952,10 @@ def run_bank(name, args, rank, world, local_rank, torch, dist, as_secondary=Fals
     launches0 = L.sdrgpu_launch_count()
     ms, _ = timed(step, stream, args.steps, args.warmup)
     launches = (L.sdrgpu_launch_count() - launches0) * args.steps // (args.steps + args.warmup)
+    if args.dump_outputs and not as_secondary and rank == 0:
+        counts = cnt.cpu().numpy()
+        dump_outputs(args.dump_outputs, {"dibits": valid_prefix(sym.cpu().numpy(), counts), "dibit_counts": counts} if hd
+                     else {"audio": valid_prefix(dem.cpu().numpy(), counts), "audio_counts": counts})
     e2e = None
     if not args.device_only:
         ms_h, wall_h = timed(step_host, stream, max(3, args.steps // 2), 3)
@@ -1059,8 +1104,10 @@ def run_gpu(args, rank, world, local_rank):
     w = TunerWorkload(args.workload, inputs, tuners, local_rank)
     if rank == 0:
         sampler.start()
-    r = measure_tuner(w, args, world, timed, full=True)
+    r = measure_tuner(w, args, world, timed, full=True, capture=bool(args.dump_outputs) and rank == 0)
     clocks = sampler.stop() if rank == 0 else None
+    if "outputs" in r:
+        dump_outputs(args.dump_outputs, r.pop("outputs"))
     main = summarize_tuner(w, r, peak, peak_src, args.steps, world)
     m, fs = w.m, cfg["fs"]
     w.dispose()
@@ -1152,7 +1199,15 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary measurements (tuner-count curve, other configs)")
     ap.add_argument("--device-only", action="store_true",
                     help="profiling aid: skip the host-buffer (e2e) passes so that every launch is a full-size one")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline workload computed as DIR/<name>.npy (float32, at "
+                         "most 64 MB: a fixed, seeded sample of rows when the output is larger); the inputs are seeded, so "
+                         "two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.sharding == "level2"):
+        ap.error("--dump-outputs writes the outputs of the GPU arm's level1 run")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,110 +1,114 @@
 """Pins the data and constants the reference embeds in its own sources (the only "golden vectors" it holds for this
-path) against what the oracle and the product carry.  Reads /root/reference, so it only runs in the build container
-(skipped elsewhere, e.g. on the GPU box)."""
+path) against what the oracle and the product carry.  The reference's values are stored in
+tests/golden/reference_constants.json: the MMSE table as tools/gen_mmse_table.py copied it from Interpolator.java, the
+rest as they stand in the Java sources named beside each check."""
+import json
 import os
 import re
 
 import numpy as np
-import pytest
 
 import oracle
 
-REF = "/root/reference/src/main/java/io/github/dsheirer"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not present")
+REF = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_constants.json")))
 
 
-def java(path):
-    return open(os.path.join(REF, path)).read()
+def source(*path):
+    return open(os.path.join(ROOT, *path)).read()
 
 
 def test_mmse_interpolator_table_is_the_references():
-    rows = []
-    for line in java("dsp/filter/interpolator/Interpolator.java").splitlines():
-        vals = re.findall(r"[-+]?\d\.\d+e[-+]\d+f", line)
-        if len(vals) == 8:
-            rows.append([np.float32(v[:-1]) for v in vals])
-    ref = np.array(rows, np.float32)
+    """dsp/filter/interpolator/Interpolator.java"""
+    ref = np.array([[np.float32(v) for v in row.split()] for row in REF["mmse_interpolator_taps"]], np.float32)
     assert ref.shape == (129, 8)
-    text = open(os.path.join(ROOT, "include", "sdr_mmse_taps.h")).read()
+    text = source("include", "sdr_mmse_taps.h")
     mine = np.array([np.float32(v[:-1]) for v in re.findall(r"[-+]?\d\.\d+e[-+]\d+f", text)], np.float32).reshape(129, 8)
     assert np.array_equal(mine, ref)
 
 
 def test_window_and_envelope_constants():
-    w = java("dsp/filter/Window.java")
-    a = [float(re.search(r"double a%d = ([0-9.]+);" % i, w).group(1)) for i in range(3)]
+    """dsp/filter/Window.java (Blackman a0..a2), sample/complex/Complex.java (envelope and fast normalisation),
+    dsp/gain/ComplexFeedForwardGainControl.java (MINIMUM_ENVELOPE)"""
+    a = [float(v) for v in REF["window_blackman_a"]]
     n = 23
     x = np.arange(n)
     want = a[0] - a[1] * np.cos(2 * np.pi * x / (n - 1)) + a[2] * np.cos(4 * np.pi * x / (n - 1))
     assert np.allclose(oracle.window("blackman", n), want, rtol=0, atol=1e-15)
-    c = java("sample/complex/Complex.java")
-    assert "(0.4f * quadratureAbsolute)" in c and "1.9999f - magnitudeSquared()" in c
-    assert "MINIMUM_ENVELOPE = 0.0001f" in java("dsp/gain/ComplexFeedForwardGainControl.java")
+    agc = REF["complex_feed_forward_gain_control"]
+    weight, scalor = "%gf" % agc["envelope_minor_axis_weight"], "%gf" % REF["complex_fast_normalize_constant"]
+    assert "(%s * qa)" % weight in source("oracle", "orc_filters.c")
+    assert "__fmul_rn(%s, b)" % weight in source("sdrtrunk_b200", "csrc", "bank.cu")
+    assert "(%s - norm)" % scalor in source("oracle", "orc_output.c")
+    assert "__fsub_rn(%s, norm)" % scalor in source("sdrtrunk_b200", "csrc", "channelizer.cu")
+    floor = np.float32(agc["minimum_envelope"])
     y = oracle.agc_block(np.array([3e-5, -1e-5] * 1024, np.float32))          # envelope below the minimum: gain 1 / 1e-4
-    assert np.array_equal(y[:2], np.array([3e-5, -1e-5], np.float32) * (np.float32(1.0) / np.float32(1e-4)))
+    assert np.array_equal(y[:2], np.array([3e-5, -1e-5], np.float32) * (np.float32(1.0) / floor))
 
 
 def test_decoder_front_end_constants():
-    assert "SAMPLE_COUNTER_GAIN = 0.3f" in java("module/decode/p25/phase1/P25P1DecoderC4FM.java")
-    assert "SAMPLE_COUNTER_GAIN = 0.3f" in java("module/decode/p25/phase1/P25P1DecoderLSM.java")
-    assert "SAMPLE_COUNTER_GAIN = 0.4f" in java("module/decode/dmr/DMRDecoder.java")
-    p2 = java("module/decode/p25/phase2/P25P2DecoderHDQPSK.java")
-    assert "SYMBOL_TIMING_GAIN = 0.1f" in p2 and "super(6000.0)" in p2 and "setPLLBandwidth(PLLBandwidth.BW_300)" in p2
-    assert "setPLLBandwidth(PLLBandwidth.BW_300)" in java("module/decode/p25/phase1/P25P1DecoderC4FM.java")
-    assert "setPLLBandwidth(PLLBandwidth.BW_200)" in java("module/decode/p25/phase1/P25P1DecoderLSM.java")
-    assert "setPLLBandwidth(PLLBandwidth.BW_300)" in java("module/decode/dmr/DMRDecoder.java")
-    bw = dict(re.findall(r"(BW_\d+)\((\d+\.\d+),", java("dsp/psk/pll/PLLBandwidth.java")))
-    assert bw == {"BW_400": "400.0", "BW_300": "300.0", "BW_250": "250.0", "BW_200": "200.0"}
-    assert "MAXIMUM_DEVIATION_SAMPLES_PER_SYMBOL = 0.02f" in java("dsp/psk/InterpolatingSampleBuffer.java")
-    dib = dict((m[0], int(m[1])) for m in re.findall(r"(D\d\d_\w+)\((?:true|false), (?:true|false), (\d),", java("dsp/symbol/Dibit.java")))
-    assert dib == {"D01_PLUS_3": 1, "D00_PLUS_1": 0, "D10_MINUS_1": 2, "D11_MINUS_3": 3}
-    # the presets of the C ABI carry the same numbers
+    """module/decode/p25/phase1/P25P1DecoderC4FM.java, P25P1DecoderLSM.java, phase2/P25P2DecoderHDQPSK.java,
+    dmr/DMRDecoder.java (symbol rate, PLL bandwidth, SAMPLE_COUNTER_GAIN / SYMBOL_TIMING_GAIN), dsp/psk/pll/PLLBandwidth.java,
+    dsp/psk/InterpolatingSampleBuffer.java, dsp/symbol/Dibit.java, dsp/filter/channelizer/PolyphaseChannelSource.java"""
     from sdrtrunk_b200 import native
+    from sdrtrunk_b200.dsp.bank import Dibit, PLLBandwidth
+    assert {b.name: b.value for b in PLLBandwidth} == REF["pll_bandwidth"]
+    assert {d.name: d.value for d in Dibit} == REF["dibit"]
+    deviation = "%gf" % REF["maximum_deviation_samples_per_symbol"]
+    for src in (source("oracle", "orc_psk.c"), source("sdrtrunk_b200", "csrc", "bank.cu")):
+        assert "sps * (1.0f + %s)" % deviation in src and "sps * (1.0f - %s)" % deviation in src
+    # the presets of the C ABI carry the same numbers
     cfg = native.BankConfig()
-    for preset, rate, bw_, gain in ((native.PRESET_P25_C4FM, 4800.0, 300.0, 0.3), (native.PRESET_P25_LSM, 4800.0, 200.0, 0.3),
-                                    (native.PRESET_P25_HDQPSK, 6000.0, 300.0, 0.1), (native.PRESET_DMR, 4800.0, 300.0, 0.4)):
-        native.check(native.lib().sdrgpu_bank_config_preset(cfg, preset, 1, 50000.0, None, 0, 1024))
-        assert (cfg.symbol_rate, cfg.pll_bandwidth) == (rate, bw_) and abs(cfg.sample_counter_gain - gain) < 1e-7
-        assert cfg.block_size == 1024 and cfg.agc == 1
-    assert "PROCESSED_BUFFER_SAMPLE_SIZE = 2048" in java("dsp/filter/channelizer/PolyphaseChannelSource.java")
+    presets = {"c4fm": native.PRESET_P25_C4FM, "lsm": native.PRESET_P25_LSM, "hdqpsk": native.PRESET_P25_HDQPSK,
+               "dmr": native.PRESET_DMR}
+    for kind, want in REF["decoders"].items():
+        native.check(native.lib().sdrgpu_bank_config_preset(cfg, presets[kind], 1, 50000.0, None, 0, 1024))
+        assert cfg.symbol_rate == want["symbol_rate"], kind
+        assert cfg.pll_bandwidth == REF["pll_bandwidth"][want["pll_bandwidth"]], kind
+        assert abs(cfg.sample_counter_gain - want["sample_counter_gain"]) < 1e-7, kind
+        assert 2 * cfg.block_size == REF["processed_buffer_sample_size"] and cfg.agc == 1
 
 
 def test_half_band_stage_plan_is_the_references():
-    """ComplexDecimateX{N}Filter stage lengths / windows (SURVEY a9)"""
-    plan = {2: [(63, "HAMMING")], 4: [(23, "BLACKMAN"), (63, "HAMMING")], 8: [(15, "BLACKMAN"), (23, "BLACKMAN"), (63, "HAMMING")]}
-    for rate, stages in plan.items():
-        src = java("dsp/filter/decimate/ComplexDecimateX%dFilter.java" % rate)
-        found = re.findall(r"DECIMATE_BY_\d+_FILTER_LENGTH = (\d+)", src)
-        wins = re.findall(r"WINDOW_TYPE = Window\.WindowType\.(\w+)", src)
-        assert [int(v) for v in found] == [stages[0][0]], (rate, found)
-        assert wins == [stages[0][1]], (rate, wins)
+    """ComplexDecimateX{N}Filter stage lengths / windows (SURVEY a9): decimation by 2^k runs the X{2^k} filter's stage, then
+    the X{2^(k-1)} one's, down to X2; the oracle (orc_filters.c) and the product (bank.cu) build the same cascade"""
+    first = {int(r): (length, window) for r, (length, window) in REF["complex_decimate_filter"].items()}
+    plan = {rate: [first[r] for r in (8, 4, 2) if r <= rate] for rate in first}
+    assert plan == {2: [(63, "HAMMING")], 4: [(23, "BLACKMAN"), (63, "HAMMING")],
+                    8: [(15, "BLACKMAN"), (23, "BLACKMAN"), (63, "HAMMING")]}
+    for src in (source("oracle", "orc_filters.c"), source("sdrtrunk_b200", "csrc", "bank.cu")):
+        stages = {int(r): (int(n), w) for r, n, w in
+                  re.findall(r"if \(r == (\d+)\) \{ len = (\d+); win = \w+_(BLACKMAN|HAMMING); \}", src)}
+        other = re.search(r"else \{ len = (\d+); win = \w+_(BLACKMAN|HAMMING); \}", src)
+        stages[2] = (int(other.group(1)), other.group(2))
+        assert re.search(r"for \(int r = [\w>-]+; r >= 2; r /= 2\)", src)
+        assert {r: stages[r] for r in first} == first
 
 
 def test_sync_patterns_and_detector_constants():
-    """FrameSync patterns, match threshold, delay lengths and PLL corrections of the P25 sync detectors, as carried by
-    the oracle (orc_sync.c) and the product (SyncTraits in bank.cu)."""
-    fs = dict((k, int(v, 16)) for k, v in re.findall(r"(P25_PHASE\d_\w+)\(\s*0x([0-9A-Fa-f]+)l\s*\)", java("dsp/symbol/FrameSync.java")))
+    """dsp/symbol/FrameSync.java patterns, match threshold, delay lengths and sync-loss lengths of the P25 sync detectors
+    (P25P1SyncDetector, P25P2SyncDetector, P25P1DataUnitDetector, P25P2SuperFrameDetector), as carried by the oracle
+    (orc_sync.c) and the product (SyncTraits in bank.cu)."""
+    fs = {k: int(v, 16) for k, v in REF["frame_sync"].items()}
+    det = REF["sync_detectors"]
     assert len(fs) == 8
-    for src in (open(os.path.join(ROOT, "oracle", "orc_sync.c")).read(),
-                open(os.path.join(ROOT, "sdrtrunk_b200", "csrc", "bank.cu")).read()):
+    oracle_src, product_src = source("oracle", "orc_sync.c"), source("sdrtrunk_b200", "csrc", "bank.cu")
+    for src in (oracle_src, product_src):
         mine = set(int(v, 16) for v in re.findall(r"0x([0-9A-Fa-f]{10,12})ull", src))
         assert set(fs.values()) <= mine
-    p1 = java("module/decode/p25/phase1/P25P1SyncDetector.java")
-    p2 = java("module/decode/p25/phase2/P25P2SyncDetector.java")
-    assert "SYNC_MATCH_THRESHOLD = 4" in p1 and "SYNC_MATCH_THRESHOLD = 4" in p2
-    assert "DEFAULT_SYMBOL_RATE = 4800" in p1 and "DEFAULT_SYMBOL_RATE = 6000" in p2
-    assert "getMessageLength(), 48)" in p1 and "MultiSyncPatternMatcher(syncDetectListener, 1440, 40)" in p2
-    assert "LOGICAL_LINK_DATA_UNIT_1(5, 1568," in java("module/decode/p25/phase1/P25P1DataUnitID.java")
-    dud = java("module/decode/p25/phase1/P25P1DataUnitDetector.java")
-    assert "DATA_UNIT_DIBIT_LENGTH = 57" in dud and "SYNC_DIBIT_LENGTH = 24" in dud
-    assert "new DibitDelayBuffer(160)" in java("module/decode/p25/phase2/P25P2SuperFrameDetector.java")
-    assert oracle.SyncDetector(oracle.SYNC_P25_PHASE1, 50000.0).delay == 57 - 24
-    assert oracle.SyncDetector(oracle.SYNC_P25_PHASE2, 50000.0).delay == 160
+    assert "s->threshold = %d;" % det["match_threshold"] in oracle_src
+    assert "kSyncMatchThreshold = %d;" % det["match_threshold"] in product_src
+    p1, p2 = det["p25_phase1"], det["p25_phase2"]
+    for n in (p1["sync_loss_bits"], p2["sync_loss_bits"]):
+        assert "s->sync_loss_threshold = %d;" % n in oracle_src and "loss_bits = %d;" % n in product_src
+    assert "sync_size = %d;" % p1["sync_bits"] in oracle_src and "sync_size = %d;" % p2["sync_bits"] in oracle_src
+    assert "symbol_rate = %.1f;" % p1["symbol_rate"] in oracle_src and "symbol_rate = %.1f;" % p2["symbol_rate"] in oracle_src
+    assert oracle.SyncDetector(oracle.SYNC_P25_PHASE1, 50000.0).delay == p1["data_unit_dibit_length"] - p1["sync_dibit_length"]
+    assert oracle.SyncDetector(oracle.SYNC_P25_PHASE2, 50000.0).delay == p2["delay_dibits"]
     # the rotated patterns are the normal one with every dibit's constellation point turned by 90 / 180 degrees:
     # +1 (00) -> +3 (01) -> -3 (11) -> -1 (10) -> +1 going counter-clockwise
     ccw = {0: 1, 1: 3, 3: 2, 2: 0}
-    for phase, bits in (("PHASE1", 48), ("PHASE2", 40)):
+    for phase, bits in (("PHASE1", p1["sync_bits"]), ("PHASE2", p2["sync_bits"])):
         d = [(fs["P25_%s_NORMAL" % phase] >> (bits - 2 - 2 * k)) & 3 for k in range(bits // 2)]
         def rotate(seq, quarter_turns):
             for _ in range(quarter_turns):

@@ -1,5 +1,5 @@
-import sys, time, json
-sys.path.insert(0, '/root/repo')
+import os, sys, time, json
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch, bench
 from sdrtrunk_b200 import native
 torch.cuda.set_device(0); native.init(0)
