@@ -347,7 +347,8 @@ def _sync_case(kind, rng, n, offset, with_sync=True):
 
 
 @pytest.mark.parametrize("kind,lanes", [("c4fm", 0), ("lsm", 0), ("hdqpsk", 0), ("c4fm", 16), ("hdqpsk", 16), ("lsm", 1),
-                                        ("c4fm", 8), ("c4fm", 4), ("lsm", 8), ("lsm", 4), ("hdqpsk", 8), ("hdqpsk", 4)])
+                                        ("c4fm", 8), ("c4fm", 4), ("lsm", 8), ("lsm", 4), ("hdqpsk", 8), ("hdqpsk", 4),
+                                        ("c4fm", 2), ("hdqpsk", 2)])
 def test_sync_detector_and_inversion_feedback_on_device(gpu, kind, lanes):
     """SURVEY 8f #3: the framer's sync detector + PLLPhaseInversionDetector feedback run inside the demodulator
     kernel.  Channels locked 90 / 180 degrees off (carrier offset = +-rate/4, rate/2) must be corrected at the very
@@ -390,7 +391,8 @@ def test_sync_detector_and_inversion_feedback_on_device(gpu, kind, lanes):
 
 
 @pytest.mark.parametrize("kind,lanes,sync", [("c4fm", 0, False), ("c4fm", 4, False), ("c4fm", 32, True), ("c4fm", 4, True),
-                                             ("lsm", 0, False), ("hdqpsk", 16, True), ("hdqpsk", 1, False)])
+                                             ("lsm", 0, False), ("hdqpsk", 16, True), ("hdqpsk", 1, False),
+                                             ("c4fm", 2, True), ("hdqpsk", 2, True)])
 def test_symbol_tap_matches_the_instrumented_demodulator(gpu, kind, lanes, sync):
     """SURVEY section 5 / DQPSK*DemodulatorInstrumented: the per-symbol tap of one channel of a bank (complex symbol, samples
     per symbol, PLL frequency, sampling point, PLL error) equals the oracle demodulator's taps on the same FIR / AGC output,

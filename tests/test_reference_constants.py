@@ -55,7 +55,7 @@ def test_decoder_front_end_constants():
     assert {b.name: b.value for b in PLLBandwidth} == REF["pll_bandwidth"]
     assert {d.name: d.value for d in Dibit} == REF["dibit"]
     deviation = "%gf" % REF["maximum_deviation_samples_per_symbol"]
-    for src in (source("oracle", "orc_psk.c"), source("sdrtrunk_b200", "csrc", "bank.cu")):
+    for src in (source("oracle", "orc_psk.c"), source("sdrtrunk_b200", "csrc", "psk.cu")):
         assert "sps * (1.0f + %s)" % deviation in src and "sps * (1.0f - %s)" % deviation in src
     # the presets of the C ABI carry the same numbers
     cfg = native.BankConfig()
@@ -88,11 +88,11 @@ def test_half_band_stage_plan_is_the_references():
 def test_sync_patterns_and_detector_constants():
     """dsp/symbol/FrameSync.java patterns, match threshold, delay lengths and sync-loss lengths of the P25 sync detectors
     (P25P1SyncDetector, P25P2SyncDetector, P25P1DataUnitDetector, P25P2SuperFrameDetector), as carried by the oracle
-    (orc_sync.c) and the product (SyncTraits in bank.cu)."""
+    (orc_sync.c) and the product (SyncTraits in psk.cu)."""
     fs = {k: int(v, 16) for k, v in REF["frame_sync"].items()}
     det = REF["sync_detectors"]
     assert len(fs) == 8
-    oracle_src, product_src = source("oracle", "orc_sync.c"), source("sdrtrunk_b200", "csrc", "bank.cu")
+    oracle_src, product_src = source("oracle", "orc_sync.c"), source("sdrtrunk_b200", "csrc", "psk.cu")
     for src in (oracle_src, product_src):
         mine = set(int(v, 16) for v in re.findall(r"0x([0-9A-Fa-f]{10,12})ull", src))
         assert set(fs.values()) <= mine

@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Demodulator kernel time by bank size and lanes per channel (C4FM, decision directed): the data behind the
-automatic layout choice in bank.cu.  usage (GPU box): python tools/psk_layout_sweep.py"""
+automatic layout choice in psk.cu.  usage (GPU box): python tools/psk_layout_sweep.py"""
 import os
 import sys
 
