@@ -295,6 +295,7 @@ __global__ void __launch_bounds__(kThreads) pfb_ifft_kernel(const ChanParams p)
 //      in registers, products rounded and added in tap order like the Java)         -> V[b][n]         (shared)
 //   2. step A: thread (b, n2) runs an R1-point DFT over n1 of V[b][R2 n1 + n2] in registers, multiplies by
 //      W_M^{n2 k1}                                                                  -> Y[b][k1][n2]    (shared)
+//      (NB = 8: V is stored in Y's layout and step A transforms it in place -- see Pfb2Layout)
 //   3. step B: thread (b, k1) runs an R2-point DFT over n2 in registers: bin k1 + R1 k2.  With the default selection
 //      (every bin, one gain) and NB = 8 the 8 lanes holding one bin's 8 consecutive samples scale and write them
 //      straight to the channel's row (64 contiguous bytes) -- done.  Otherwise                -> X[b][k] (shared)
@@ -322,11 +323,18 @@ struct Pfb2Layout {
     static constexpr int y_base = R1 * R2P;
     static constexpr int y_want = NB == 8 ? 2 : (((R2 % 16) + 1) & ~1);
     static constexpr int YB = y_base + ((y_want - y_base % 16) + 16) % 16;
-    static constexpr int region0 = (NB * SV > NB * XS) ? NB * SV : NB * XS;
+    // NB == 8: the filter bank writes V[b][R2 n1 + n2] straight into Y's layout, at Y[b][n1][n2].  Step A's thread (b, n2)
+    // reads column n2 of block b for every n1 and writes the same column for every k1, so it transforms in place and V
+    // needs no region of its own; X (general selection) gets one behind Y.  NB == 16: V / X share region 0, Y follows.
+    static constexpr bool v_in_y = NB == 8;
+    static constexpr int region0 = v_in_y ? NB * XS : (NB * SV > NB * XS) ? NB * SV : NB * XS;
+    static constexpr int y_off = v_in_y ? 0 : region0, x_off = v_in_y ? NB * YB : 0;
     static constexpr size_t smem_bytes = sizeof(float2) * (size_t)(region0 + NB * YB);
+    static constexpr size_t smem_direct = v_in_y ? sizeof(float2) * (size_t)(NB * YB) : smem_bytes;   // no X
 };
 
-template <int M, int NB, int TT, bool FAST, bool RAW>
+// V[bl * SV + vidx(n)]: vidx(n) = n, or with R2 > 0 the row layout of Y, R2 = row length, R2P = row pitch
+template <int M, int NB, int TT, bool FAST, bool RAW, int R2 = 0, int R2P = 0>
 __device__ __forceinline__ void fb_thread(const ChanParams &p, const float2 *__restrict__ xin, long long first, int b0, int r,
                                           float2 *V, int SV)
 {
@@ -377,26 +385,30 @@ __device__ __forceinline__ void fb_thread(const ChanParams &p, const float2 *__r
         }
     }
     const int par = (p.parity0 + b0) & 1;
+    const int ilo = R2 > 0 ? (n / R2) * R2P + n % R2 : n;
+    const int ihi = R2 > 0 ? ((n + half) / R2) * R2P + (n + half) % R2 : n + half;
 #pragma unroll
     for (int bl = 0; bl < NB; bl++) {
         const int odd = (par + bl) & 1;   // "middle" blocks: the two halves swap (the M/2 circular shift)
-        V[bl * SV + (odd ? n + half : n)] = accA[bl];
-        V[bl * SV + (odd ? n : n + half)] = accB[bl];
+        V[bl * SV + (odd ? ihi : ilo)] = accA[bl];
+        V[bl * SV + (odd ? ilo : ihi)] = accB[bl];
     }
 }
 
 template <int M, int R1, int R2, int NB, int TT, int NT, int MINB, bool RAW>
-// M = 800: bounded as if the CTA had one more warp -- ptxas then settles for 96 registers instead of the 128 the bound allows,
-// without a spill and at the same speed (1.40 ms per 8 launches either way), which leaves a quarter of the register file to
-// whatever runs beside the channelizers (the oscillator producers of frequency-corrected channels: their one-warp CTAs
-// otherwise wait for -- or keep out -- a whole 32 K-register channelizer CTA).  M = 400 needs its 72 (64: a spill, 1 % slower).
-__global__ void __launch_bounds__(M == 800 ? NT + 32 : NT, MINB) pfb2_kernel(const ChanParams p)
+// M = 800 runs three CTAs per SM: 80 registers (no spill; 8 bytes with 8-bit input) and, with V inside Y, 53 KB of shared
+// memory per CTA on the direct-store path.  The third CTA's phases fill the barriers of the other two: 1.40 -> 1.15 ms per
+// 8 launches on a B200 at 1000 W (profiles/r5f_pfb_pipe_time.txt); 3 x 256 x 80 registers still leave 4 K to the one-warp oscillator
+// producers of frequency-corrected channels.  M = 400 needs its 72 (64: a spill, 1 % slower).
+__global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
 {
     using L = Pfb2Layout<M, R1, R2, NB, TT, NT>;
     constexpr int half = M / 2, SV = L::SV, XS = L::XS, R2P = L::R2P, YB = L::YB;
     extern __shared__ __align__(16) float2 smem[];
-    float2 *V = smem;                 // [NB][SV], later X [NB][XS]
-    float2 *Y = smem + L::region0;    // [NB][R1][R2P]
+    float2 *Y = smem + L::y_off;      // [NB][R1][R2P]
+    float2 *V = L::v_in_y ? Y : smem; // [NB][SV], or Y's layout
+    float2 *X = smem + L::x_off;      // [NB][XS]
+    constexpr int VS = L::v_in_y ? YB : SV, VR2 = L::v_in_y ? R2 : 0, VR2P = L::v_in_y ? R2P : 0;
     const int tid = threadIdx.x;
     const int b0 = blockIdx.x * NB;
 
@@ -430,9 +442,9 @@ __global__ void __launch_bounds__(M == 800 ? NT + 32 : NT, MINB) pfb2_kernel(con
                 }
         }
         if (fast) {
-            for (int r = tid; r < half; r += NT) fb_thread<M, NB, TT, true, RAW>(p, xin, first, b0, r, V, SV);
+            for (int r = tid; r < half; r += NT) fb_thread<M, NB, TT, true, RAW, VR2, VR2P>(p, xin, first, b0, r, V, VS);
         } else {
-            for (int r = tid; r < half; r += NT) fb_thread<M, NB, TT, false, RAW>(p, xin, first, b0, r, V, SV);
+            for (int r = tid; r < half; r += NT) fb_thread<M, NB, TT, false, RAW, VR2, VR2P>(p, xin, first, b0, r, V, VS);
         }
     }
     __syncthreads();
@@ -441,9 +453,9 @@ __global__ void __launch_bounds__(M == 800 ? NT + 32 : NT, MINB) pfb2_kernel(con
     for (int item = tid; item < NB * R2; item += NT) {
         const int b = NB == 8 ? (item & 7) : item / R2, n2 = NB == 8 ? (item >> 3) : item - b * R2;
         float2 a[R1];
-        const float2 *v = V + b * SV + n2;
+        const float2 *v = V + b * VS + n2;
 #pragma unroll
-        for (int n1 = 0; n1 < R1; n1++) a[n1] = v[R2 * n1];
+        for (int n1 = 0; n1 < R1; n1++) a[n1] = v[(L::v_in_y ? R2P : R2) * n1];
         rfft::dft<R1>(a);
         float2 *y = Y + b * YB + n2;
         y[0] = a[0];
@@ -456,7 +468,6 @@ __global__ void __launch_bounds__(M == 800 ? NT + 32 : NT, MINB) pfb2_kernel(con
     __syncthreads();
 
     // ------------------------------------------------------------------ 3. step B: R2-point DFTs over n2
-    float2 *X = V;
     // Default selection (every bin in order, one float-representable gain) with block-fastest lanes: the 8 lanes that
     // hold one bin's 8 consecutive samples write them straight to that channel's row (64 contiguous bytes), so the
     // X transpose, its barrier and the store pass are skipped.
@@ -1001,8 +1012,10 @@ sdrgpu_status launch_pfb2(const sdrgpu_channelizer *h, const ChanParams &p)
     using L = Pfb2Layout<M, R1, R2, NB, TT, NT>;
     auto kernel = pfb2_kernel<M, R1, R2, NB, TT, NT, MINB, RAW>;
     // a pipeline that overlaps its time chunks with the demodulator holds the channelizer to a few CTAs per SM
-    const size_t smem = (h->throttled || g_tuning[SDRGPU_TUNE_THROTTLE_ALWAYS]) ? smem_for_ctas_per_sm(L::smem_bytes, 0, g_tuning[SDRGPU_TUNE_PFB_CTAS_PER_SM]) : L::smem_bytes;
-    SDRGPU_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem > L::smem_bytes ? 227 * 1024 : L::smem_bytes)));
+    // the direct row stores (NB = 8, default selection, channel layout) need no X region
+    const size_t need = (p.identity && p.layout == SDRGPU_LAYOUT_CHANNELS) ? L::smem_direct : L::smem_bytes;
+    const size_t smem = (h->throttled || g_tuning[SDRGPU_TUNE_THROTTLE_ALWAYS]) ? smem_for_ctas_per_sm(need, 0, g_tuning[SDRGPU_TUNE_PFB_CTAS_PER_SM]) : need;
+    SDRGPU_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem > need ? 227 * 1024 : L::smem_bytes)));
     const int grid = (p.n_blocks + NB - 1) / NB;
     kernel<<<grid, NT, smem, h->stream>>>(p);
     count_launch();
@@ -1143,11 +1156,12 @@ sdrgpu_status sdrgpu::chan_enqueue(sdrgpu_channelizer *h, const float2 *d_in, in
         }
         h->timer.begin(h->stream);
         sdrgpu_status st;
-        // tile sizes measured on B200 (profiles/): M = 400 runs best as 8-block tiles, 200 threads, 4 CTAs per SM
+        // tile sizes measured on B200 (profiles/): M = 400 runs best as 8-block tiles, 200 threads, 4 CTAs per SM; M = 800 as
+        // 8-block tiles, 256 threads, 3 CTAs per SM
         if (fuse_convert && h->M == 400) st = launch_pfb2<400, 20, 20, 8, 9, 200, 4, true>(h, p);
-        else if (fuse_convert && h->M == 800) st = launch_pfb2<800, 32, 25, 8, 9, 256, 2, true>(h, p);
+        else if (fuse_convert && h->M == 800) st = launch_pfb2<800, 32, 25, 8, 9, 256, 3, true>(h, p);
         else if (h->fast_r1 && h->M == 400) st = launch_pfb2<400, 20, 20, 8, 9, 200, 4>(h, p);
-        else if (h->fast_r1 && h->M == 800) st = launch_pfb2<800, 32, 25, 8, 9, 256, 2>(h, p);
+        else if (h->fast_r1 && h->M == 800) st = launch_pfb2<800, 32, 25, 8, 9, 256, 3>(h, p);
         else if (h->fast_r1 && h->M == 96) st = launch_pfb2<96, 8, 12, 16, 9, 192, 2>(h, p);
         else if (h->fast_r1 && h->M == 640) st = launch_pfb2<640, 32, 20, 8, 9, 320, 2>(h, p);
         else if (h->fast_r1 && h->M == 320) st = launch_pfb2<320, 16, 20, 8, 9, 160, 4>(h, p);
