@@ -96,30 +96,37 @@ def test_agc_block_bit_exact(gpu):
 
 @pytest.mark.parametrize("n_taps", [5, 8, 24, 72, 154, 301])
 def test_fir_agc_whole_buffers_bit_exact(gpu, n_taps):
-    """FIR + block AGC over whole 1024-sample assembler buffers -- the decoders' framing, served by
-    fir_agc_split_kernel (per-warp windows, split-phase maximum exchange) -- in calls of 1, 7, 2, 4 and 3 buffers
-    (odd and even tile counts per CTA), with ragged calls in between that the general fir_agc_kernel takes: the
-    history a kernel leaves is the history the other one starts from"""
+    """FIR + block AGC over whole 1024-sample assembler buffers -- the decoders' framing -- in calls of 1, 7, 2, 4 and 3
+    buffers (odd and even tile counts per CTA).  Calls that are not throttled run fir_agc_split_kernel (per-warp windows,
+    split-phase maximum exchange); calls held to 1 or 2 CTAs per SM ask for more shared memory than the window needs and
+    run the general fir_agc_kernel.  The two kernels alternate on one bank: the history a kernel leaves is the history
+    the other one starts from"""
     from sdrtrunk_b200 import native
     from sdrtrunk_b200.dsp import Bank
     rng = np.random.default_rng(100 + n_taps)
     taps = (rng.standard_normal(n_taps) / n_taps).astype(np.float32)
     c = 7
-    steps = (1024, 7 * 1024, 1000, 24, 2 * 1024, 4 * 1024, 500, 524, 3 * 1024)
-    n = sum(steps)
+    # (samples, FIR CTAs per SM: 0 = not throttled)
+    steps = ((1024, 0), (7 * 1024, 1), (1000, 0), (24, 2), (2 * 1024, 0), (4 * 1024, 2), (500, 0), (524, 1), (3 * 1024, 0))
+    n = sum(step for step, _ in steps)
     x = _noise(rng, c, n, 0.05)
     x[1, 2 * 3000:2 * 6000] = 0.0     # silent buffers: the gain clamps at 1 / 1e-4
     x[2] *= 1e-6
     bank = Bank(c, 50000.0, fir_taps=taps, fir_gain=1.25, agc=True, max_samples_per_call=8 * 1024)
+    lib = native.lib()
     # a small bank would get one buffer per CTA: ask for the large banks' launch shape (3 consecutive buffers per CTA)
-    native.check(native.lib().sdrgpu_set_tuning(native.TUNE_FIR_TILES_PER_CTA, 3))
+    native.check(lib.sdrgpu_set_tuning(native.TUNE_FIR_TILES_PER_CTA, 3))
     try:
         parts, pos = [], 0
-        for step in steps:
+        for step, ctas in steps:
+            native.check(lib.sdrgpu_set_tuning(native.TUNE_THROTTLE_ALWAYS, 1 if ctas else 0))
+            native.check(lib.sdrgpu_set_tuning(native.TUNE_FIR_CTAS_PER_SM, ctas))
             parts.append(bank.process(x[:, 2 * pos:2 * (pos + step)]))
             pos += step
     finally:
-        native.check(native.lib().sdrgpu_set_tuning(native.TUNE_FIR_TILES_PER_CTA, 0))
+        native.check(lib.sdrgpu_set_tuning(native.TUNE_FIR_TILES_PER_CTA, 0))
+        native.check(lib.sdrgpu_set_tuning(native.TUNE_THROTTLE_ALWAYS, 0))
+        native.check(lib.sdrgpu_set_tuning(native.TUNE_FIR_CTAS_PER_SM, 0))
     got = np.concatenate(parts, axis=1)
     assert got.shape == (c, 2 * n)
     for k in range(c):
@@ -236,6 +243,46 @@ def test_fused_nbfm_kernel_all_cascade_depths(gpu, rate):
         want = np.concatenate(want)
         assert np.array_equal(got[k] == 0.0, want == 0.0), (rate, k)       # identical gating
         assert np.any(want != 0.0) and np.any(want == 0.0)
+        assert np.max(np.abs(got[k] - want)) < 1e-6, (rate, k)
+        assert np.mean(got[k] == want) > 0.999
+
+
+@pytest.mark.parametrize("rate, agc", [(16, False), (32, False), (4, True)])
+def test_five_kernel_nbfm_path(gpu, rate, agc):
+    """FM banks that nbfm_fused_kernel does not fit: halfband_kernel stages, the FIR kernels, then squelch_gate_kernel,
+    fm_kernel and fm_carry_kernel -- four half-band stages (decimation 16), an 11-tap first stage (decimation 32), and
+    block AGC (512-sample AGC buffers) -- against the oracle's decimator -> ComplexFIR [-> AGC] -> SquelchingFMDemodulator,
+    buffer by buffer.  Every channel has a quiet stretch of 1536 output samples: the squelch opens, closes and opens
+    again at the output rate."""
+    from sdrtrunk_b200.dsp import Bank
+    rng = np.random.default_rng(60 + rate)
+    c, block = 3, 2048
+    n = 4096 * rate                                   # channel-rate input samples per channel (4096 outputs)
+    fir = oracle.nbfm_iq_taps()
+    x = []
+    for k in range(c):
+        loud = sg.nbfm(25000.0 * rate, n, audio_hz=300.0 * (k + 1), carrier_offset=150.0 * k, amplitude=0.3) + sg.awgn(rng, n, 1e-3)
+        env = np.ones(n)
+        q0 = n // 8 + k * n // 16
+        env[q0:q0 + 3 * n // 8] = 1e-7                # quiet enough to close the squelch behind the AGC's 1e4 gain too
+        x.append(sg.interleave(loud * env))
+    x = np.stack(x)
+    bank = Bank(c, 25000.0 * rate, demod=gpu.DEMOD_FM_SQUELCH, fir_taps=fir, decimation=rate, agc=agc, squelch_alpha=0.01,
+                squelch_threshold_db=-40.0, squelch_ramp=4, block_size=block, max_samples_per_call=n // 2)
+    cuts = sorted({0, 3 * block, 4 * block, n // 2, n})
+    got = np.concatenate([bank.process(x[:, 2 * a:2 * b]) for a, b in zip(cuts[:-1], cuts[1:])], axis=1)
+    assert got.shape == (c, n // rate)
+    for k in range(c):
+        dec, f = oracle.Decimator(rate), oracle.ComplexFIR(fir)
+        fm = oracle.SquelchingFMDemodulator(0.01, -40.0, 4)
+        want = []
+        for b in range(n // block):
+            y = f.filter(dec.decimate_complex(x[k, 2 * block * b:2 * block * (b + 1)]))
+            want.append(fm.demodulate(oracle.agc_block(y) if agc else y))
+        want = np.concatenate(want)
+        assert np.array_equal(got[k] == 0.0, want == 0.0), (rate, k)       # identical gating
+        on = np.flatnonzero(want != 0.0)
+        assert on.size and np.any(want[on[0]:] == 0.0), (rate, k)         # opens, then closes
         assert np.max(np.abs(got[k] - want)) < 1e-6, (rate, k)
         assert np.mean(got[k] == want) > 0.999
 

@@ -38,7 +38,7 @@ def test_window_and_envelope_constants():
     agc = REF["complex_feed_forward_gain_control"]
     weight, scalor = "%gf" % agc["envelope_minor_axis_weight"], "%gf" % REF["complex_fast_normalize_constant"]
     assert "(%s * qa)" % weight in source("oracle", "orc_filters.c")
-    assert "__fmul_rn(%s, b)" % weight in source("sdrtrunk_b200", "csrc", "bank.cu")
+    assert "__fmul_rn(%s, b)" % weight in source("sdrtrunk_b200", "csrc", "filters.cu")
     assert "(%s - norm)" % scalor in source("oracle", "orc_output.c")
     assert "__fsub_rn(%s, norm)" % scalor in source("sdrtrunk_b200", "csrc", "channelizer.cu")
     floor = np.float32(agc["minimum_envelope"])
