@@ -24,13 +24,13 @@
 // 128-byte line for NB = 16) are bank-conflict free and coalesced.
 #include <cmath>
 #include <cstdint>
-#include <cstdlib>
 #include <cstring>
 #include <utility>
 #include <vector>
 
 #include "common.cuh"
 #include "fft_regs.cuh"
+#include "outputs.cuh"
 
 using namespace sdrgpu;
 
@@ -86,15 +86,22 @@ __device__ __forceinline__ float2 load_raw(const ChanParams &p, long long idx)
     return make_float2(__fmul_rn((float)vi, 0.0078125f), __fmul_rn((float)vq, 0.0078125f));
 }
 
+// sample idx of the virtual stream [state | in | zeros] the filter bank reads: the history (and leftover samples) the call
+// starts from, its new samples, then zeros; state(i) and in(i) load sample i of the first two
+template <class State, class In>
+__device__ __forceinline__ float2 stream_sample(int idx, int state_len, int n_in, State state, In in)
+{
+    if (idx < state_len) return state(idx);
+    idx -= state_len;
+    return idx < n_in ? in(idx) : make_float2(0.0f, 0.0f);
+}
+
 template <bool RAW = false>
 __device__ __forceinline__ float2 load_x(const ChanParams &p, int unit, int r)
 {
-    // virtual concatenation [state | in | zeros]; unit 0 starts right after the history
-    int idx = p.H + unit * p.half + r;
-    if (idx < p.state_len) return __ldg(p.state + idx);
-    idx -= p.state_len;
-    if (idx < p.n_in) return RAW ? load_raw(p, idx) : __ldg(p.in + idx);
-    return make_float2(0.0f, 0.0f);
+    // unit 0 starts right after the history
+    return stream_sample(p.H + unit * p.half + r, p.state_len, p.n_in, [&](int i) { return __ldg(p.state + i); },
+                         [&](int i) { return RAW ? load_raw(p, i) : __ldg(p.in + i); });
 }
 
 __device__ __forceinline__ float2 cmul(float2 a, float2 w)
@@ -289,7 +296,7 @@ __global__ void __launch_bounds__(kThreads) pfb_ifft_kernel(const ChanParams p)
 
 // ---------------------------------------------------------------------------------------------------------------
 // pfb2_kernel: the fast path for channel counts that split as M = R1 * R2 with register-sized factors
-// (400 = 20 x 20, 800 = 32 x 25, 96 = 8 x 12, ... see sdrgpu_chan_create).  One CTA per tile of NB consecutive blocks:
+// (400 = 20 x 20, 800 = 32 x 25, 96 = 8 x 12, ... see kPfbRows).  One CTA per tile of NB consecutive blocks:
 //   0. L2 read-ahead of the input the tile one wave later will need (its first touch is otherwise a DRAM round trip)
 //   1. filter bank (as above: thread <-> input offset r, taps in registers, NB blocks of two branches accumulated
 //      in registers, products rounded and added in tap order like the Java)         -> V[b][n]         (shared)
@@ -361,26 +368,16 @@ __device__ __forceinline__ void fb_thread(const ChanParams &p, const float2 *__r
         for (int t = 0; t < TT; t++) {
             const int bl = pp + 2 * t;  // branch n: unit P = B - 2t
             if (bl >= 0 && bl < NB) {
-#ifdef SDRGPU_PFB_FMA
-                if (t == 0) accA[bl] = make_float2(__fmul_rn(x.x, hA[t]), __fmul_rn(x.y, hA[t]));
-                else accA[bl] = make_float2(__fmaf_rn(x.x, hA[t], accA[bl].x), __fmaf_rn(x.y, hA[t], accA[bl].y));
-#else
                 const float2 pr = __ffma2_rn(x, make_float2(hA[t], hA[t]), nz);
                 // (the Java's 0.0f + product differs from the product only in the sign of a zero)
                 if (t == 0) accA[bl] = pr;
                 else accA[bl] = __fadd2_rn(accA[bl], pr);
-#endif
             }
             const int bm = pp + 1 + 2 * t;  // branch n + M/2: unit P = B - 1 - 2t
             if (bm >= 0 && bm < NB) {
-#ifdef SDRGPU_PFB_FMA
-                if (t == 0) accB[bm] = make_float2(__fmul_rn(x.x, hB[t]), __fmul_rn(x.y, hB[t]));
-                else accB[bm] = make_float2(__fmaf_rn(x.x, hB[t], accB[bm].x), __fmaf_rn(x.y, hB[t], accB[bm].y));
-#else
                 const float2 pr = __ffma2_rn(x, make_float2(hB[t], hB[t]), nz);
                 if (t == 0) accB[bm] = pr;
                 else accB[bm] = __fadd2_rn(accB[bm], pr);
-#endif
             }
         }
     }
@@ -415,13 +412,9 @@ __global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
     // the history the next call starts from, next_state[i] = [state | in][consumed + i]: a few KB copied by one CTA of
     // the middle of the grid into the other half of the state ping-pong (a separate launch costs 3 % of the step)
     if (p.next_state != nullptr && blockIdx.x == (gridDim.x >> 1)) {
-        for (int i = tid; i < p.next_len; i += NT) {
-            const int idx = p.consumed + i;
-            float2 v = make_float2(0.0f, 0.0f);
-            if (idx < p.state_len) v = p.state[idx];
-            else if (idx - p.state_len < p.n_in) v = RAW ? load_raw(p, idx - p.state_len) : p.in[idx - p.state_len];
-            p.next_state[i] = v;
-        }
+        for (int i = tid; i < p.next_len; i += NT)
+            p.next_state[i] = stream_sample(p.consumed + i, p.state_len, p.n_in, [&](int j) { return p.state[j]; },
+                                            [&](int j) { return RAW ? load_raw(p, j) : p.in[j]; });
     }
 
     // ------------------------------------------------------------------ 1. filter bank
@@ -500,12 +493,8 @@ __global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
                     const size_t zstep = (size_t)R1 * p.osc_ring_len;
 #pragma unroll
                     for (int k2 = 0; k2 < R2; k2++) {
-                        const float2 z = __ldg(zp);
-                        const float vx = __fmul_rn(a[k2].x, inv), vy = __fmul_rn(a[k2].y, inv);
-                        float2 v;
-                        v.x = __fmul_rn(__fsub_rn(__fmul_rn(vx, z.x), __fmul_rn(vy, z.y)), g);
-                        v.y = __fmul_rn(__fadd_rn(__fmul_rn(vy, z.x), __fmul_rn(vx, z.y)), g);
-                        *reinterpret_cast<float2 *>(o) = v;
+                        const float2 m = mix_complex(make_float2(__fmul_rn(a[k2].x, inv), __fmul_rn(a[k2].y, inv)), __ldg(zp));
+                        *reinterpret_cast<float2 *>(o) = make_float2(__fmul_rn(m.x, g), __fmul_rn(m.y, g));
                         o += ostep;
                         zp += zstep;
                     }
@@ -588,205 +577,6 @@ __global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Post-processing of the "special" output channels, in place on their rows, one warp per channel:
-//   two-bin channels  TwoChannelOutputProcessor.process + TwoChannelSynthesizerM2.process + FS4DownConverter
-//                     (J/dsp/filter/channelizer/output/TwoChannelOutputProcessor.java:98-121,
-//                      J/dsp/filter/channelizer/TwoChannelSynthesizerM2.java:90-158, J/dsp/mixer/FS4DownConverter.java:32-68)
-//   frequency offset  Oscillator mix (J/dsp/mixer/Oscillator.java:42-68, AbstractOscillator.java:102-116): the rotator
-//                     is a float recursion with fastNormalize, so it runs as a sequential chain that every lane
-//                     walks, lane i keeping the value of sample i
-//   gain              ReusableComplexBuffer.applyGain: samples[x] = (float)(samples[x] * (double) gain)
-// The pfb kernels leave these rows at gain 1 (bin values after the 1/M of the inverse FFT).
-// ---------------------------------------------------------------------------------------------------------------
-constexpr int kMaxSynthEntries = 32;   // serpentine entries (4 floats each): filter.length / 2
-
-struct PostChannel {
-    int row, row2;          // output row; scratch row of the second bin (-1 for one-bin channels)
-    int mix;                // oscillator enabled
-    float angle_i, angle_q; // Oscillator: Complex.fromAngle((float)(2 pi f / fs))
-    double gain;
-};
-
-struct PostState {
-    float cur_i, cur_q;     // Oscillator current vector, starts at (0, -1)
-    int top_block, fs4;
-    float4 hist[kMaxSynthEntries];  // the newest serpentine entries, oldest first
-};
-
-struct SynthFilter {
-    float f[4 * kMaxSynthEntries];  // taps duplicated for I and Q (TwoChannelSynthesizerM2.init)
-    int entries;                     // len / 4
-};
-
-__global__ void __launch_bounds__(32) post_channel_kernel(float *out, long long out_stride, const float *out2,
-                                                          long long out2_stride, int n, const PostChannel *chans,
-                                                          PostState *states, const __grid_constant__ SynthFilter filt)
-{
-    __shared__ float4 ent[kMaxSynthEntries + 32];
-    const int lane = threadIdx.x;
-    const PostChannel c = chans[blockIdx.x];
-    PostState *st = states + blockIdx.x;
-    float2 *row = reinterpret_cast<float2 *>(out + (size_t)c.row * out_stride);
-    const float2 *row2 = c.row2 >= 0 ? reinterpret_cast<const float2 *>(out2 + (size_t)c.row2 * out2_stride) : nullptr;
-    const int H = filt.entries - 1;   // history entries a sample needs besides its own
-    float cur_i = st->cur_i, cur_q = st->cur_q;
-    const int top0 = st->top_block, fs40 = st->fs4;
-    if (row2)
-        for (int i = lane; i < H; i += 32) ent[i] = st->hist[i];
-    __syncwarp();
-    for (int base = 0; base < n; base += 32) {
-        const int k = base + lane;
-        const bool valid = k < n;
-        float2 v = valid ? row[k] : make_float2(0.f, 0.f);
-        if (row2) {
-            const float2 b = valid ? row2[k] : make_float2(0.f, 0.f);
-            // FloatFFT_1D(2).complexInverse(buffer, true): butterfly, then * 1/2
-            const float i0 = __fmul_rn(__fadd_rn(v.x, b.x), 0.5f), i1 = __fmul_rn(__fadd_rn(v.y, b.y), 0.5f);
-            const float i2 = __fmul_rn(__fsub_rn(v.x, b.x), 0.5f), i3 = __fmul_rn(__fsub_rn(v.y, b.y), 0.5f);
-            const bool top = ((top0 ^ k) & 1) != 0;   // mTopBlockIndicator toggles per sample
-            ent[H + lane] = top ? make_float4(i0, i1, i2, i3) : make_float4(i2, i3, i0, i1);
-            __syncwarp();
-            // product[y] = serpentine[y] * filter[y]; accumulators sum the I / Q lanes in index order
-            float acc_i = 0.0f, acc_q = 0.0f;
-            for (int j = 0; j < filt.entries; j++) {
-                const float4 e = ent[H + lane - j];
-                const float p0 = __fmul_rn(e.x, filt.f[4 * j]), p1 = __fmul_rn(e.y, filt.f[4 * j + 1]);
-                const float p2 = __fmul_rn(e.z, filt.f[4 * j + 2]), p3 = __fmul_rn(e.w, filt.f[4 * j + 3]);
-                acc_i = __fadd_rn(__fadd_rn(acc_i, p0), p2);
-                acc_q = __fadd_rn(__fadd_rn(acc_q, p1), p3);
-            }
-            // FS4DownConverter: multiply by (-j)^pointer
-            switch ((fs40 + k) & 3) {
-                case 1: v = make_float2(acc_q, -acc_i); break;
-                case 2: v = make_float2(-acc_i, -acc_q); break;
-                case 3: v = make_float2(-acc_q, acc_i); break;
-                default: v = make_float2(acc_i, acc_q); break;
-            }
-            __syncwarp();
-            // keep the newest H entries for the next 32 samples
-            const int count = min(32, n - base);
-            float4 keep = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (lane < H) keep = ent[count + lane];
-            __syncwarp();
-            if (lane < H) ent[lane] = keep;
-            __syncwarp();
-        }
-        if (c.mix) {
-            // AbstractOscillator.mixComplex: sample * current, then rotate(): current *= angle, fastNormalize
-            float my_i = cur_i, my_q = cur_q;
-            const int count = min(32, n - base);
-            for (int i = 0; i < count; i++) {
-                if (i == lane) {
-                    my_i = cur_i;
-                    my_q = cur_q;
-                }
-                const float ni = __fsub_rn(__fmul_rn(cur_i, c.angle_i), __fmul_rn(cur_q, c.angle_q));
-                const float nq = __fadd_rn(__fmul_rn(cur_q, c.angle_i), __fmul_rn(cur_i, c.angle_q));
-                const float norm = __fadd_rn(__fmul_rn(ni, ni), __fmul_rn(nq, nq));
-                const float scalor = __fsub_rn(1.9999f, norm);
-                cur_i = __fmul_rn(ni, scalor);
-                cur_q = __fmul_rn(nq, scalor);
-            }
-            const float mi = __fsub_rn(__fmul_rn(v.x, my_i), __fmul_rn(v.y, my_q));
-            const float mq = __fadd_rn(__fmul_rn(v.y, my_i), __fmul_rn(v.x, my_q));
-            v = make_float2(mi, mq);
-        }
-        v.x = __double2float_rn(__dmul_rn((double)v.x, c.gain));
-        v.y = __double2float_rn(__dmul_rn((double)v.y, c.gain));
-        if (valid) row[k] = v;
-    }
-    if (lane == 0) {
-        st->cur_i = cur_i;
-        st->cur_q = cur_q;
-        st->top_block = (top0 ^ n) & 1;
-        st->fs4 = (fs40 + n) & 3;
-    }
-    if (row2)
-        for (int i = lane; i < H; i += 32) st->hist[i] = ent[i];
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// One-bin channels with a frequency offset (the usual case: a requested channel frequency is rarely the centre of its
-// polyphase bin).  The oscillator is a float recursion -- rotate by the angle, fastNormalize -- that is neutrally stable
-// in phase: two runs never merge, so unlike the Airspy DC filter it cannot be cut into speculative segments, and one
-// chain step costs 44 cycles (12 fma-pipe instructions): 1.1 ms per 50 000-sample row, 14 x the whole polyphase
-// kernel.  But the values do not depend on the samples.  osc_produce_kernel therefore runs AHEAD: after every call it
-// tops a per-channel ring up to one call's worth of oscillator values on a side stream, one thread per channel, while
-// the caller's FIR / demodulator kernels run; the call itself only does the element-wise osc_mix_kernel.
-// (AbstractOscillator.mixComplex, J/dsp/mixer/AbstractOscillator.java:102-116: sample * current, then rotate();
-// Oscillator.rotate + Complex.fastNormalize, J/dsp/mixer/Oscillator.java:42-68.)
-// ---------------------------------------------------------------------------------------------------------------
-struct MixChannel {
-    int row;
-    float angle_i, angle_q;
-    double gain;
-};
-
-__global__ void __launch_bounds__(32) osc_produce_kernel(const MixChannel *__restrict__ chans, float2 *__restrict__ state,
-                                                           float2 *__restrict__ ring, int ring_len, long long start, int count,
-                                                           int n_mix)
-{
-    const int ch = blockIdx.x * blockDim.x + threadIdx.x;
-    if (ch >= n_mix) return;
-    const float angle_i = chans[ch].angle_i, angle_q = chans[ch].angle_q;
-    float cur_i = state[ch].x, cur_q = state[ch].y;
-    float2 *r = ring + (size_t)ch * ring_len;
-    int pos = (int)(start % ring_len);
-#define SDRGPU_OSC_ROTATE()                                                                        \
-    {                                                                                              \
-        const float ni = __fsub_rn(__fmul_rn(cur_i, angle_i), __fmul_rn(cur_q, angle_q));          \
-        const float nq = __fadd_rn(__fmul_rn(cur_q, angle_i), __fmul_rn(cur_i, angle_q));          \
-        const float scalor = __fsub_rn(1.9999f, __fadd_rn(__fmul_rn(ni, ni), __fmul_rn(nq, nq)));  \
-        cur_i = __fmul_rn(ni, scalor);                                                             \
-        cur_q = __fmul_rn(nq, scalor);                                                             \
-    }
-    int k = 0;
-    while (k < count) {
-        if ((pos & 1) == 0 && k + 8 <= count && pos + 8 <= ring_len) {
-            // eight steps with nothing but the recursion between them, then four 16-byte stores (ring_len is even and
-            // the rows are 16-byte aligned)
-            float4 w[4];
-#pragma unroll
-            for (int j = 0; j < 4; j++) {
-                w[j].x = cur_i;
-                w[j].y = cur_q;
-                SDRGPU_OSC_ROTATE()
-                w[j].z = cur_i;
-                w[j].w = cur_q;
-                SDRGPU_OSC_ROTATE()
-            }
-#pragma unroll
-            for (int j = 0; j < 4; j++) reinterpret_cast<float4 *>(r + pos)[j] = w[j];
-            pos += 8;
-            k += 8;
-        } else {
-            r[pos] = make_float2(cur_i, cur_q);
-            SDRGPU_OSC_ROTATE()
-            pos += 1;
-            k += 1;
-        }
-        if (pos >= ring_len) pos = 0;
-    }
-#undef SDRGPU_OSC_ROTATE
-    state[ch] = make_float2(cur_i, cur_q);
-}
-
-// grid (ceil(n / 256), n_mix): row[k] = (float)((double)(row[k] * osc[start + k]) * gain)
-__global__ void osc_mix_kernel(float *out, long long out_stride, const MixChannel *__restrict__ chans,
-                               const float2 *__restrict__ ring, int ring_len, long long start, int n)
-{
-    const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= n) return;
-    const MixChannel c = chans[blockIdx.y];
-    float2 *row = reinterpret_cast<float2 *>(out + (size_t)c.row * out_stride);
-    const float2 v = row[k];
-    const float2 z = ring[(size_t)blockIdx.y * ring_len + (int)((start + k) % ring_len)];
-    const float mi = __fsub_rn(__fmul_rn(v.x, z.x), __fmul_rn(v.y, z.y));
-    const float mq = __fadd_rn(__fmul_rn(v.y, z.x), __fmul_rn(v.x, z.y));
-    row[k] = make_float2(__double2float_rn(__dmul_rn((double)mi, c.gain)), __double2float_rn(__dmul_rn((double)mq, c.gain)));
-}
-
-// ---------------------------------------------------------------------------------------------------------------
 // tuner sample converters (ByteSampleConverter / SignedByteSampleConverter lookup tables, ConversionUtils 16-bit)
 // ---------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float convert_value(int format, const void *src, size_t i)
@@ -804,18 +594,25 @@ __global__ void convert_kernel(int format, const void *__restrict__ src, float *
         dst[i] = convert_value(format, src, i);
 }
 
-// new_state[i] = S[consumed + i], S = [state | in]
+// new_state[i] = S[consumed + i], S = [state | in | zeros]
 __global__ void save_state_kernel(const float2 *state, int state_len, const float2 *in, int n_in, int consumed,
                                   float2 *new_state, int new_len)
 {
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < new_len; i += gridDim.x * blockDim.x) {
-        int idx = consumed + i;
-        float2 v = make_float2(0.0f, 0.0f);
-        if (idx < state_len) v = state[idx];
-        else if (idx - state_len < n_in) v = in[idx - state_len];
-        new_state[i] = v;
-    }
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < new_len; i += gridDim.x * blockDim.x)
+        new_state[i] = stream_sample(consumed + i, state_len, n_in, [&](int j) { return state[j]; }, [&](int j) { return in[j]; });
 }
+
+// L2 read-ahead distance of pfb2_kernel in blocks: two 8-block tiles for each of the 148 SMs of a B200, the measured
+// optimum (half a wave of the M = 400 kernel at 4 CTAs per SM, two thirds of one of the M = 800 kernel at 3)
+constexpr int kPfbPrefetchBlocks = 148 * 8 * 2;
+
+// One pfb2_kernel shape: M = R1 x R2 channels, NB blocks per tile, NT threads, at least MINB CTAs per SM.  f32 launches
+// the instance for float input; raw, if there is one, the instance that reads 8-bit tuner samples and converts on load.
+using PfbLauncher = sdrgpu_status (*)(const sdrgpu_channelizer *h, const ChanParams &p);
+struct PfbRow {
+    int M, R1, R2, NB, NT, MINB;
+    PfbLauncher f32, raw;
+};
 
 }  // namespace
 
@@ -826,8 +623,8 @@ struct sdrgpu_channelizer {
     int max_in_complex = 0, max_blocks = 0;
     int leftover = 0, parity0 = 0;
     bool throttled = false;   // chan_set_throttled: the pipeline is overlapping this launch with the demodulator
-    // chan_convert leaves 8-bit tuner samples unconverted for chan_enqueue: the M = 400 / 800 filter bank converts them on
-    // load (no float copy of the input in HBM); anything else converts them with convert_kernel first
+    // chan_convert leaves 8-bit tuner samples unconverted for chan_enqueue when the filter bank converts them on load (no
+    // float copy of the input in HBM, converts_on_load); otherwise convert_kernel converts them first
     const uint8_t *defer_src = nullptr;
     const float2 *defer_dst = nullptr;
     int defer_n = 0;
@@ -845,7 +642,7 @@ struct sdrgpu_channelizer {
     float *d_taps = nullptr;
     float2 *d_tw = nullptr;
     float2 *d_tw2 = nullptr;   // pfb2_kernel inter-step twiddles
-    int fast_r1 = 0, fast_r2 = 0;  // factors of the pfb2 fast path (0 = generic kernel)
+    const PfbRow *fast = nullptr;   // the pfb2_kernel row of this channel count (nullptr: pfb_ifft_kernel)
     float2 *d_state[2] = {nullptr, nullptr};
     int cur_state = 0;
     float2 *d_in = nullptr;    // staging for host input (float I/Q)
@@ -866,21 +663,7 @@ struct sdrgpu_channelizer {
     double *d_gain_d = nullptr;
     double sample_rate = 0.0;          // tuner sample rate (Hz); needed for frequency-corrected channels
     int n_rows = 0;                    // rows the pfb kernel writes: n_sel output rows + scratch rows of second bins
-    int n_post = 0;                    // special channels (two-bin and / or frequency offset)
-    PostChannel *d_post = nullptr;
-    PostState *d_post_state = nullptr;
-    float *d_out2 = nullptr;           // scratch rows [n_rows - n_sel][2 * max_blocks]
-    // one-bin frequency-corrected channels: oscillator values produced ahead of use (osc_produce_kernel)
-    int n_mix = 0, osc_ring_len = 0;
-    MixChannel *d_mix = nullptr;
-    float2 *d_mix_state = nullptr;     // oscillator vector at the producer's position
-    float2 *d_osc = nullptr;           // [n_mix][osc_ring_len]
-    long long osc_produced = 0, osc_consumed = 0, osc_safe = 0;   // osc_safe: produced by launches already waited for
-    cudaStream_t osc_stream = nullptr;
-    cudaEvent_t ev_mix = nullptr, ev_osc = nullptr;
-    bool osc_pending = false;
-    bool mix_recorded = false;   // ev_mix marks the end of the last kernel that read the rings
-    SynthFilter synth{};
+    ChanOutputs outputs;               // two-bin and frequency-corrected channels (outputs.cu)
     int gain_exact = 1;
     int identity = 0;
     float gain_uniform = 0.0f;
@@ -895,118 +678,40 @@ namespace {
 
 sdrgpu_status upload_selection(sdrgpu_channelizer *h)
 {
-    const int n = (int)h->channels.size();
-    std::vector<int> sel;
-    std::vector<float> gf;
-    std::vector<double> gd;
-    std::vector<PostChannel> post;
-    std::vector<MixChannel> mix;
-    int exact = 1, n_two = 0;
-    for (int i = 0; i < n; i++) {
-        const sdrgpu_output_channel &c = h->channels[i];
-        const bool special = c.bin2 >= 0 || c.frequency_offset_hz != 0;
-        sel.push_back(c.bin1);
-        // special rows leave the pfb kernel at gain 1; post_channel_kernel applies the gain after mixing
-        gd.push_back(special ? 1.0 : c.gain);
-        gf.push_back((float)gd.back());
-        if ((double)gf.back() != gd.back()) exact = 0;
-        if (special) {
-            PostChannel pc{};
-            pc.row = i;
-            pc.row2 = c.bin2 >= 0 ? n_two++ : -1;
-            // TwoChannelOutputProcessor mixes unconditionally, OneChannelOutputProcessor only with an offset
-            pc.mix = 1;
-            // Oscillator.update: anglePerSample = (float)(2 pi f / fs); Complex.fromAngle(float) -> (float)cos, (float)sin
-            const double channel_rate = 2.0 * h->sample_rate / (double)h->M;
-            const float angle = (float)(2.0 * 3.14159265358979323846 * (double)c.frequency_offset_hz / channel_rate);
-            pc.angle_i = (float)cos((double)angle);
-            pc.angle_q = (float)sin((double)angle);
-            pc.gain = c.gain;
-            if (c.bin2 >= 0) post.push_back(pc);                                        // two-bin: post_channel_kernel
-            else mix.push_back(MixChannel{pc.row, pc.angle_i, pc.angle_q, pc.gain});    // one bin + offset: look-ahead
-        }
+    OutputRows r;
+    SDRGPU_TRY(outputs_select(h->outputs, h->channels, h->M, h->sample_rate, h->max_blocks, &r));
+    const int n = (int)h->channels.size(), rows = (int)r.sel.size();
+    std::vector<float> gf(rows);
+    int exact = 1;
+    for (int i = 0; i < rows; i++) {
+        gf[i] = (float)r.gain[i];
+        if ((double)gf[i] != r.gain[i]) exact = 0;
     }
-    for (int i = 0; i < n; i++)
-        if (h->channels[i].bin2 >= 0) {   // scratch rows: the second bins, gain 1
-            sel.push_back(h->channels[i].bin2);
-            gd.push_back(1.0);
-            gf.push_back(1.0f);
-        }
-    const int rows = (int)sel.size();
-    h->mix_identity = (int)mix.size() == n && n == h->M && rows == n;
-    for (size_t m = 0; m < mix.size() && h->mix_identity; m++)
-        if (mix[m].row != (int)m || sel[m] != (int)m || mix[m].gain != mix[0].gain || (double)(float)mix[m].gain != mix[m].gain)
-            h->mix_identity = 0;
-    h->mix_gain = mix.empty() ? 0.0f : (float)mix[0].gain;
     cudaFree(h->d_sel);
     cudaFree(h->d_gain_f);
     cudaFree(h->d_gain_d);
-    cudaFree(h->d_post);
-    cudaFree(h->d_post_state);
-    cudaFree(h->d_out2);
-    if (h->osc_stream) SDRGPU_CUDA(cudaStreamSynchronize(h->osc_stream));
-    cudaFree(h->d_mix);
-    cudaFree(h->d_mix_state);
-    cudaFree(h->d_osc);
-    h->d_mix = nullptr;
-    h->d_mix_state = nullptr;
-    h->d_osc = nullptr;
-    h->osc_produced = h->osc_consumed = h->osc_safe = 0;
-    h->osc_pending = false;
     h->d_sel = nullptr;
     h->d_gain_f = nullptr;
     h->d_gain_d = nullptr;
-    h->d_post = nullptr;
-    h->d_post_state = nullptr;
-    h->d_out2 = nullptr;
     SDRGPU_CUDA(cudaMalloc(&h->d_sel, sizeof(int) * (size_t)rows));
     SDRGPU_CUDA(cudaMalloc(&h->d_gain_f, sizeof(float) * (size_t)rows));
     SDRGPU_CUDA(cudaMalloc(&h->d_gain_d, sizeof(double) * (size_t)rows));
-    SDRGPU_CUDA(cudaMemcpy(h->d_sel, sel.data(), sizeof(int) * (size_t)rows, cudaMemcpyHostToDevice));
+    SDRGPU_CUDA(cudaMemcpy(h->d_sel, r.sel.data(), sizeof(int) * (size_t)rows, cudaMemcpyHostToDevice));
     SDRGPU_CUDA(cudaMemcpy(h->d_gain_f, gf.data(), sizeof(float) * (size_t)rows, cudaMemcpyHostToDevice));
-    SDRGPU_CUDA(cudaMemcpy(h->d_gain_d, gd.data(), sizeof(double) * (size_t)rows, cudaMemcpyHostToDevice));
-    if (!post.empty()) {
-        std::vector<PostState> init(post.size());
-        std::memset(init.data(), 0, sizeof(PostState) * init.size());
-        for (auto &st : init) {
-            st.cur_i = 0.0f;   // Oscillator.java:24: mCurrentAngle = new Complex(0.0f, -1.0f)
-            st.cur_q = -1.0f;
-            st.top_block = 1;  // TwoChannelSynthesizerM2: mTopBlockIndicator = true
-        }
-        SDRGPU_CUDA(cudaMalloc(&h->d_post, sizeof(PostChannel) * post.size()));
-        SDRGPU_CUDA(cudaMalloc(&h->d_post_state, sizeof(PostState) * post.size()));
-        SDRGPU_CUDA(cudaMemcpy(h->d_post, post.data(), sizeof(PostChannel) * post.size(), cudaMemcpyHostToDevice));
-        SDRGPU_CUDA(cudaMemcpy(h->d_post_state, init.data(), sizeof(PostState) * init.size(), cudaMemcpyHostToDevice));
-    }
-    if (n_two > 0) SDRGPU_CUDA(cudaMalloc(&h->d_out2, sizeof(float) * 2 * (size_t)h->max_blocks * (size_t)n_two));
-    if (!mix.empty()) {
-        if (!h->osc_stream) {
-            SDRGPU_CUDA(cudaStreamCreateWithFlags(&h->osc_stream, cudaStreamNonBlocking));
-            SDRGPU_CUDA(cudaEventCreateWithFlags(&h->ev_mix, cudaEventDisableTiming));
-            SDRGPU_CUDA(cudaEventCreateWithFlags(&h->ev_osc, cudaEventDisableTiming));
-        }
-        // two calls' worth: a pipeline tops the ring up at the START of a call, for the call after it (chan_osc_ahead)
-        h->osc_ring_len = (2 * h->max_blocks + 8 + 1) & ~1;   // even: the producer stores pairs
-        std::vector<float2> start(mix.size(), make_float2(0.0f, -1.0f));   // Oscillator.java:24
-        SDRGPU_CUDA(cudaMalloc(&h->d_mix, sizeof(MixChannel) * mix.size()));
-        SDRGPU_CUDA(cudaMalloc(&h->d_mix_state, sizeof(float2) * mix.size()));
-        SDRGPU_CUDA(cudaMalloc(&h->d_osc, sizeof(float2) * mix.size() * (size_t)h->osc_ring_len));
-        SDRGPU_CUDA(cudaMemcpy(h->d_mix, mix.data(), sizeof(MixChannel) * mix.size(), cudaMemcpyHostToDevice));
-        SDRGPU_CUDA(cudaMemcpy(h->d_mix_state, start.data(), sizeof(float2) * mix.size(), cudaMemcpyHostToDevice));
-    }
-    h->n_mix = (int)mix.size();
+    SDRGPU_CUDA(cudaMemcpy(h->d_gain_d, r.gain.data(), sizeof(double) * (size_t)rows, cudaMemcpyHostToDevice));
+    h->mix_identity = r.mix_identity;
+    h->mix_gain = r.mix_gain;
     h->n_sel = n;
     h->n_rows = rows;
-    h->n_post = (int)post.size();
     h->gain_exact = exact;
-    h->identity = exact && n == h->M && post.empty() && mix.empty();
+    h->identity = exact && n == h->M && h->outputs.n_post == 0 && h->outputs.n_mix == 0;
     for (int i = 0; i < n && h->identity; i++)
-        if (sel[i] != i || gf[i] != gf[0]) h->identity = 0;
+        if (r.sel[i] != i || gf[i] != gf[0]) h->identity = 0;
     h->gain_uniform = n > 0 ? gf[0] : 0.0f;
     return SDRGPU_OK;
 }
 
-template <int M, int R1, int R2, int NB, int TT, int NT, int MINB, bool RAW = false>
+template <int M, int R1, int R2, int NB, int TT, int NT, int MINB, bool RAW>
 sdrgpu_status launch_pfb2(const sdrgpu_channelizer *h, const ChanParams &p)
 {
     using L = Pfb2Layout<M, R1, R2, NB, TT, NT>;
@@ -1033,6 +738,45 @@ sdrgpu_status launch_pfb(const sdrgpu_channelizer *h, const ChanParams &p, int g
     SDRGPU_CUDA(cudaGetLastError());
     return SDRGPU_OK;
 }
+
+template <int M, int R1, int R2, int NB, int NT, int MINB, bool RAW>
+constexpr PfbRow pfb_row()
+{
+    PfbRow row{M, R1, R2, NB, NT, MINB, launch_pfb2<M, R1, R2, NB, 9, NT, MINB, false>, nullptr};
+    if constexpr (RAW) row.raw = launch_pfb2<M, R1, R2, NB, 9, NT, MINB, true>;
+    return row;
+}
+
+// The pfb2_kernel instances: the channel counts of the common tuner rates (25 kHz channels: 2 / 2.4 / 2.5 / 3 / 4 / 5 / 6 /
+// 8 / 10 / 16 / 20 MS/s) with the reference's 9 taps per channel.  Tile shapes measured on a B200 (profiles/): M = 400 runs
+// best as 8-block tiles, 200 threads, 4 CTAs per SM; M = 800 as 8-block tiles, 256 threads, 3 CTAs per SM.  8-block tiles
+// store a default selection straight from step B (and mix the oscillators in there, fused_mix in chan_enqueue).
+constexpr PfbRow kPfbRows[] = {
+    pfb_row<400, 20, 20, 8, 200, 4, true>(),
+    pfb_row<800, 32, 25, 8, 256, 3, true>(),
+    pfb_row<96, 8, 12, 16, 192, 2, false>(),
+    pfb_row<640, 32, 20, 8, 320, 2, false>(),
+    pfb_row<320, 16, 20, 8, 160, 4, false>(),
+    pfb_row<240, 12, 20, 8, 160, 4, false>(),
+    pfb_row<200, 10, 20, 8, 160, 4, false>(),
+    pfb_row<160, 8, 20, 8, 160, 4, false>(),
+    pfb_row<120, 10, 12, 16, 192, 2, false>(),
+    pfb_row<100, 10, 10, 16, 160, 2, false>(),
+    pfb_row<80, 8, 10, 16, 160, 2, false>(),
+};
+
+// The filter bank and inverse DFT of one call: the handle's pfb2_kernel row (its 8-bit instance if raw), else
+// pfb_ifft_kernel.
+sdrgpu_status pfb_launch(const sdrgpu_channelizer *h, const ChanParams &p, bool raw)
+{
+    if (h->fast) return (raw ? h->fast->raw : h->fast->f32)(h, p);
+    const int grid = (p.n_blocks + h->NB - 1) / h->NB;
+    if (h->NB == 16) return h->T == 9 ? launch_pfb<16, 9>(h, p, grid) : launch_pfb<16, 0>(h, p, grid);
+    return h->T == 9 ? launch_pfb<8, 9>(h, p, grid) : launch_pfb<8, 0>(h, p, grid);
+}
+
+// whether the filter bank reads 8-bit tuner samples as they are
+bool converts_on_load(const sdrgpu_channelizer *h) { return h->fast && h->fast->raw; }
 
 }  // namespace
 
@@ -1065,46 +809,25 @@ sdrgpu_status sdrgpu::chan_enqueue(sdrgpu_channelizer *h, const float2 *d_in, in
     // 8-bit samples chan_convert left unconverted: the filter bank reads them as they are when it runs, else convert now
     const uint8_t *raw = (h->defer_src && d_in == h->defer_dst && n_in == h->defer_n) ? h->defer_src : nullptr;
     h->defer_src = nullptr;
-    const bool fuse_convert = raw && n_blocks > 0 && h->fast_r1 && (h->M == 400 || h->M == 800);
+    const bool fuse_convert = raw && n_blocks > 0 && converts_on_load(h);
     if (raw && !fuse_convert) launch_convert(h, raw, const_cast<float2 *>(d_in), n_in);
+    ChanOutputs &o = h->outputs;
     // checked before anything is launched or the framing state advances: a failing call leaves the handle as it was
-    if (n_blocks > 0 && (h->n_mix > 0 || h->n_post > 0)) {
+    if (n_blocks > 0 && (o.n_mix > 0 || o.n_post > 0)) {
         // The reference rotates every channel's mixer for every buffer; the results layout has no per-channel rows to
         // mix, and skipping the oscillators would leave them out of step with the sample stream for later calls.
         if (layout != SDRGPU_LAYOUT_CHANNELS)
             return fail(SDRGPU_ERR_BAD_STATE, "two-bin / frequency-corrected channels are selected: use SDRGPU_LAYOUT_CHANNELS");
-        if (h->n_mix > 0 && n_blocks > h->osc_ring_len)
+        if (o.n_mix > 0 && n_blocks > o.osc_ring_len)
             return fail(SDRGPU_ERR_OVERFLOW, "%d blocks exceed the oscillator look-ahead", n_blocks);
     }
     // Frequency-corrected one-bin channels: the oscillator values come from the look-ahead rings (osc_produce_kernel on a
-    // side stream).  When every bin is such a channel pfb2_kernel multiplies them in where it stores the rows (no separate
-    // pass over the channel streams); otherwise the rows leave the kernel at gain 1 and osc_mix_kernel finishes them.
-    static const int fuse_mix_env = getenv("SDRGPU_FUSE_MIX") ? atoi(getenv("SDRGPU_FUSE_MIX")) : 1;
-    // (pfb2_kernel instances with 8-block tiles store straight from step B: M = 160 ... 800, see the launch table below)
-    const bool direct_store = h->fast_r1 && (h->M == 800 || h->M == 640 || h->M == 400 || h->M == 320 || h->M == 240 ||
-                                             h->M == 200 || h->M == 160);
-    const bool fused_mix = fuse_mix_env && h->n_mix > 0 && h->mix_identity && direct_store &&
-                           layout == SDRGPU_LAYOUT_CHANNELS && n_blocks > 0;
-    auto ensure_osc = [&]() -> sdrgpu_status {
-        const int pgrid = (h->n_mix + 31) / 32;
-        const long long have = h->osc_produced - h->osc_consumed;
-        // wait for the top-up in flight only if this call reaches into what it writes (or has to produce itself)
-        if (h->osc_pending && (h->osc_consumed + n_blocks > h->osc_safe || have < n_blocks)) {
-            SDRGPU_CUDA(cudaStreamWaitEvent(h->stream, h->ev_osc, 0));
-            h->osc_pending = false;
-            h->osc_safe = h->osc_produced;
-        }
-        if (have < n_blocks) {  // first call, or a call longer than the look-ahead: produce the rest in line
-            osc_produce_kernel<<<pgrid, 32, 0, h->stream>>>(h->d_mix, h->d_mix_state, h->d_osc, h->osc_ring_len,
-                                                           h->osc_produced, (int)(n_blocks - have), h->n_mix);
-            h->osc_produced += n_blocks - have;
-            h->osc_safe = h->osc_produced;
-            count_launch();
-        }
-        return SDRGPU_OK;
-    };
+    // side stream).  When every bin is such a channel and the pfb2_kernel instance stores the rows straight from step B
+    // (8-block tiles), it multiplies them in there (no separate pass over the channel streams); otherwise the rows leave
+    // the kernel at gain 1 and osc_mix_kernel finishes them.
+    const bool fused_mix = o.n_mix > 0 && h->mix_identity && h->fast && h->fast->NB == 8 && layout == SDRGPU_LAYOUT_CHANNELS &&
+                           n_blocks > 0;
     if (n_blocks > 0) {
-        if (fused_mix) SDRGPU_TRY(ensure_osc());
         ChanParams p{};
         p.neg_zero = -0.0f;
         p.state = state;
@@ -1120,7 +843,7 @@ sdrgpu_status sdrgpu::chan_enqueue(sdrgpu_channelizer *h, const float2 *d_in, in
         p.gain_f = h->d_gain_f;
         p.gain_d = h->d_gain_d;
         p.out_stride = stride;
-        p.out2 = h->d_out2;
+        p.out2 = o.d_out2;
         p.out2_stride = 2LL * h->max_blocks;
         p.n_main = h->n_sel;
         p.state_len = state_len;
@@ -1135,11 +858,9 @@ sdrgpu_status sdrgpu::chan_enqueue(sdrgpu_channelizer *h, const float2 *d_in, in
         p.layout = layout;
         p.gain_exact = h->gain_exact;
         p.identity = fused_mix ? 1 : h->identity;   // (every bin in order, one gain: the direct store path, with the mix)
-        p.osc = fused_mix ? h->d_osc : nullptr;
-        p.osc_ring_len = h->osc_ring_len;
-        p.osc_start = fused_mix ? (int)(h->osc_consumed % h->osc_ring_len) : 0;
-        static const int pf_waves = getenv("SDRGPU_PFB_PREFETCH") ? atoi(getenv("SDRGPU_PFB_PREFETCH")) : 2;
-        p.prefetch_blocks = 148 * 8 * pf_waves;   // in quarter waves of 148 SMs x 4 CTAs x 8 blocks
+        p.osc_ring_len = o.osc_ring_len;
+        if (fused_mix) SDRGPU_TRY(outputs_before(o, n_blocks, h->stream, &p.osc, &p.osc_start));
+        p.prefetch_blocks = kPfbPrefetchBlocks;
         p.gain_uniform = fused_mix ? h->mix_gain : h->gain_uniform;
         p.inv_m = 1.0f / (float)h->M;
         p.n_factors = (int)h->factors.size();
@@ -1147,71 +868,17 @@ sdrgpu_status sdrgpu::chan_enqueue(sdrgpu_channelizer *h, const float2 *d_in, in
             p.factors[i] = h->factors[i];
             p.magic_s[i] = h->magic[i];
         }
-        const int grid = (n_blocks + h->NB - 1) / h->NB;
-        if (h->fast_r1 && n_in > 0) {
+        if (h->fast && n_in > 0) {
             p.next_state = next;
             p.next_len = new_len;
             p.consumed = consumed;
             state_saved = true;
         }
         h->timer.begin(h->stream);
-        sdrgpu_status st;
-        // tile sizes measured on B200 (profiles/): M = 400 runs best as 8-block tiles, 200 threads, 4 CTAs per SM; M = 800 as
-        // 8-block tiles, 256 threads, 3 CTAs per SM
-        if (fuse_convert && h->M == 400) st = launch_pfb2<400, 20, 20, 8, 9, 200, 4, true>(h, p);
-        else if (fuse_convert && h->M == 800) st = launch_pfb2<800, 32, 25, 8, 9, 256, 3, true>(h, p);
-        else if (h->fast_r1 && h->M == 400) st = launch_pfb2<400, 20, 20, 8, 9, 200, 4>(h, p);
-        else if (h->fast_r1 && h->M == 800) st = launch_pfb2<800, 32, 25, 8, 9, 256, 3>(h, p);
-        else if (h->fast_r1 && h->M == 96) st = launch_pfb2<96, 8, 12, 16, 9, 192, 2>(h, p);
-        else if (h->fast_r1 && h->M == 640) st = launch_pfb2<640, 32, 20, 8, 9, 320, 2>(h, p);
-        else if (h->fast_r1 && h->M == 320) st = launch_pfb2<320, 16, 20, 8, 9, 160, 4>(h, p);
-        else if (h->fast_r1 && h->M == 240) st = launch_pfb2<240, 12, 20, 8, 9, 160, 4>(h, p);
-        else if (h->fast_r1 && h->M == 200) st = launch_pfb2<200, 10, 20, 8, 9, 160, 4>(h, p);
-        else if (h->fast_r1 && h->M == 160) st = launch_pfb2<160, 8, 20, 8, 9, 160, 4>(h, p);
-        else if (h->fast_r1 && h->M == 120) st = launch_pfb2<120, 10, 12, 16, 9, 192, 2>(h, p);
-        else if (h->fast_r1 && h->M == 100) st = launch_pfb2<100, 10, 10, 16, 9, 160, 2>(h, p);
-        else if (h->fast_r1 && h->M == 80) st = launch_pfb2<80, 8, 10, 16, 9, 160, 2>(h, p);
-        else if (h->NB == 16) st = (h->T == 9) ? launch_pfb<16, 9>(h, p, grid) : launch_pfb<16, 0>(h, p, grid);
-        else st = (h->T == 9) ? launch_pfb<8, 9>(h, p, grid) : launch_pfb<8, 0>(h, p, grid);
+        const sdrgpu_status st = pfb_launch(h, p, fuse_convert);
         h->timer.end(h->stream);
         SDRGPU_TRY(st);
-        if (layout == SDRGPU_LAYOUT_CHANNELS && h->n_post > 0) {
-            post_channel_kernel<<<h->n_post, 32, 0, h->stream>>>(d_out, stride, h->d_out2, 2LL * h->max_blocks, n_blocks, h->d_post,
-                                                                 h->d_post_state, h->synth);
-            count_launch();
-            SDRGPU_CUDA(cudaGetLastError());
-        }
-        if (layout == SDRGPU_LAYOUT_CHANNELS && h->n_mix > 0) {
-            if (!fused_mix) {
-                SDRGPU_TRY(ensure_osc());
-                osc_mix_kernel<<<dim3((n_blocks + 255) / 256, h->n_mix), 256, 0, h->stream>>>(d_out, stride, h->d_mix, h->d_osc,
-                                                                                              h->osc_ring_len, h->osc_consumed, n_blocks);
-                count_launch();
-            }
-            h->osc_consumed += n_blocks;
-            SDRGPU_CUDA(cudaEventRecord(h->ev_mix, h->stream));
-            h->mix_recorded = true;
-            // top the ring up to a call's worth on the side stream, behind the kernel that has just read it
-            const int pgrid = (h->n_mix + 31) / 32;
-            const int top_up = h->max_blocks - (int)(h->osc_produced - h->osc_consumed);
-            if (top_up > 0) {
-                SDRGPU_CUDA(cudaStreamWaitEvent(h->osc_stream, h->ev_mix, 0));
-                // Round 1 kept other blocks off the producer's SMs by asking for 220 KB of shared memory it never touched
-                // (SDRGPU_OSC_EXCLUSIVE=1 still does); that only worked for one pipeline per GPU and starves everything else
-                // once several tuners share the device, so the producer is an ordinary small kernel on its side stream and
-                // the cost is reported as measured (bench.py: with_frequency_corrected_channels).
-                static const int exclusive = getenv("SDRGPU_OSC_EXCLUSIVE") ? atoi(getenv("SDRGPU_OSC_EXCLUSIVE")) : 0;
-                const int smem = (exclusive && pgrid <= 16) ? 220 * 1024 : 0;
-                if (smem) SDRGPU_CUDA(cudaFuncSetAttribute(osc_produce_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-                osc_produce_kernel<<<pgrid, 32, smem, h->osc_stream>>>(h->d_mix, h->d_mix_state, h->d_osc, h->osc_ring_len,
-                                                                       h->osc_produced, top_up, h->n_mix);
-                SDRGPU_CUDA(cudaEventRecord(h->ev_osc, h->osc_stream));
-                h->osc_produced += top_up;
-                h->osc_pending = true;
-                count_launch();
-            }
-            SDRGPU_CUDA(cudaGetLastError());
-        }
+        if (layout == SDRGPU_LAYOUT_CHANNELS) SDRGPU_TRY(outputs_after(o, d_out, stride, n_blocks, fused_mix, h->stream));
     }
     // carry the history + leftover over to the next call
     if (n_in > 0) {
@@ -1271,8 +938,7 @@ const float2 *sdrgpu::chan_convert(sdrgpu_channelizer *h, const void *iq_device,
             return nullptr;
     } else if (n > 0) {
         const bool eight_bit = h->in_format == SDRGPU_FORMAT_U8 || h->in_format == SDRGPU_FORMAT_S8;
-        static const int fuse_env = getenv("SDRGPU_FUSE_CONVERT") ? atoi(getenv("SDRGPU_FUSE_CONVERT")) : 1;
-        if (fuse_env && eight_bit && h->fast_r1 && (h->M == 400 || h->M == 800)) {
+        if (eight_bit && converts_on_load(h)) {
             h->defer_src = src + cb * first;
             h->defer_dst = h->d_in + first;
             h->defer_n = n;
@@ -1282,34 +948,9 @@ const float2 *sdrgpu::chan_convert(sdrgpu_channelizer *h, const void *iq_device,
     }
     return h->d_in + first;
 }
-// Oscillator look-ahead of a pipeline: at the START of a call (before its channelizer kernels) the rings are topped up to
-// two calls' worth, i.e. the values of the NEXT call are produced beside this call's channelizer / first FIR launches --
-// throughput-bound kernels that lose little to 200 latency-bound warps -- instead of behind them, beside the demodulator,
-// whose launch time is set by its most loaded scheduler (8 tuners, all 6400 channels corrected: 9.1 -> see DESIGN.md).
-sdrgpu_status sdrgpu::chan_osc_ahead(sdrgpu_channelizer *h)
-{
-    static const int ahead_env = getenv("SDRGPU_OSC_AHEAD") ? atoi(getenv("SDRGPU_OSC_AHEAD")) : 1;
-    if (!ahead_env || h->n_mix <= 0 || !h->d_osc) return SDRGPU_OK;
-    const int top_up = 2 * h->max_blocks - (int)(h->osc_produced - h->osc_consumed);
-    if (top_up <= 0) return SDRGPU_OK;
-    // the producer in flight (this call's values) first: ev_osc is about to be re-recorded
-    if (h->osc_pending) {
-        SDRGPU_CUDA(cudaStreamWaitEvent(h->stream, h->ev_osc, 0));
-        h->osc_pending = false;
-        h->osc_safe = h->osc_produced;
-    }
-    if (h->mix_recorded) SDRGPU_CUDA(cudaStreamWaitEvent(h->osc_stream, h->ev_mix, 0));   // the slots' last reader
-    osc_produce_kernel<<<(h->n_mix + 31) / 32, 32, 0, h->osc_stream>>>(h->d_mix, h->d_mix_state, h->d_osc, h->osc_ring_len,
-                                                                       h->osc_produced, top_up, h->n_mix);
-    SDRGPU_CUDA(cudaGetLastError());
-    SDRGPU_CUDA(cudaEventRecord(h->ev_osc, h->osc_stream));
-    h->osc_produced += top_up;
-    h->osc_pending = true;
-    count_launch();
-    return SDRGPU_OK;
-}
+sdrgpu_status sdrgpu::chan_osc_ahead(sdrgpu_channelizer *h) { return outputs_ahead(h->outputs, h->stream); }
 
-cudaStream_t sdrgpu::chan_osc_stream(const sdrgpu_channelizer *h) { return h->n_mix > 0 ? h->osc_stream : nullptr; }
+cudaStream_t sdrgpu::chan_osc_stream(const sdrgpu_channelizer *h) { return h->outputs.n_mix > 0 ? h->outputs.osc_stream : nullptr; }
 
 void sdrgpu::chan_swap_staging(sdrgpu_channelizer *h)
 {
@@ -1407,22 +1048,15 @@ sdrgpu_status sdrgpu_chan_create(sdrgpu_channelizer **out, const float *taps, in
     CHK(cudaMemcpy(h->d_taps, padded.data(), sizeof(float) * padded.size(), cudaMemcpyHostToDevice));
     CHK(cudaMalloc(&h->d_tw, sizeof(float2) * (size_t)M));
     CHK(cudaMemcpy(h->d_tw, tw.data(), sizeof(float2) * (size_t)M, cudaMemcpyHostToDevice));
-    // fast path (pfb2_kernel) for the channel counts of the common tuner rates with the reference's 9 taps per channel
-    if (h->T == 9) {
-        // channel counts of the common tuner rates (25 kHz channels): 2 / 2.4 / 2.5 / 3 / 4 / 5 / 6 / 8 / 10 / 16 / 20 MS/s
-        static const int fast[][3] = {{400, 20, 20}, {800, 32, 25}, {96, 8, 12}, {640, 32, 20}, {320, 16, 20}, {240, 12, 20}, {200, 10, 20}, {160, 8, 20}, {120, 10, 12}, {100, 10, 10}, {80, 8, 10}};
-        for (const auto &f : fast)
-            if (M == f[0]) {
-                h->fast_r1 = f[1];
-                h->fast_r2 = f[2];
-            }
-    }
-    if (h->fast_r1) {
+    if (h->T == 9)
+        for (const PfbRow &row : kPfbRows)
+            if (row.M == M) h->fast = &row;
+    if (h->fast) {
         std::vector<float2> tw2((size_t)M);
-        for (int k1 = 0; k1 < h->fast_r1; k1++)
-            for (int n2 = 0; n2 < h->fast_r2; n2++) {
+        for (int k1 = 0; k1 < h->fast->R1; k1++)
+            for (int n2 = 0; n2 < h->fast->R2; n2++) {
                 const double a = 2.0 * 3.14159265358979323846 * (double)((long long)k1 * n2 % M) / (double)M;
-                tw2[(size_t)k1 * h->fast_r2 + n2] = make_float2((float)cos(a), (float)sin(a));
+                tw2[(size_t)k1 * h->fast->R2 + n2] = make_float2((float)cos(a), (float)sin(a));
             }
         CHK(cudaMalloc(&h->d_tw2, sizeof(float2) * (size_t)M));
         CHK(cudaMemcpy(h->d_tw2, tw2.data(), sizeof(float2) * (size_t)M, cudaMemcpyHostToDevice));
@@ -1461,18 +1095,7 @@ sdrgpu_status sdrgpu_chan_destroy(sdrgpu_channelizer *h)
     cudaFree(h->d_sel);
     cudaFree(h->d_gain_f);
     cudaFree(h->d_gain_d);
-    cudaFree(h->d_post);
-    cudaFree(h->d_post_state);
-    cudaFree(h->d_out2);
-    if (h->osc_stream) {
-        cudaStreamSynchronize(h->osc_stream);
-        cudaStreamDestroy(h->osc_stream);
-        cudaEventDestroy(h->ev_mix);
-        cudaEventDestroy(h->ev_osc);
-    }
-    cudaFree(h->d_mix);
-    cudaFree(h->d_mix_state);
-    cudaFree(h->d_osc);
+    sdrgpu::outputs_destroy(h->outputs);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     if (h->copy_in) cudaStreamDestroy(h->copy_in);
     if (h->copy_out) cudaStreamDestroy(h->copy_out);
@@ -1575,7 +1198,7 @@ sdrgpu_status sdrgpu_chan_set_sample_rate(sdrgpu_channelizer *h, double sample_r
     h->sample_rate = sample_rate;
     // the oscillator angles of frequency-corrected / two-bin channels depend on the channel rate: re-derive them
     // (like Oscillator.setSampleRate -> update(); this restarts the oscillators, as selecting does)
-    if (changed && (h->n_mix > 0 || h->n_post > 0)) {
+    if (changed && (h->outputs.n_mix > 0 || h->outputs.n_post > 0)) {
         SDRGPU_CUDA(cudaSetDevice(h->device));
         SDRGPU_CUDA(cudaStreamSynchronize(h->stream));
         return upload_selection(h);
@@ -1606,12 +1229,13 @@ sdrgpu_status sdrgpu_chan_select(sdrgpu_channelizer *h, const sdrgpu_output_chan
         const int entries = n_synthesis_taps / 2;
         if (entries > kMaxSynthEntries)
             return fail(SDRGPU_ERR_INVALID_ARG, "synthesis filter longer than %d taps", 2 * kMaxSynthEntries);
-        std::memset(&h->synth, 0, sizeof(h->synth));
-        h->synth.entries = entries;
+        SynthFilter &synth = h->outputs.synth;
+        std::memset(&synth, 0, sizeof(synth));
+        synth.entries = entries;
         int fp = 0;
         for (int cp = 0; cp < n_synthesis_taps && fp + 1 < 4 * entries; cp++) {
-            h->synth.f[fp++] = synthesis_filter[cp];
-            h->synth.f[fp++] = synthesis_filter[cp];
+            synth.f[fp++] = synthesis_filter[cp];
+            synth.f[fp++] = synthesis_filter[cp];
         }
     }
     SDRGPU_CUDA(cudaStreamSynchronize(h->stream));

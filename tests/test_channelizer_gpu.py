@@ -277,11 +277,12 @@ def test_frequency_corrected_channels_oscillator_look_ahead_is_bit_exact(gpu):
                 break
 
 
-@pytest.mark.parametrize("m", [400, 800])
+@pytest.mark.parametrize("m", [96, 160, 400, 800])
 def test_every_bin_frequency_corrected_is_mixed_in_the_channelizer_kernel(gpu, m):
-    """all M bins selected in order as frequency-corrected one-bin channels with one gain: pfb2_kernel multiplies the
-    look-ahead oscillator values in where it stores the rows (no osc_mix_kernel pass).  Every row must equal the oracle's
-    Oscillator + applyGain on the GPU's own uncorrected row, bit for bit, across ragged calls that wrap the rings."""
+    """all M bins selected in order as frequency-corrected one-bin channels with one gain: a pfb2_kernel instance with
+    8-block tiles (M = 160 ... 800) multiplies the look-ahead oscillator values in where it stores the rows (no
+    osc_mix_kernel pass); one with 16-block tiles (M = 96) leaves them to osc_mix_kernel.  Every row must equal the
+    oracle's Oscillator + applyGain on the GPU's own uncorrected row, bit for bit, across ragged calls that wrap the rings."""
     from sdrtrunk_b200.dsp import ComplexPolyphaseChannelizerM2
     fs = 25000.0 * m
     rng = np.random.default_rng(29)

@@ -40,7 +40,7 @@ def test_window_and_envelope_constants():
     assert "(%s * qa)" % weight in source("oracle", "orc_filters.c")
     assert "__fmul_rn(%s, b)" % weight in source("sdrtrunk_b200", "csrc", "filters.cu")
     assert "(%s - norm)" % scalor in source("oracle", "orc_output.c")
-    assert "__fsub_rn(%s, norm)" % scalor in source("sdrtrunk_b200", "csrc", "channelizer.cu")
+    assert "__fsub_rn(%s, norm)" % scalor in source("sdrtrunk_b200", "csrc", "outputs.cu")
     floor = np.float32(agc["minimum_envelope"])
     y = oracle.agc_block(np.array([3e-5, -1e-5] * 1024, np.float32))          # envelope below the minimum: gain 1 / 1e-4
     assert np.array_equal(y[:2], np.array([3e-5, -1e-5], np.float32) * (np.float32(1.0) / floor))
