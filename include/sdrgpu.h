@@ -379,6 +379,29 @@ sdrgpu_status sdrgpu_pipeline_wait(sdrgpu_pipeline *p);
  * chunk).  Default: by bank size -- 6 from 2400 channels (several tuners in one bank), else 1 */
 sdrgpu_status sdrgpu_pipeline_set_device_chunks(sdrgpu_pipeline *p, int chunks);
 
+/* Several tuners, several banks: one channelizer pass feeds banks of different decoder types (a tuner serving a P25
+ * control channel, P25 traffic, DMR and NBFM channels at once, as PolyphaseChannelManager serves channels of every
+ * decoder type from one channelizer).  route[r], one entry per selected channel in pipeline row order (chans[0]'s
+ * selection in order, then chans[1]'s, ...), is the index in banks[] of the bank that decodes that channel; bank j's rows
+ * are the rows routed to it, in that order.  Every bank must receive exactly its n_channels rows, all banks must have the
+ * same block_size and no pending samples (they are kept in step), and the channelizers the same channel count
+ * (INVALID_ARG / BAD_STATE, checked before any device work: a refused create leaves every handle usable).  While the
+ * pipeline lives, every bank runs on banks[0]'s stream (sdrgpu_bank_set_stream; destroy restores the others').
+ * sdrgpu_pipeline_create_multi is the one-bank, all-zero route of this.  outputs[j] takes bank j's outputs, as the
+ * arguments of sdrgpu_pipeline_process_multi would; every bank runs the schedule it would run alone, and bank j's
+ * results equal those of a one-bank pipeline whose channelizers select only bank j's channels.  A channelizer whose
+ * selection no longer has the row count the route was built for gets BAD_STATE; so do sdrgpu_pipeline_process_multi and
+ * sdrgpu_pipeline_submit_multi on a pipeline of several banks. */
+typedef struct {
+    uint8_t *symbols; int symbol_stride;          /* as sdrgpu_pipeline_process_multi, per bank */
+    float *demod; long long demod_stride_floats;
+    int *counts;
+} sdrgpu_bank_output;
+sdrgpu_status sdrgpu_pipeline_create_routed(sdrgpu_pipeline **p, sdrgpu_channelizer *const *chans, int n_chans,
+                                            sdrgpu_bank *const *banks, int n_banks, const int *route);
+sdrgpu_status sdrgpu_pipeline_process_routed(sdrgpu_pipeline *p, const void *const *iq, int n_floats, int in_mem,
+                                             const sdrgpu_bank_output *outputs /* [n_banks] */, int out_mem);
+
 #ifdef __cplusplus
 }
 #endif

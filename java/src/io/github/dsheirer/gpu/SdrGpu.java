@@ -45,6 +45,12 @@ public final class SdrGpu
     public static final StructLayout OUTPUT_CHANNEL = MemoryLayout.structLayout(JAVA_INT.withName("bin1"), JAVA_INT.withName("bin2"),
         JAVA_LONG.withName("frequency_offset_hz"), JAVA_DOUBLE.withName("gain"));
 
+    /** struct sdrgpu_bank_output { uint8_t *symbols; int symbol_stride; float *demod; long long demod_stride_floats; int *counts; }:
+     * one bank's outputs of sdrgpu_pipeline_process_routed */
+    public static final StructLayout BANK_OUTPUT = MemoryLayout.structLayout(
+        ADDRESS.withName("symbols"), JAVA_INT.withName("symbol_stride"), MemoryLayout.paddingLayout(4),
+        ADDRESS.withName("demod"), JAVA_LONG.withName("demod_stride_floats"), ADDRESS.withName("counts"));
+
     /** struct sdrgpu_bank_config (include/sdrgpu.h), natural C alignment on x86-64 / aarch64 */
     public static final StructLayout BANK_CONFIG = MemoryLayout.structLayout(
         JAVA_INT.withName("n_channels"), MemoryLayout.paddingLayout(4),
@@ -90,6 +96,13 @@ public final class SdrGpu
         FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS));
     static final MethodHandle PIPELINE_CREATE_MULTI = h("sdrgpu_pipeline_create_multi",
         FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS));
+    /** (pipeline*, channelizers[], nChans, banks[], nBanks, int[] route): one channelizer pass feeds several banks; route[r] is
+     * the bank index of selected channel r in pipeline row order */
+    static final MethodHandle PIPELINE_CREATE_ROUTED = h("sdrgpu_pipeline_create_routed",
+        FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS, JAVA_INT, ADDRESS));
+    /** (pipeline, iq[], nFloats, inMem, BANK_OUTPUT[nBanks], outMem) */
+    static final MethodHandle PIPELINE_PROCESS_ROUTED = h("sdrgpu_pipeline_process_routed",
+        FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, ADDRESS, JAVA_INT));
     static final MethodHandle PIPELINE_DESTROY = h("sdrgpu_pipeline_destroy", FunctionDescriptor.of(JAVA_INT, ADDRESS));
     static final MethodHandle PIPELINE_PROCESS_MULTI = h("sdrgpu_pipeline_process_multi",
         FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, JAVA_LONG, ADDRESS, JAVA_INT));

@@ -75,6 +75,9 @@ struct ChanParams {
     float2 *next_state;  // pfb2_kernel only: one CTA also writes the next call's history (else save_state_kernel)
     int next_len, consumed;
     float neg_zero;      // -0.0f as a run-time value: the addend of the filter bank's packed products (fb_thread)
+    // the ROUTED kernel instances: row c < n_main goes to rows[c] + col instead of out + c * out_stride (channel_row)
+    float *const *rows;
+    long long col;
 };
 
 // ByteSampleConverter / SignedByteSampleConverter (J/source/tuner/... lookup tables: (b - 127) / 128.0f, b / 128.0f): both
@@ -113,7 +116,7 @@ __device__ __forceinline__ float2 cadd(float2 a, float2 b) { return make_float2(
 __device__ __forceinline__ float2 csub(float2 a, float2 b) { return make_float2(a.x - b.x, a.y - b.y); }
 __device__ __forceinline__ float2 jmul(float2 a) { return make_float2(-a.y, a.x); }  // * (+j)
 
-template <int NB, int TT>
+template <int NB, int TT, bool ROUTED>
 __global__ void __launch_bounds__(kThreads) pfb_ifft_kernel(const ChanParams p)
 {
     extern __shared__ float2 smem[];
@@ -276,7 +279,8 @@ __global__ void __launch_bounds__(kThreads) pfb_ifft_kernel(const ChanParams p)
                 v.x = __double2float_rn(__dmul_rn((double)v.x, g));
                 v.y = __double2float_rn(__dmul_rn((double)v.y, g));
             }
-            float *row = c < p.n_main ? p.out + (size_t)c * p.out_stride : p.out2 + (size_t)(c - p.n_main) * p.out2_stride;
+            float *row = c < p.n_main ? channel_row<ROUTED>(p.out, p.out_stride, p.rows, p.col, c)
+                                      : p.out2 + (size_t)(c - p.n_main) * p.out2_stride;
             *reinterpret_cast<float2 *>(row + 2 * (size_t)b) = v;
         }
     } else {
@@ -392,7 +396,7 @@ __device__ __forceinline__ void fb_thread(const ChanParams &p, const float2 *__r
     }
 }
 
-template <int M, int R1, int R2, int NB, int TT, int NT, int MINB, bool RAW>
+template <int M, int R1, int R2, int NB, int TT, int NT, int MINB, bool RAW, bool ROUTED>
 // M = 800 runs three CTAs per SM: 80 registers (no spill; 8 bytes with 8-bit input) and, with V inside Y, 53 KB of shared
 // memory per CTA on the direct-store path.  The third CTA's phases fill the barriers of the other two: 1.40 -> 1.15 ms per
 // 8 launches on a B200 at 1000 W (profiles/r5f_pfb_pipe_time.txt); 3 x 256 x 80 registers still leave 4 K to the one-warp oscillator
@@ -481,8 +485,12 @@ __global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
             if (b0 + b < p.n_blocks) {
                 // FloatFFT_1D.complexInverse(a, true): a[i] *= 1.0f / n; then applyGain
                 const float inv = p.inv_m, g = p.gain_uniform;
-                float *o = p.out + (size_t)k1 * p.out_stride + 2 * (size_t)(b0 + b);
+                // bin k1 + R1 k2 is row k1 + R1 k2; routed rows are looked up one by one (channel_row)
+                float *o = ROUTED ? nullptr : p.out + (size_t)k1 * p.out_stride + 2 * (size_t)(b0 + b);
                 const size_t ostep = (size_t)R1 * p.out_stride;
+                auto dst = [&](int k2) {
+                    return ROUTED ? channel_row<true>(nullptr, 0, p.rows, p.col + 2 * (b0 + b), k1 + R1 * k2) : o;
+                };
                 if (p.osc != nullptr) {
                     // every bin frequency-corrected (OneChannelOutputProcessor + Oscillator, row == bin == oscillator): the
                     // oscillator value of this block from the look-ahead rings, multiplied in between the 1/M of the inverse
@@ -494,8 +502,8 @@ __global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
 #pragma unroll
                     for (int k2 = 0; k2 < R2; k2++) {
                         const float2 m = mix_complex(make_float2(__fmul_rn(a[k2].x, inv), __fmul_rn(a[k2].y, inv)), __ldg(zp));
-                        *reinterpret_cast<float2 *>(o) = make_float2(__fmul_rn(m.x, g), __fmul_rn(m.y, g));
-                        o += ostep;
+                        *reinterpret_cast<float2 *>(dst(k2)) = make_float2(__fmul_rn(m.x, g), __fmul_rn(m.y, g));
+                        if (!ROUTED) o += ostep;
                         zp += zstep;
                     }
                 } else {
@@ -503,8 +511,8 @@ __global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
                     for (int k2 = 0; k2 < R2; k2++) {
                         // (1 / M, then the gain: two packed multiplies for four scalar ones)
                         const float2 v = __fmul2_rn(__fmul2_rn(a[k2], make_float2(inv, inv)), make_float2(g, g));
-                        *reinterpret_cast<float2 *>(o) = v;
-                        o += ostep;
+                        *reinterpret_cast<float2 *>(dst(k2)) = v;
+                        if (!ROUTED) o += ostep;
                     }
                 }
             }
@@ -531,7 +539,7 @@ __global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
             if (p.identity) {
                 // default selection: every bin in order, one float-representable gain
                 const float g = p.gain_uniform;
-                float *o = out + (size_t)row0 * p.out_stride;
+                float *o = ROUTED ? nullptr : out + (size_t)row0 * p.out_stride;
                 const size_t ostep = (size_t)ROWS * p.out_stride;
                 const float2 *xr = X + bl * XS;
 #pragma unroll 5
@@ -539,8 +547,8 @@ __global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
                     float2 v = xr[c];
                     v.x = __fmul_rn(__fmul_rn(v.x, inv_m), g);
                     v.y = __fmul_rn(__fmul_rn(v.y, inv_m), g);
-                    *reinterpret_cast<float2 *>(o) = v;
-                    o += ostep;
+                    *reinterpret_cast<float2 *>(ROUTED ? channel_row<true>(nullptr, 0, p.rows, p.col + 2 * b, c) : o) = v;
+                    if (!ROUTED) o += ostep;
                 }
             } else if (p.gain_exact) {
                 for (int c = row0; c < p.n_sel; c += ROWS) {
@@ -548,7 +556,8 @@ __global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
                     float2 v = X[bl * XS + __ldg(p.sel + c)];
                     v.x = __fmul_rn(__fmul_rn(v.x, inv_m), g);
                     v.y = __fmul_rn(__fmul_rn(v.y, inv_m), g);
-                    float *row = c < p.n_main ? p.out + (size_t)c * p.out_stride : p.out2 + (size_t)(c - p.n_main) * p.out2_stride;
+                    float *row = c < p.n_main ? channel_row<ROUTED>(p.out, p.out_stride, p.rows, p.col, c)
+                                              : p.out2 + (size_t)(c - p.n_main) * p.out2_stride;
                     *reinterpret_cast<float2 *>(row + 2 * (size_t)b) = v;
                 }
             } else {
@@ -557,7 +566,8 @@ __global__ void __launch_bounds__(NT, MINB) pfb2_kernel(const ChanParams p)
                     float2 v = X[bl * XS + __ldg(p.sel + c)];
                     v.x = __double2float_rn(__dmul_rn((double)__fmul_rn(v.x, inv_m), g));
                     v.y = __double2float_rn(__dmul_rn((double)__fmul_rn(v.y, inv_m), g));
-                    float *row = c < p.n_main ? p.out + (size_t)c * p.out_stride : p.out2 + (size_t)(c - p.n_main) * p.out2_stride;
+                    float *row = c < p.n_main ? channel_row<ROUTED>(p.out, p.out_stride, p.rows, p.col, c)
+                                              : p.out2 + (size_t)(c - p.n_main) * p.out2_stride;
                     *reinterpret_cast<float2 *>(row + 2 * (size_t)b) = v;
                 }
             }
@@ -608,10 +618,11 @@ constexpr int kPfbPrefetchBlocks = 148 * 8 * 2;
 
 // One pfb2_kernel shape: M = R1 x R2 channels, NB blocks per tile, NT threads, at least MINB CTAs per SM.  f32 launches
 // the instance for float input; raw, if there is one, the instance that reads 8-bit tuner samples and converts on load.
+// Each comes as [0] contiguous rows and [1] routed rows (ChanParams::rows).
 using PfbLauncher = sdrgpu_status (*)(const sdrgpu_channelizer *h, const ChanParams &p);
 struct PfbRow {
     int M, R1, R2, NB, NT, MINB;
-    PfbLauncher f32, raw;
+    PfbLauncher f32[2], raw[2];
 };
 
 }  // namespace
@@ -711,11 +722,11 @@ sdrgpu_status upload_selection(sdrgpu_channelizer *h)
     return SDRGPU_OK;
 }
 
-template <int M, int R1, int R2, int NB, int TT, int NT, int MINB, bool RAW>
+template <int M, int R1, int R2, int NB, int TT, int NT, int MINB, bool RAW, bool ROUTED>
 sdrgpu_status launch_pfb2(const sdrgpu_channelizer *h, const ChanParams &p)
 {
     using L = Pfb2Layout<M, R1, R2, NB, TT, NT>;
-    auto kernel = pfb2_kernel<M, R1, R2, NB, TT, NT, MINB, RAW>;
+    auto kernel = pfb2_kernel<M, R1, R2, NB, TT, NT, MINB, RAW, ROUTED>;
     // a pipeline that overlaps its time chunks with the demodulator holds the channelizer to a few CTAs per SM
     // the direct row stores (NB = 8, default selection, channel layout) need no X region
     const size_t need = (p.identity && p.layout == SDRGPU_LAYOUT_CHANNELS) ? L::smem_direct : L::smem_bytes;
@@ -728,10 +739,10 @@ sdrgpu_status launch_pfb2(const sdrgpu_channelizer *h, const ChanParams &p)
     return SDRGPU_OK;
 }
 
-template <int NB, int TT>
+template <int NB, int TT, bool ROUTED>
 sdrgpu_status launch_pfb(const sdrgpu_channelizer *h, const ChanParams &p, int grid)
 {
-    auto kernel = pfb_ifft_kernel<NB, TT>;
+    auto kernel = pfb_ifft_kernel<NB, TT, ROUTED>;
     SDRGPU_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes));
     kernel<<<grid, kThreads, h->smem_bytes, h->stream>>>(p);
     count_launch();
@@ -742,8 +753,12 @@ sdrgpu_status launch_pfb(const sdrgpu_channelizer *h, const ChanParams &p, int g
 template <int M, int R1, int R2, int NB, int NT, int MINB, bool RAW>
 constexpr PfbRow pfb_row()
 {
-    PfbRow row{M, R1, R2, NB, NT, MINB, launch_pfb2<M, R1, R2, NB, 9, NT, MINB, false>, nullptr};
-    if constexpr (RAW) row.raw = launch_pfb2<M, R1, R2, NB, 9, NT, MINB, true>;
+    PfbRow row{M, R1, R2, NB, NT, MINB, {launch_pfb2<M, R1, R2, NB, 9, NT, MINB, false, false>,
+                                         launch_pfb2<M, R1, R2, NB, 9, NT, MINB, false, true>}, {nullptr, nullptr}};
+    if constexpr (RAW) {
+        row.raw[0] = launch_pfb2<M, R1, R2, NB, 9, NT, MINB, true, false>;
+        row.raw[1] = launch_pfb2<M, R1, R2, NB, 9, NT, MINB, true, true>;
+    }
     return row;
 }
 
@@ -769,14 +784,19 @@ constexpr PfbRow kPfbRows[] = {
 // pfb_ifft_kernel.
 sdrgpu_status pfb_launch(const sdrgpu_channelizer *h, const ChanParams &p, bool raw)
 {
-    if (h->fast) return (raw ? h->fast->raw : h->fast->f32)(h, p);
+    const bool routed = p.rows != nullptr;
+    if (h->fast) return (raw ? h->fast->raw : h->fast->f32)[routed](h, p);
     const int grid = (p.n_blocks + h->NB - 1) / h->NB;
-    if (h->NB == 16) return h->T == 9 ? launch_pfb<16, 9>(h, p, grid) : launch_pfb<16, 0>(h, p, grid);
-    return h->T == 9 ? launch_pfb<8, 9>(h, p, grid) : launch_pfb<8, 0>(h, p, grid);
+    if (routed) {
+        if (h->NB == 16) return h->T == 9 ? launch_pfb<16, 9, true>(h, p, grid) : launch_pfb<16, 0, true>(h, p, grid);
+        return h->T == 9 ? launch_pfb<8, 9, true>(h, p, grid) : launch_pfb<8, 0, true>(h, p, grid);
+    }
+    if (h->NB == 16) return h->T == 9 ? launch_pfb<16, 9, false>(h, p, grid) : launch_pfb<16, 0, false>(h, p, grid);
+    return h->T == 9 ? launch_pfb<8, 9, false>(h, p, grid) : launch_pfb<8, 0, false>(h, p, grid);
 }
 
 // whether the filter bank reads 8-bit tuner samples as they are
-bool converts_on_load(const sdrgpu_channelizer *h) { return h->fast && h->fast->raw; }
+bool converts_on_load(const sdrgpu_channelizer *h) { return h->fast && h->fast->raw[0]; }
 
 }  // namespace
 
@@ -794,7 +814,7 @@ static void launch_convert(sdrgpu_channelizer *h, const uint8_t *src, float2 *ds
 }
 
 sdrgpu_status sdrgpu::chan_enqueue(sdrgpu_channelizer *h, const float2 *d_in, int n_in, float *d_out, long long stride,
-                                   int layout, int *n_blocks_out)
+                                   int layout, int *n_blocks_out, float *const *rows, long long col)
 {
     const int total = h->leftover + n_in;
     const int n_blocks = total / h->half;
@@ -830,6 +850,8 @@ sdrgpu_status sdrgpu::chan_enqueue(sdrgpu_channelizer *h, const float2 *d_in, in
     if (n_blocks > 0) {
         ChanParams p{};
         p.neg_zero = -0.0f;
+        p.rows = rows;
+        p.col = col;
         p.state = state;
         p.in = d_in;
         p.raw = fuse_convert ? raw : nullptr;
@@ -878,7 +900,7 @@ sdrgpu_status sdrgpu::chan_enqueue(sdrgpu_channelizer *h, const float2 *d_in, in
         const sdrgpu_status st = pfb_launch(h, p, fuse_convert);
         h->timer.end(h->stream);
         SDRGPU_TRY(st);
-        if (layout == SDRGPU_LAYOUT_CHANNELS) SDRGPU_TRY(outputs_after(o, d_out, stride, n_blocks, fused_mix, h->stream));
+        if (layout == SDRGPU_LAYOUT_CHANNELS) SDRGPU_TRY(outputs_after(o, d_out, stride, n_blocks, fused_mix, h->stream, rows, col));
     }
     // carry the history + leftover over to the next call
     if (n_in > 0) {

@@ -54,9 +54,10 @@ inline sdrgpu_status fail(sdrgpu_status code, const char *fmt, ...)
 
 // number of output rows the channelizer currently selects (channelizer.cu)
 int chan_selected_count(const sdrgpu_channelizer *h);
-// channelizer internals the fused pipeline (bank.cu) drives directly
+// channelizer internals the fused pipeline (bank.cu) drives directly.  chan_enqueue writes channel-layout row c to
+// d_out + c * stride, or, given a row table (a pipeline routing the rows to several banks), to rows[c] + col (floats)
 sdrgpu_status chan_enqueue(sdrgpu_channelizer *h, const float2 *d_in, int n_in, float *d_out, long long stride, int layout,
-                           int *n_blocks_out);
+                           int *n_blocks_out, float *const *rows = nullptr, long long col = 0);
 cudaStream_t chan_stream(const sdrgpu_channelizer *h);
 // host-buffer staging of the chunked paths: enqueue the H2D copy of complex samples [first, first + n) of the caller's
 // buffer (in the handle's input format) on copy_stream; then, on the handle's stream, convert them to float I/Q if the

@@ -32,15 +32,17 @@ __device__ __forceinline__ float2 osc_rotate(float2 cur, float2 angle)
 //                     walks, lane i keeping the value of sample i
 //   gain              ReusableComplexBuffer.applyGain: samples[x] = (float)(samples[x] * (double) gain)
 // ---------------------------------------------------------------------------------------------------------------
+template <bool ROUTED>
 __global__ void __launch_bounds__(32) post_channel_kernel(float *out, long long out_stride, const float *out2,
                                                           long long out2_stride, int n, const PostChannel *chans,
-                                                          PostState *states, const __grid_constant__ SynthFilter filt)
+                                                          PostState *states, const __grid_constant__ SynthFilter filt,
+                                                          float *const *rows, long long col)
 {
     __shared__ float4 ent[kMaxSynthEntries + 32];
     const int lane = threadIdx.x;
     const PostChannel c = chans[blockIdx.x];
     PostState *st = states + blockIdx.x;
-    float2 *row = reinterpret_cast<float2 *>(out + (size_t)c.row * out_stride);
+    float2 *row = reinterpret_cast<float2 *>(channel_row<ROUTED>(out, out_stride, rows, col, c.row));
     const float2 *row2 = c.row2 >= 0 ? reinterpret_cast<const float2 *>(out2 + (size_t)c.row2 * out2_stride) : nullptr;
     const int H = filt.entries - 1;   // history entries a sample needs besides its own
     const float2 angle = make_float2(c.angle_i, c.angle_q);
@@ -162,13 +164,15 @@ __global__ void __launch_bounds__(32) osc_produce_kernel(const MixChannel *__res
 }
 
 // grid (ceil(n / 256), n_mix): row[k] = (float)((double)(row[k] * osc[start + k]) * gain)
+template <bool ROUTED>
 __global__ void osc_mix_kernel(float *out, long long out_stride, const MixChannel *__restrict__ chans,
-                               const float2 *__restrict__ ring, int ring_len, long long start, int n)
+                               const float2 *__restrict__ ring, int ring_len, long long start, int n, float *const *rows,
+                               long long col)
 {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
     const MixChannel c = chans[blockIdx.y];
-    float2 *row = reinterpret_cast<float2 *>(out + (size_t)c.row * out_stride);
+    float2 *row = reinterpret_cast<float2 *>(channel_row<ROUTED>(out, out_stride, rows, col, c.row));
     const float2 m = mix_complex(row[k], ring[(size_t)blockIdx.y * ring_len + (int)((start + k) % ring_len)]);
     row[k] = make_float2(__double2float_rn(__dmul_rn((double)m.x, c.gain)), __double2float_rn(__dmul_rn((double)m.y, c.gain)));
 }
@@ -334,19 +338,19 @@ sdrgpu_status sdrgpu::outputs_before(ChanOutputs &o, int n_blocks, cudaStream_t 
 }
 
 sdrgpu_status sdrgpu::outputs_after(ChanOutputs &o, float *out, long long stride, int n_blocks, bool mix_fused,
-                                    cudaStream_t stream)
+                                    cudaStream_t stream, float *const *rows, long long col)
 {
     if (o.n_post > 0) {
-        post_channel_kernel<<<o.n_post, 32, 0, stream>>>(out, stride, o.d_out2, 2LL * o.max_blocks, n_blocks, o.d_post,
-                                                         o.d_post_state, o.synth);
+        (rows ? post_channel_kernel<true> : post_channel_kernel<false>)<<<o.n_post, 32, 0, stream>>>(
+            out, stride, o.d_out2, 2LL * o.max_blocks, n_blocks, o.d_post, o.d_post_state, o.synth, rows, col);
         count_launch();
         SDRGPU_CUDA(cudaGetLastError());
     }
     if (o.n_mix > 0) {
         if (!mix_fused) {
             SDRGPU_TRY(ensure_osc(o, n_blocks, stream));
-            osc_mix_kernel<<<dim3((n_blocks + 255) / 256, o.n_mix), 256, 0, stream>>>(out, stride, o.d_mix, o.d_osc, o.osc_ring_len,
-                                                                                      o.osc_consumed, n_blocks);
+            (rows ? osc_mix_kernel<true> : osc_mix_kernel<false>)<<<dim3((n_blocks + 255) / 256, o.n_mix), 256, 0, stream>>>(
+                out, stride, o.d_mix, o.d_osc, o.osc_ring_len, o.osc_consumed, n_blocks, rows, col);
             count_launch();
         }
         o.osc_consumed += n_blocks;

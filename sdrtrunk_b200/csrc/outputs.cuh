@@ -45,6 +45,17 @@ __device__ __forceinline__ float2 mix_complex(float2 v, float2 z)
     return make_float2(x, y);
 }
 
+// Where channel-layout row c of a call starts.  A channelizer's own rows are contiguous: out + c * stride.  A pipeline
+// that routes one channelizer's rows to several banks passes a table instead (ROUTED, the kernels' separate instances):
+// rows[c] is that row's place in its bank's pending input, and this call's samples start col floats behind it -- one
+// offset for every row, because the banks of a pipeline are kept in step.
+template <bool ROUTED>
+__device__ __forceinline__ float *channel_row(float *out, long long stride, float *const *rows, long long col, int c)
+{
+    if constexpr (ROUTED) return rows[c] + col;
+    else return out + (size_t)c * stride;
+}
+
 struct ChanOutputs {
     int max_blocks = 0;             // blocks one channelizer call can produce: scratch rows and rings are sized for it
     SynthFilter synth{};            // two-bin channels' synthesis filter (sdrgpu_chan_select)
@@ -80,9 +91,11 @@ sdrgpu_status outputs_select(ChanOutputs &o, const std::vector<sdrgpu_output_cha
 // Before a filter bank that mixes the oscillators in: makes the rings hold n_blocks values from osc_consumed on (on
 // `stream`) and gives the rings ([n_mix][osc_ring_len]) and the slot of the first value.
 sdrgpu_status outputs_before(ChanOutputs &o, int n_blocks, cudaStream_t stream, const float2 **osc, int *osc_start);
-// After the filter bank wrote n_blocks blocks to the rows of `out`: runs post_channel_kernel and, unless the filter bank
-// mixed them (mix_fused), osc_mix_kernel; then tops the rings up behind the mix on the side stream.
-sdrgpu_status outputs_after(ChanOutputs &o, float *out, long long stride, int n_blocks, bool mix_fused, cudaStream_t stream);
+// After the filter bank wrote n_blocks blocks to the rows of `out` (or, with a row table, to rows[c] + col: channel_row):
+// runs post_channel_kernel and, unless the filter bank mixed them (mix_fused), osc_mix_kernel; then tops the rings up
+// behind the mix on the side stream.
+sdrgpu_status outputs_after(ChanOutputs &o, float *out, long long stride, int n_blocks, bool mix_fused, cudaStream_t stream,
+                            float *const *rows = nullptr, long long col = 0);
 // A pipeline's look-ahead (chan_osc_ahead): tops the rings up to two calls' worth now.
 sdrgpu_status outputs_ahead(ChanOutputs &o, cudaStream_t stream);
 void outputs_destroy(ChanOutputs &o);

@@ -205,14 +205,29 @@ class Pipeline:
     `channelizer` may be a list of channelizers of equal channel count (several tuners): their selected channels are
     consecutive row ranges of the one bank, and process() then takes one sample buffer per tuner
     (sdrgpu_pipeline_create_multi: the reference runs every channel as its own task whichever tuner it came from,
-    J/source/tuner/channel/TunerChannelSource.java:290-319)."""
+    J/source/tuner/channel/TunerChannelSource.java:290-319).
 
-    def __init__(self, channelizer, bank):
+    Pipeline(channelizers, banks=[...], route=[...]) feeds several banks (decoder types) from the same channelizer pass
+    (sdrgpu_pipeline_create_routed): route[r] is the index in `banks` of the bank that decodes selected channel r, in
+    pipeline row order (the first channelizer's selection, then the next one's, ...), and process() returns one list of
+    per-row results per bank."""
+
+    def __init__(self, channelizer, bank=None, banks=None, route=None):
         self.channelizers = list(channelizer) if isinstance(channelizer, (list, tuple)) else [channelizer]
-        self.channelizer, self.bank = self.channelizers[0], bank
+        self.channelizer = self.channelizers[0]
+        self.routed = banks is not None
+        self.banks = list(banks) if self.routed else [bank]
+        self.bank = self.banks[0]
         self._h = C.c_void_p()
         handles = (C.c_void_p * len(self.channelizers))(*[c._h for c in self.channelizers])
-        native.check(native.lib().sdrgpu_pipeline_create_multi(C.byref(self._h), handles, len(self.channelizers), bank._h))
+        if self.routed:
+            bank_handles = (C.c_void_p * len(self.banks))(*[b._h for b in self.banks])
+            r = np.ascontiguousarray(route, dtype=np.int32)
+            native.check(native.lib().sdrgpu_pipeline_create_routed(C.byref(self._h), handles, len(self.channelizers),
+                                                                   bank_handles, len(self.banks),
+                                                                   r.ctypes.data_as(C.POINTER(C.c_int))))
+        else:
+            native.check(native.lib().sdrgpu_pipeline_create_multi(C.byref(self._h), handles, len(self.channelizers), bank._h))
         self._pending = 0
 
     def setChunks(self, chunks):
@@ -240,6 +255,8 @@ class Pipeline:
         blocks = (self._pending + n) // bank.block_size
         n_out = blocks * (bank.block_size // max(bank.decimation, 1))
         self._pending = (self._pending + n) % bank.block_size
+        if self.routed:
+            return self._process_routed(in_ptrs, n_floats, samples_mem, blocks)
         counts = np.zeros(bank.n_channels, np.int32)
         if bank.is_dqpsk:
             stride = max(16, n_out // 3 + 16)
@@ -252,6 +269,33 @@ class Pipeline:
         native.check(L.sdrgpu_pipeline_process_multi(self._h, in_ptrs, n_floats, samples_mem, None, 0, native.ptr(dem),
                                                      dem.shape[1], native.ptr(counts), native.HOST))
         return dem[:, :width]
+
+    def _process_routed(self, in_ptrs, n_floats, samples_mem, blocks):
+        """every bank's outputs in the shape Pipeline.process gives for one bank: dibit arrays per row (DQPSK), else
+        demodulated floats [rows, n]"""
+        outs = (native.BankOutput * len(self.banks))()
+        keep = []
+        for o, bank in zip(outs, self.banks):
+            n_out = blocks * (bank.block_size // max(bank.decimation, 1))
+            counts = np.zeros(bank.n_channels, np.int32)
+            o.counts = counts.ctypes.data
+            if bank.is_dqpsk:
+                stride = max(16, n_out // 3 + 16)
+                buf = np.zeros((bank.n_channels, stride), np.uint8)
+                o.symbols, o.symbol_stride = buf.ctypes.data, stride
+            else:
+                width = n_out if bank.is_fm else 2 * n_out
+                buf = np.zeros((bank.n_channels, max(width, 1)), np.float32)
+                o.demod, o.demod_stride_floats = buf.ctypes.data, buf.shape[1]
+            keep.append((bank, buf, counts, n_out))
+        native.check(native.lib().sdrgpu_pipeline_process_routed(self._h, in_ptrs, n_floats, samples_mem, outs, native.HOST))
+        result = []
+        for bank, buf, counts, n_out in keep:
+            if bank.is_dqpsk:
+                result.append([buf[c, :counts[c]].copy() for c in range(bank.n_channels)])
+            else:
+                result.append(buf[:, :n_out if bank.is_fm else 2 * n_out])
+        return result
 
     def submit(self, samples):
         """asynchronous process() for a continuous stream of host buffers (DQPSK banks): enqueues the call and returns;

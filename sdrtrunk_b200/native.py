@@ -61,6 +61,12 @@ class BankConfig(C.Structure):
     ]
 
 
+class BankOutput(C.Structure):
+    """sdrgpu_bank_output: one bank's outputs of sdrgpu_pipeline_process_routed"""
+    _fields_ = [("symbols", C.c_void_p), ("symbol_stride", C.c_int), ("demod", C.c_void_p),
+                ("demod_stride_floats", C.c_longlong), ("counts", C.c_void_p)]
+
+
 _f32p = C.POINTER(C.c_float)
 _i32p = C.POINTER(C.c_int)
 _u8p = C.POINTER(C.c_uint8)
@@ -135,6 +141,8 @@ PROTOTYPES = {
     "sdrgpu_pipeline_wait": (C.c_int, [_vp]),
     "sdrgpu_pipeline_destroy": (C.c_int, [_vp]),
     "sdrgpu_pipeline_process": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp, C.c_int, _vp, C.c_longlong, _vp, C.c_int]),
+    "sdrgpu_pipeline_create_routed": (C.c_int, [_vpp, _vp, C.c_int, _vp, C.c_int, _i32p]),
+    "sdrgpu_pipeline_process_routed": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.POINTER(BankOutput), C.c_int]),
 }
 
 _lib = None
