@@ -1,8 +1,10 @@
 """Parity of the CUDA polyphase channelizer (through the C ABI) against the oracle.
 
-Tolerance: 1e-4 relative RMS per channel (BASELINE.json north_star; the inverse DFT's summation order differs
+Tolerance here: 1e-4 relative RMS per channel (BASELINE.json north_star; the inverse DFT's summation order differs
 from JTransforms' by construction).  The filter-bank stage itself is arithmetic-identical (products rounded,
-sequential adds) so the end result is typically ~1e-7.
+sequential adds), so the only legitimate difference is the rounding of the float32 inverse DFT, ~1e-7:
+test_channelizer_paths_gpu.py holds every row of every kernel instance to 1e-6 of the RMS of all rows against a
+float64 reference (the oracle's float32 filter-bank accumulators through a float64 inverse DFT).
 """
 import numpy as np
 import pytest
@@ -42,7 +44,7 @@ def test_results_layout_matches_oracle(gpu, m):
         assert sg.rel_rms(got[:, 2 * k:2 * k + 2], want[:, 2 * k:2 * k + 2]) < TOL
 
 
-@pytest.mark.parametrize("m", [96, 400, 800, 100, 320, 640])
+@pytest.mark.parametrize("m", [96, 400, 800, 100, 320, 640, 80, 120, 160, 200, 240])
 def test_channel_layout_matches_oracle_output_processor(gpu, m):
     """m = 800 is BASELINE configs[4]'s channel count (pfb2_kernel<800, 32, 25>: odd second factor, direct row stores)"""
     from sdrtrunk_b200.dsp import ComplexPolyphaseChannelizerM2
