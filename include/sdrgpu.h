@@ -260,7 +260,9 @@ sdrgpu_status sdrgpu_bank_sync(sdrgpu_bank *b);
 
 /* Feeds n_samples complex samples per channel: channel c starts at iq + c * in_stride_floats.
  * Outputs (each may be NULL; `out_mem` applies to all of them):
- *   symbols  [n_channels][symbol_stride] one byte per decoded Dibit (Dibit.getValue 0..3, J/dsp/symbol/Dibit.java:27-30)
+ *   symbols  [n_channels][symbol_stride] one byte per decoded Dibit (Dibit.getValue 0..3, J/dsp/symbol/Dibit.java:27-30);
+ *            FM_SQUELCH banks with squelch reporting on: one status byte per assembler buffer (see
+ *            sdrgpu_bank_set_squelch_reporting); other banks ignore it
  *   demod    [n_channels][demod_stride_floats] float: FM demodulated samples (FM demods) or the filtered /
  *            gain-controlled interleaved complex stream (SDRGPU_DEMOD_NONE, and as a tap point for DQPSK)
  *   counts   [n_channels] number of symbols (DQPSK) or floats (otherwise) written per channel by this call
@@ -326,6 +328,29 @@ sdrgpu_status sdrgpu_bank_set_demodulator_lanes(sdrgpu_bank *b, int lanes_per_ch
  * sdrgpu_bank_read_symbol_tap returns the symbols of the last process call (values[6 * capacity_symbols]). */
 sdrgpu_status sdrgpu_bank_set_symbol_tap(sdrgpu_bank *b, int channel);
 sdrgpu_status sdrgpu_bank_read_symbol_tap(sdrgpu_bank *b, double *values, int capacity_symbols, int *n_symbols);
+/* Squelch state per assembler buffer, for SDRGPU_DEMOD_FM_SQUELCH banks: what NBFMDecoder asks its
+ * SquelchingFMDemodulator after each demodulate(buffer) (isSquelchChanged, J/dsp/fm/SquelchingFMDemodulator.java;
+ * PowerSquelch.java:88-159).  While reporting is on (default off), every process call -- sdrgpu_bank_process,
+ * sdrgpu_pipeline_process / _multi, and sdrgpu_pipeline_process_routed through sdrgpu_bank_output.symbols -- writes one
+ * status byte per assembler buffer it consumes into `symbols`: byte i of channel c at symbols[c * symbol_stride + i],
+ * for i < counts[c] / (block_size / decimation) (a bank consumes whole buffers, so every call starts on a buffer
+ * boundary).  Bits 0-1: the squelch state after the buffer's last sample (SDRGPU_SQUELCH_ATTACK .. _UNMUTE); bit 2,
+ * SDRGPU_SQUELCH_CHANGED: the state changed at least once during the buffer (PowerSquelch.mSquelchChanged).  The
+ * demodulated samples are 0.0f in MUTE and ATTACK.  symbols == NULL writes no statuses; a symbol_stride smaller than
+ * the call's buffers gets INVALID_ARG before any device work.  With reporting off `symbols` is not touched.  Any other
+ * bank gets INVALID_ARG, with nothing changed. */
+enum {
+    SDRGPU_SQUELCH_ATTACK = 0,
+    SDRGPU_SQUELCH_DECAY = 1,
+    SDRGPU_SQUELCH_MUTE = 2,
+    SDRGPU_SQUELCH_UNMUTE = 3,
+    SDRGPU_SQUELCH_CHANGED = 4
+};
+sdrgpu_status sdrgpu_bank_set_squelch_reporting(sdrgpu_bank *b, int enabled);
+/* PowerSquelch.setSquelchThreshold per channel (channel = -1: every channel), in dB as squelch_threshold_db (the
+ * configured value is every channel's initial one).  Used from the next buffer the bank processes; the squelch's IIR
+ * and ramp state carry on.  INVALID_ARG for a bank without squelch, a channel out of range or a non-finite value. */
+sdrgpu_status sdrgpu_bank_set_squelch_threshold(sdrgpu_bank *b, int channel, double threshold_db);
 /* loop state tap points of one channel: {pll phase, pll frequency, sampling point, detected samples/symbol} */
 sdrgpu_status sdrgpu_bank_get_loop_state(sdrgpu_bank *b, int channel, double *state4);
 /* 4 dibits per byte MSB first (J/dsp/symbol/DibitToByteBufferAssembler.java:58-93); host helper */

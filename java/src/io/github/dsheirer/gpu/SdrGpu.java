@@ -89,6 +89,13 @@ public final class SdrGpu
     static final MethodHandle BANK_CORRECT_INVERSION = h("sdrgpu_bank_correct_inversion",
         FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_DOUBLE));
     static final MethodHandle BANK_SET_SYNC_DETECTOR = h("sdrgpu_bank_set_sync_detector", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT));
+    /** (bank, enabled): FM_SQUELCH banks write one squelch status byte per assembler buffer into `symbols`
+     *  (state after the buffer in bits 0-1: 0 ATTACK, 1 DECAY, 2 MUTE, 3 UNMUTE; bit 2: the squelch changed during it) */
+    static final MethodHandle BANK_SET_SQUELCH_REPORTING = h("sdrgpu_bank_set_squelch_reporting",
+        FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT));
+    /** (bank, channel | -1 for all, threshold dB): PowerSquelch.setSquelchThreshold per channel, from the next buffer on */
+    static final MethodHandle BANK_SET_SQUELCH_THRESHOLD = h("sdrgpu_bank_set_squelch_threshold",
+        FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_DOUBLE));
     /** the listeners of DQPSKDecisionDirectedDemodulatorInstrumented for one channel of a bank: (bank, channel | -1) */
     static final MethodHandle BANK_SET_SYMBOL_TAP = h("sdrgpu_bank_set_symbol_tap", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT));
     /** (bank, double[6 * capacity] values, capacity, int[1] nSymbols): symbol I, Q, samples per symbol, loop frequency, sampling point, PLL error */

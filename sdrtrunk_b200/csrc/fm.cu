@@ -55,23 +55,40 @@ __device__ __forceinline__ bool squelch_step(int &state, int &ramp_count, bool m
     return s == 3 || s == 1;
 }
 
-// one thread per channel: writes gate[n] = 1 where SquelchingFMDemodulator demodulates (UNMUTE or DECAY)
+// one thread per channel: writes gate[n] = 1 where SquelchingFMDemodulator demodulates (UNMUTE or DECAY) and, with
+// `status`, one squelch status byte per buffer_len samples.  Within the ramp machine the state changes
+// (PowerSquelch.mSquelchChanged) exactly where the gate flips, so a buffer's CHANGED bit is "the gate has an edge in
+// it"; the gate in front of the call's first sample is that of the state it starts from.
 __global__ void squelch_gate_kernel(const float2 *__restrict__ in, long long in_stride, int n, SquelchState *states,
                                     uint8_t *__restrict__ gate, long long gate_stride, double alpha,
-                                    double threshold, int ramp, int n_channels)
+                                    const double *__restrict__ thresholds, int ramp, uint8_t *__restrict__ status,
+                                    long long status_stride, int buffer_len, int n_channels)
 {
     const int ch = blockIdx.x * blockDim.x + threadIdx.x;
     if (ch >= n_channels) return;
     SquelchState st = states[ch];
-    const double one_minus = 1.0 - alpha;
+    const double one_minus = 1.0 - alpha, threshold = thresholds[ch];
     const float2 *x = in + (size_t)ch * in_stride;
     uint8_t *g = gate + (size_t)ch * gate_stride;
+    uint8_t *rep = status ? status + (size_t)ch * status_stride : nullptr;
+    bool on_before = st.state & 1, changed = false;
+    int left = buffer_len;
     for (int k = 0; k < n; k++) {
         const float2 s = x[k];
         const double i = (double)s.x, q = (double)s.y;
         const double power_in = __dadd_rn(__dmul_rn(i, i), __dmul_rn(q, q));
         st.output = __dadd_rn(__dmul_rn(st.output, one_minus), __dmul_rn(alpha, power_in));
-        g[k] = squelch_step(st.state, st.ramp_count, st.output < threshold, ramp) ? 1 : 0;
+        const bool on = squelch_step(st.state, st.ramp_count, st.output < threshold, ramp);
+        g[k] = on ? 1 : 0;
+        if (rep) {
+            changed |= on != on_before;
+            on_before = on;
+            if (--left == 0) {
+                *rep++ = (uint8_t)(st.state | (changed ? SDRGPU_SQUELCH_CHANGED : 0));
+                changed = false;
+                left = buffer_len;
+            }
+        }
     }
     states[ch].output = st.output;
     states[ch].state = st.state;
@@ -139,6 +156,14 @@ __global__ void fm_carry_kernel(const float2 *__restrict__ in, long long in_stri
     }
 }
 
+// sdrgpu_bank_set_squelch_threshold: a launch rather than a copy, so that the value is ordered behind the calls already
+// enqueued without a host buffer that has to outlive them
+__global__ void set_threshold_kernel(double *thresholds, int n, double value)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) thresholds[i] = value;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // nbfm_fused_kernel: the whole NBFM front end of one channel in ONE launch (NBFMDecoder.receive,
 // J/module/decode/nbfm/NBFMDecoder.java:129-181):
@@ -177,12 +202,16 @@ struct NbfmParams {
     int cap_e0, cap_o0, cap_e1, cap_o1, cap_z;   // float2 per plane / FIR input buffer (decimating variant, nbfm_fused_layout)
     float neg_zero;            // -0.0f, as a run-time value (see the half-band stages)
     int squelch;               // SquelchingFMDemodulator (else FMDemodulator: every sample demodulated)
-    double alpha, threshold;
+    double alpha;
+    const double *thresholds;  // [C]
     int ramp;
     float fm_gain;
     SquelchState *sq;
     float *out;                // [C][n_new / 2^n_stages] demodulated floats, may be null
     long long out_stride;
+    uint8_t *status;           // kStatus: [C][status_stride] one squelch status byte per buffer_out outputs
+    long long status_stride;
+    int buffer_out;
     int n_channels;
 };
 
@@ -223,13 +252,16 @@ inline size_t nbfm_fused_smem(const NbfmParams &q)
     return (bytes + 15) & ~(size_t)15;
 }
 
-template <bool kDecim>
+// kStatus: the chain thread also writes one squelch status byte per assembler buffer (p.status); a separate instance, so
+// that banks which do not ask for statuses run the chain without the bookkeeping
+template <bool kDecim, bool kStatus>
 __global__ void __launch_bounds__(kNbfmThreads, 8)
 nbfm_fused_kernel(const __grid_constant__ NbfmParams p, const __grid_constant__ NbfmStageTaps taps, const __grid_constant__ FirTaps fir)
 {
     extern __shared__ __align__(16) unsigned char nbfm_smem[];
     __shared__ __align__(8) uint64_t bars[2];
     __shared__ float s_prev[2];          // FMDemodulator.mPreviousI / Q carried from tile to tile
+    __shared__ double s_threshold;       // this channel's squelch threshold (read by the chain thread once per tile)
     __shared__ __align__(16) float hs[kMaxFirTaps];
     const int tid = threadIdx.x, c = blockIdx.x;
     const int S = p.n_stages, d = 1 << S, T = p.tile_out, N = p.n_fir;
@@ -255,7 +287,13 @@ nbfm_fused_kernel(const __grid_constant__ NbfmParams p, const __grid_constant__ 
     if (tid == 0) {
         s_prev[0] = st.prev_i;
         s_prev[1] = st.prev_q;
+        if (p.squelch) s_threshold = p.thresholds[c];
     }
+    // kStatus: the output index that ends the current assembler buffer, whether the gate has had an edge in it so far,
+    // and where its status byte goes
+    int buffer_end = p.buffer_out - 1;
+    bool changed = false;
+    uint8_t *status_at = kStatus ? p.status + (size_t)c * p.status_stride : nullptr;
 
     // raw window of tile t: stream samples [t d T - hist0, t d T + d T_t); negative indices are history
     auto tile_outputs = [&](int t) { return min(T, n_out_total - t * T); };
@@ -527,7 +565,7 @@ nbfm_fused_kernel(const __grid_constant__ NbfmParams p, const __grid_constant__ 
         {
             int last_gated = -1;     // -1: the sample carried in s_prev
             if (p.squelch) {
-                const double one_minus = 1.0 - p.alpha, threshold = p.threshold;
+                const double one_minus = 1.0 - p.alpha, threshold = s_threshold;
                 double output = st.output;
                 int state = st.state, ramp_count = st.ramp_count;
                 const int ramp = p.ramp;
@@ -550,16 +588,43 @@ nbfm_fused_kernel(const __grid_constant__ NbfmParams p, const __grid_constant__ 
                         }
                     }
                     const uint32_t all = n == 32 ? 0xffffffffu : ((1u << n) - 1u);
+                    // kStatus: bit j = output k0 + j ends an assembler buffer (tiles and buffers need not line up).
+                    // Within the ramp machine the state changes exactly where the gate flips (ATTACK / MUTE -> UNMUTE,
+                    // DECAY / UNMUTE -> MUTE), so a buffer's CHANGED bit is "an edge of the gate in it"; the gate in
+                    // front of a word is that of the state it starts from.
+                    uint32_t end_bits = 0;
+                    if constexpr (kStatus) {
+                        const int g0 = t * T + k0;
+                        for (; buffer_end < g0 + n; buffer_end += p.buffer_out) end_bits |= 1u << (buffer_end - g0);
+                    }
+                    auto report = [&](bool edge) {
+                        *status_at++ = (uint8_t)(state | (changed || edge ? SDRGPU_SQUELCH_CHANGED : 0));
+                        changed = false;
+                    };
                     uint32_t on_bits;
                     if (state == 3 && mute_bits == 0) {
                         on_bits = all;            // UNMUTE and never below the threshold: every sample demodulated
+                        if constexpr (kStatus)    // (no edge in a stable word)
+                            for (uint32_t e = end_bits; e; e &= e - 1) report(false);
                     } else if (state == 2 && mute_bits == all) {
                         on_bits = 0;              // MUTE and never above it
+                        if constexpr (kStatus)
+                            for (uint32_t e = end_bits; e; e &= e - 1) report(false);
                     } else {
                         on_bits = 0;
+                        const uint32_t gate_in = (uint32_t)state & 1u;   // UNMUTE / DECAY: the gate is on
+                        uint32_t open = 0xffffffffu;                     // bits of this word in the current buffer
                         for (int j = 0; j < n; j++) {
                             if (squelch_step(state, ramp_count, (mute_bits >> j) & 1u, ramp)) on_bits |= 1u << j;
+                            if constexpr (kStatus) {
+                                if ((end_bits >> j) & 1u) {
+                                    const uint32_t upto = 0xffffffffu >> (31 - j);
+                                    report(((on_bits ^ ((on_bits << 1) | gate_in)) & upto & open) != 0);
+                                    open = ~upto;
+                                }
+                            }
                         }
+                        if constexpr (kStatus) changed |= ((on_bits ^ ((on_bits << 1) | gate_in)) & all & open) != 0;
                     }
                     gate_t[k0 >> 5] = on_bits;
                     if (on_bits) last_gated = k0 + 31 - __clz(on_bits);
@@ -654,12 +719,15 @@ sdrgpu_status nbfm_fused_launch(const FmLaunch &a)
     q.use_bulk = (reinterpret_cast<uintptr_t>(q.in) % 16 == 0) && (q.in_stride % 2 == 0) && (a.n_stages > 0 || a.n % 2 == 0);
     q.squelch = a.squelch;
     q.alpha = a.alpha;
-    q.threshold = a.threshold;
+    q.thresholds = a.thresholds;
     q.ramp = a.ramp;
     q.fm_gain = a.gain;
     q.sq = a.states;
     q.out = a.out;
     q.out_stride = a.out_stride;
+    q.status = a.squelch ? a.status : nullptr;
+    q.status_stride = a.status_stride;
+    q.buffer_out = a.buffer_out;
     q.n_channels = a.n_channels;
     q.neg_zero = -0.0f;
     NbfmStageTaps st{};
@@ -669,12 +737,15 @@ sdrgpu_status nbfm_fused_launch(const FmLaunch &a)
     const size_t smem = nbfm_fused_smem(q);
     static bool attr_set = false;
     if (!attr_set) {
-        SDRGPU_CUDA(cudaFuncSetAttribute(nbfm_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-        SDRGPU_CUDA(cudaFuncSetAttribute(nbfm_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+        SDRGPU_CUDA(cudaFuncSetAttribute(nbfm_fused_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+        SDRGPU_CUDA(cudaFuncSetAttribute(nbfm_fused_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+        SDRGPU_CUDA(cudaFuncSetAttribute(nbfm_fused_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+        SDRGPU_CUDA(cudaFuncSetAttribute(nbfm_fused_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
         attr_set = true;
     }
-    if (a.n_stages >= 1) nbfm_fused_kernel<true><<<a.n_channels, kNbfmThreads, smem, a.stream>>>(q, st, *a.fir);
-    else nbfm_fused_kernel<false><<<a.n_channels, kNbfmThreads, smem, a.stream>>>(q, st, *a.fir);
+    auto *kernel = a.n_stages >= 1 ? (q.status ? nbfm_fused_kernel<true, true> : nbfm_fused_kernel<true, false>)
+                                   : (q.status ? nbfm_fused_kernel<false, true> : nbfm_fused_kernel<false, false>);
+    kernel<<<a.n_channels, kNbfmThreads, smem, a.stream>>>(q, st, *a.fir);
     count_launch();
     SDRGPU_CUDA(cudaGetLastError());
     h.cur ^= 1;
@@ -698,13 +769,25 @@ bool nbfm_fused_fits(const sdrgpu_bank_config &cfg, const HalfBandTaps *stages, 
     return true;
 }
 
-sdrgpu_status fm_create(int n_channels, SquelchState **d_states)
+sdrgpu_status fm_create(int n_channels, double threshold, SquelchState **d_states, double **d_thresholds)
 {
     std::vector<SquelchState> init((size_t)n_channels);
     std::memset(init.data(), 0, sizeof(SquelchState) * (size_t)n_channels);
     for (auto &s : init) s.state = 2;  // PowerSquelch starts MUTE (PowerSquelch.java:18)
     SDRGPU_CUDA(cudaMalloc(d_states, sizeof(SquelchState) * (size_t)n_channels));
     SDRGPU_CUDA(cudaMemcpy(*d_states, init.data(), sizeof(SquelchState) * (size_t)n_channels, cudaMemcpyHostToDevice));
+    const std::vector<double> thresholds((size_t)n_channels, threshold);
+    SDRGPU_CUDA(cudaMalloc(d_thresholds, sizeof(double) * (size_t)n_channels));
+    SDRGPU_CUDA(cudaMemcpy(*d_thresholds, thresholds.data(), sizeof(double) * (size_t)n_channels, cudaMemcpyHostToDevice));
+    return SDRGPU_OK;
+}
+
+sdrgpu_status fm_set_threshold(double *d_thresholds, int n_channels, int channel, double threshold, cudaStream_t stream)
+{
+    const int first = channel < 0 ? 0 : channel, count = channel < 0 ? n_channels : 1;
+    set_threshold_kernel<<<(count + 255) / 256, 256, 0, stream>>>(d_thresholds + first, count, threshold);
+    count_launch();
+    SDRGPU_CUDA(cudaGetLastError());
     return SDRGPU_OK;
 }
 
@@ -716,7 +799,7 @@ sdrgpu_status fm_launch(const FmLaunch &a)
     const uint8_t *gate = nullptr;
     if (a.squelch) {
         squelch_gate_kernel<<<(C + 63) / 64, 64, 0, s>>>(a.in, a.in_stride, a.n, a.states, a.gate, a.in_stride, a.alpha,
-                                                         a.threshold, a.ramp, C);
+                                                         a.thresholds, a.ramp, a.status, a.status_stride, a.buffer_out, C);
         count_launch();
         SDRGPU_CUDA(cudaGetLastError());
         gate = a.gate;

@@ -28,8 +28,13 @@ struct NbfmHistory {
 // needs (*hist0).
 bool nbfm_fused_fits(const sdrgpu_bank_config &cfg, const HalfBandTaps *stages, int n_stages, int n_fir, int *hist0);
 
-// Allocates and uploads n_channels fresh channel states: squelch muted, no previous sample.
-sdrgpu_status fm_create(int n_channels, SquelchState **d_states);
+// Allocates and uploads n_channels fresh channel states (squelch muted, no previous sample) and their squelch
+// thresholds, every one `threshold` (linear power).
+sdrgpu_status fm_create(int n_channels, double threshold, SquelchState **d_states, double **d_thresholds);
+
+// Sets the squelch threshold (linear power) of one channel, or of every channel with channel = -1, in stream order:
+// the FM launches enqueued after it use the new value.
+sdrgpu_status fm_set_threshold(double *d_thresholds, int n_channels, int channel, double threshold, cudaStream_t stream);
 
 // what one FM launch reads and advances
 struct FmLaunch {
@@ -38,12 +43,16 @@ struct FmLaunch {
     int n;                     // samples per channel in `in`
     int n_channels;
     int squelch;               // SquelchingFMDemodulator (else FMDemodulator: every sample demodulated)
-    double alpha, threshold;
+    double alpha;
+    const double *thresholds;  // [C] squelch thresholds (linear power)
     int ramp;
     float gain;
     SquelchState *states;
     float *out;                // [C][n / decimation] demodulated floats, may be null
     long long out_stride;
+    uint8_t *status;           // with squelch, may be null: [C][status_stride] one squelch status byte per assembler
+    long long status_stride;   // buffer (SDRGPU_SQUELCH_*: state after its last sample | CHANGED)
+    int buffer_out;            // demodulated samples per assembler buffer
     uint8_t *gate;             // without `fused`, with squelch: [C][in_stride] gate bytes
     NbfmHistory *fused;        // non-null: nbfm_fused_kernel filters `in` behind this history and flips it
     int n_stages;              // the fused kernel's decimation cascade and FIR

@@ -107,16 +107,19 @@ class Bank:
         per_block = self.block_size // max(self.decimation, 1)
         return blocks, blocks * per_block
 
-    def process(self, iq, want_filtered=False):
+    def process(self, iq, want_filtered=False, want_squelch=False):
         """iq: float32 [C, 2*n] (interleaved I/Q per channel row).  Returns
         DQPSK: list of uint8 dibit arrays per channel (and the AGC output [C, 2*n_out] if want_filtered)
-        FM:    float32 [C, n_out] demodulated samples;  NONE: float32 [C, 2*n_out] filtered complex stream."""
+        FM:    float32 [C, n_out] demodulated samples;  NONE: float32 [C, 2*n_out] filtered complex stream.
+        want_squelch (FM_SQUELCH banks): also uint8 [C, buffers] squelch statuses, one per assembler buffer consumed
+        (native.SQUELCH_ATTACK .. _UNMUTE | native.SQUELCH_CHANGED), i.e. (demodulated, statuses)."""
         iq = native.f32(iq)
         if iq.ndim == 1:
             iq = iq.reshape(1, -1)
         assert iq.shape[0] == self.n_channels and iq.shape[1] % 2 == 0
         n = iq.shape[1] // 2
         blocks, n_out = self._outputs_for(n)
+        status = self._status_rows(blocks) if want_squelch else None
         self._pending = (self._pending + n) % self.block_size
         counts = np.zeros(self.n_channels, np.int32)
         L = native.lib()
@@ -131,9 +134,27 @@ class Bank:
             return (out, filt[:, :2 * n_out]) if want_filtered else out
         width = n_out if self.is_fm else 2 * n_out
         dem = np.zeros((self.n_channels, max(width, 1)), np.float32)
-        native.check(L.sdrgpu_bank_process(self._h, native.ptr(iq), iq.shape[1], n, native.HOST, None, 0, native.ptr(dem),
-                                           dem.shape[1], native.ptr(counts), native.HOST))
+        native.check(L.sdrgpu_bank_process(self._h, native.ptr(iq), iq.shape[1], n, native.HOST, native.ptr(status),
+                                           status.shape[1] if status is not None else 0, native.ptr(dem), dem.shape[1],
+                                           native.ptr(counts), native.HOST))
+        if status is not None:
+            return dem[:, :width], status[:, :blocks]
         return dem[:, :width]
+
+    def _status_rows(self, blocks):
+        """host rows for the squelch statuses of a call that consumes `blocks` buffers (turns the bank's status
+        reporting on)"""
+        if self.demod != native.DEMOD_FM_SQUELCH:
+            raise native.IllegalArgumentException("squelch statuses come from SquelchingFMDemodulator banks only")
+        if not getattr(self, "_reporting", False):
+            native.check(native.lib().sdrgpu_bank_set_squelch_reporting(self._h, 1))
+            self._reporting = True
+        return np.zeros((self.n_channels, max(blocks, 1)), np.uint8)
+
+    def setSquelchThreshold(self, threshold_db, channel=-1):
+        """PowerSquelch.setSquelchThreshold (dB) of one channel, or of every channel (channel = -1), from the next
+        buffer on; the squelch's IIR and ramp state carry on"""
+        native.check(native.lib().sdrgpu_bank_set_squelch_threshold(self._h, int(channel), float(threshold_db)))
 
     def correctInversion(self, channel, radians):
         native.check(native.lib().sdrgpu_bank_correct_inversion(self._h, int(channel), float(radians)))
@@ -236,9 +257,10 @@ class Pipeline:
     def setDeviceChunks(self, chunks):
         native.check(native.lib().sdrgpu_pipeline_set_device_chunks(self._h, int(chunks)))
 
-    def process(self, samples, samples_mem=native.HOST, n_floats=None):
+    def process(self, samples, samples_mem=native.HOST, n_floats=None, want_squelch=False):
         """samples: interleaved tuner I/Q in the channelizer's input format (one array, or one per tuner).  Returns
-        per-channel dibit arrays (DQPSK) or demod floats, indexed by bank row."""
+        per-channel dibit arrays (DQPSK) or demod floats, indexed by bank row.  want_squelch: every FM_SQUELCH bank's
+        result is (demodulated, squelch statuses), as Bank.process gives them."""
         L = native.lib()
         bank = self.bank
         multi = len(self.channelizers) > 1
@@ -256,7 +278,7 @@ class Pipeline:
         n_out = blocks * (bank.block_size // max(bank.decimation, 1))
         self._pending = (self._pending + n) % bank.block_size
         if self.routed:
-            return self._process_routed(in_ptrs, n_floats, samples_mem, blocks)
+            return self._process_routed(in_ptrs, n_floats, samples_mem, blocks, want_squelch)
         counts = np.zeros(bank.n_channels, np.int32)
         if bank.is_dqpsk:
             stride = max(16, n_out // 3 + 16)
@@ -266,11 +288,15 @@ class Pipeline:
             return [symbols[c, :counts[c]].copy() for c in range(bank.n_channels)]
         width = n_out if bank.is_fm else 2 * n_out
         dem = np.zeros((bank.n_channels, max(width, 1)), np.float32)
-        native.check(L.sdrgpu_pipeline_process_multi(self._h, in_ptrs, n_floats, samples_mem, None, 0, native.ptr(dem),
+        status = bank._status_rows(blocks) if want_squelch else None
+        native.check(L.sdrgpu_pipeline_process_multi(self._h, in_ptrs, n_floats, samples_mem, native.ptr(status),
+                                                     status.shape[1] if status is not None else 0, native.ptr(dem),
                                                      dem.shape[1], native.ptr(counts), native.HOST))
+        if status is not None:
+            return dem[:, :width], status[:, :blocks]
         return dem[:, :width]
 
-    def _process_routed(self, in_ptrs, n_floats, samples_mem, blocks):
+    def _process_routed(self, in_ptrs, n_floats, samples_mem, blocks, want_squelch=False):
         """every bank's outputs in the shape Pipeline.process gives for one bank: dibit arrays per row (DQPSK), else
         demodulated floats [rows, n]"""
         outs = (native.BankOutput * len(self.banks))()
@@ -287,14 +313,19 @@ class Pipeline:
                 width = n_out if bank.is_fm else 2 * n_out
                 buf = np.zeros((bank.n_channels, max(width, 1)), np.float32)
                 o.demod, o.demod_stride_floats = buf.ctypes.data, buf.shape[1]
-            keep.append((bank, buf, counts, n_out))
+            status = None
+            if want_squelch and bank.demod == native.DEMOD_FM_SQUELCH:
+                status = bank._status_rows(blocks)
+                o.symbols, o.symbol_stride = status.ctypes.data, status.shape[1]
+            keep.append((bank, buf, counts, n_out, status))
         native.check(native.lib().sdrgpu_pipeline_process_routed(self._h, in_ptrs, n_floats, samples_mem, outs, native.HOST))
         result = []
-        for bank, buf, counts, n_out in keep:
+        for bank, buf, counts, n_out, status in keep:
             if bank.is_dqpsk:
                 result.append([buf[c, :counts[c]].copy() for c in range(bank.n_channels)])
             else:
-                result.append(buf[:, :n_out if bank.is_fm else 2 * n_out])
+                dem = buf[:, :n_out if bank.is_fm else 2 * n_out]
+                result.append((dem, status[:, :blocks]) if status is not None else dem)
         return result
 
     def submit(self, samples):
@@ -465,15 +496,35 @@ class FMDemodulator(_LazyBank):
 
 
 class SquelchingFMDemodulator(_LazyBank):
-    """SquelchingFMDemodulator(alpha, threshold, ramp).demodulate(buffer) -> float[]"""
+    """SquelchingFMDemodulator(alpha, threshold, ramp).demodulate(buffer) -> float[], and the squelch questions
+    NBFMDecoder asks after each buffer: isSquelchChanged(), isMuted(), setSquelchThreshold(db)."""
 
     def __init__(self, alpha, threshold, ramp, sampleRate=25000.0):
         super().__init__(sample_rate=sampleRate, demod=native.DEMOD_FM_SQUELCH, squelch_alpha=alpha,
                          squelch_threshold_db=threshold, squelch_ramp=ramp)
+        self._status = native.SQUELCH_MUTE      # PowerSquelch starts muted
 
     def demodulate(self, samples):
         samples = native.f32(samples)
-        return self._get(samples.size // 2).process(samples.reshape(1, -1))[0]
+        dem, status = self._get(samples.size // 2).process(samples.reshape(1, -1), want_squelch=True)
+        self._status = int(status[0, -1])
+        return dem[0]
+
+    def isSquelchChanged(self):
+        """the squelch changed state at least once during the last demodulate(buffer)"""
+        return bool(self._status & native.SQUELCH_CHANGED)
+
+    def isMuted(self):
+        """passing no audio after the last buffer: the squelch is in MUTE or ATTACK, the states in which demodulate
+        writes 0.0f (the reference's class has no such query; NBFMDecoder's use of the squelch state means this)"""
+        return (self._status & 3) in (native.SQUELCH_MUTE, native.SQUELCH_ATTACK)
+
+    def setSquelchThreshold(self, threshold):
+        """PowerSquelch.setSquelchThreshold(dB): used from the next buffer on"""
+        if self._bank is None:
+            self._kw["squelch_threshold_db"] = float(threshold)
+        else:
+            self._bank.setSquelchThreshold(threshold)
 
 
 class CostasLoop:

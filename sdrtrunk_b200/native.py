@@ -22,6 +22,7 @@ SYNC_NONE, SYNC_P25_PHASE1, SYNC_P25_PHASE2, SYNC_P25_PHASE2_FRAMED = 0, 1, 2, 3
 P2_EVENT_FRAGMENT, P2_EVENT_SYNC_LOSS, P2_EVENT_INVERSION, P2_EVENT_SYNCHRONIZED = 1, 2, 4, 32
 (SYNC_EVENT_NONE, SYNC_EVENT_SYNC, SYNC_EVENT_INVERSION_90_CW, SYNC_EVENT_INVERSION_90_CCW, SYNC_EVENT_INVERSION_180,
  SYNC_EVENT_LOST) = range(6)
+SQUELCH_ATTACK, SQUELCH_DECAY, SQUELCH_MUTE, SQUELCH_UNMUTE, SQUELCH_CHANGED = 0, 1, 2, 3, 4
 
 OK, ERR_INVALID_ARG, ERR_BAD_STATE, ERR_CUDA, ERR_OVERFLOW, ERR_DESIGN, ERR_NOMEM = range(7)
 
@@ -129,6 +130,8 @@ PROTOTYPES = {
     "sdrgpu_bank_read_symbol_tap": (C.c_int, [_vp, C.POINTER(C.c_double), C.c_int, _i32p]),
     "sdrgpu_bank_reset_pll": (C.c_int, [_vp, C.c_int]),
     "sdrgpu_bank_get_loop_state": (C.c_int, [_vp, C.c_int, C.POINTER(C.c_double)]),
+    "sdrgpu_bank_set_squelch_reporting": (C.c_int, [_vp, C.c_int]),
+    "sdrgpu_bank_set_squelch_threshold": (C.c_int, [_vp, C.c_int, C.c_double]),
     "sdrgpu_pack_dibits": (C.c_int, [_u8p, C.c_int, _u8p]),
     "sdrgpu_bank_enable_timing": (C.c_int, [_vp, C.c_int]),
     "sdrgpu_bank_last_kernel_ms": (C.c_int, [_vp, _f32p]),
