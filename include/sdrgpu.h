@@ -179,9 +179,24 @@ typedef struct {
  * offset).  synthesis_filter (may be NULL if no two-bin channel) = getSincM2Synthesizer taps.  Two-bin channels run
  * TwoChannelSynthesizerM2 + FS4DownConverter + the frequency-correction Oscillator (always, as
  * TwoChannelOutputProcessor.java:113 does); one-bin channels run the Oscillator only with a non-zero offset
- * (OneChannelOutputProcessor.java:92-95).  Selecting resets the oscillators and synthesizer histories. */
+ * (OneChannelOutputProcessor.java:92-95).  Selecting resets the oscillators and synthesizer histories: to change only
+ * the frequency offsets of selected channels without that reset, use sdrgpu_chan_set_frequency_offsets. */
 sdrgpu_status sdrgpu_chan_select(sdrgpu_channelizer *h, const sdrgpu_output_channel *channels, int n_channels,
                                  const float *synthesis_filter, int n_synthesis_taps);
+
+/* ChannelOutputProcessor.setFrequencyOffset for running channels: channels[i] is an index into the current selection
+ * (sdrgpu_chan_select order), offsets_hz[i] its new offset.  It takes effect from the first output block of the next
+ * call that runs this channelizer (sdrgpu_chan_process or any pipeline call, including the next submit); calls
+ * already enqueued, such as submitted pipeline calls not yet waited for, keep the old offsets.  As in the reference only
+ * the oscillator's angle changes: the next sample is mixed with the phasor the old angle produced, and two-bin
+ * channels keep their synthesizer history and FS/4 position.  A one-bin channel whose offset goes to 0 stops mixing
+ * and holds its phasor; when its offset becomes nonzero again it resumes from that phasor ((0, -1) if it has not
+ * mixed since the selection).  Such a switch waits for the channelizer's work in flight; a change between nonzero
+ * offsets does not.  Other channels, the selection and any pipeline built on it are untouched.  SDRGPU_ERR_INVALID_ARG
+ * for NULL arguments, n <= 0, an index out of range or listed twice; SDRGPU_ERR_BAD_STATE for a nonzero offset
+ * before sdrgpu_chan_set_sample_rate; a refused call changes nothing. */
+sdrgpu_status sdrgpu_chan_set_frequency_offsets(sdrgpu_channelizer *h, const int *channels, const long long *offsets_hz,
+                                                int n);
 
 enum {
     SDRGPU_LAYOUT_RESULTS = 0, /* [n_blocks][2*M] floats: ReusableChannelResultsBuffer, all bins, no gain */

@@ -83,8 +83,10 @@ public class GpuChannelOutputProcessor implements IPolyphaseChannelOutputProcess
     @Override
     public void setFrequencyOffset(long frequency)
     {
+        //only the oscillator's angle changes (ChannelOutputProcessor.java:91-95): applied before the next buffer without
+        //re-selecting, so the other channels of the tuner keep their oscillators and synthesizers
         mFrequencyOffset = frequency;
-        mChannelizer.selectionChanged();
+        mChannelizer.frequencyOffsetChanged(this);
     }
 
     @Override

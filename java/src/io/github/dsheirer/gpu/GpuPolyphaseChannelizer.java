@@ -15,12 +15,15 @@ import io.github.dsheirer.sample.buffer.ReusableComplexBuffer;
 
 import java.lang.foreign.Arena;
 import java.lang.foreign.MemorySegment;
+import java.util.ArrayList;
 import java.util.List;
+import java.util.concurrent.ConcurrentLinkedQueue;
 import java.util.concurrent.CopyOnWriteArrayList;
 
 import static java.lang.foreign.ValueLayout.ADDRESS;
 import static java.lang.foreign.ValueLayout.JAVA_FLOAT;
 import static java.lang.foreign.ValueLayout.JAVA_INT;
+import static java.lang.foreign.ValueLayout.JAVA_LONG;
 
 public class GpuPolyphaseChannelizer extends AbstractComplexPolyphaseChannelizer
 {
@@ -35,6 +38,7 @@ public class GpuPolyphaseChannelizer extends AbstractComplexPolyphaseChannelizer
     private int mMaxInputFloats;
     private int mMaxBlocks;
     private boolean mSelectionChanged = true;
+    private final ConcurrentLinkedQueue<GpuChannelOutputProcessor> mOffsetsChanged = new ConcurrentLinkedQueue<>();
 
     /**
      * @param taps prototype low-pass filter, channelCount * tapsPerChannel long (FilterFactory.getSincM2Channelizer)
@@ -102,6 +106,56 @@ public class GpuPolyphaseChannelizer extends AbstractComplexPolyphaseChannelizer
         mSelectionChanged = true;
     }
 
+    /** a registered processor's offset changed: sent with the others changed since the last buffer (updateOffsets) */
+    void frequencyOffsetChanged(GpuChannelOutputProcessor processor)
+    {
+        mOffsetsChanged.add(processor);
+    }
+
+    /**
+     * sdrgpu_chan_set_frequency_offsets for the processors whose offset changed since the last buffer: the index of each
+     * in the selection (registration order) and its current offset.  Not needed after a re-selection, which carries the
+     * offsets itself.
+     */
+    private void updateOffsets() throws Throwable
+    {
+        List<GpuChannelOutputProcessor> processors = mProcessors;
+        List<Integer> indexes = new ArrayList<>();
+        List<Long> offsets = new ArrayList<>();
+        GpuChannelOutputProcessor changed;
+
+        while((changed = mOffsetsChanged.poll()) != null)
+        {
+            int index = processors.indexOf(changed);
+
+            if(index >= 0 && !indexes.contains(index))
+            {
+                indexes.add(index);
+                offsets.add(changed.getFrequencyOffset());
+            }
+        }
+
+        if(indexes.isEmpty())
+        {
+            return;
+        }
+
+        try(Arena arena = Arena.ofConfined())
+        {
+            int n = indexes.size();
+            MemorySegment nativeIndexes = arena.allocate(JAVA_INT, n);
+            MemorySegment nativeOffsets = arena.allocate(JAVA_LONG, n);
+
+            for(int i = 0; i < n; i++)
+            {
+                nativeIndexes.setAtIndex(JAVA_INT, i, indexes.get(i));
+                nativeOffsets.setAtIndex(JAVA_LONG, i, offsets.get(i));
+            }
+
+            SdrGpu.check((int)SdrGpu.CHAN_SET_FREQUENCY_OFFSETS.invokeExact(mHandle, nativeIndexes, nativeOffsets, n));
+        }
+    }
+
     /** sdrgpu_chan_select: one sdrgpu_output_channel per registered processor, in registration order */
     private void updateSelection() throws Throwable
     {
@@ -159,7 +213,12 @@ public class GpuPolyphaseChannelizer extends AbstractComplexPolyphaseChannelizer
         {
             if(mSelectionChanged)
             {
+                mOffsetsChanged.clear();   //the selection carries every processor's current offset
                 updateSelection();
+            }
+            else
+            {
+                updateOffsets();
             }
 
             List<GpuChannelOutputProcessor> processors = mProcessors;

@@ -76,6 +76,10 @@ public final class SdrGpu
     static final MethodHandle CHAN_SET_INPUT_FORMAT = h("sdrgpu_chan_set_input_format", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT));
     static final MethodHandle CHAN_SELECT = h("sdrgpu_chan_select",
         FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS, JAVA_INT));
+    /** (channelizer, int[] selection indexes, long[] offsets Hz, n): ChannelOutputProcessor.setFrequencyOffset for running
+     *  channels, from the next process call on; only the oscillator angles change */
+    static final MethodHandle CHAN_SET_FREQUENCY_OFFSETS = h("sdrgpu_chan_set_frequency_offsets",
+        FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_INT));
     static final MethodHandle CHAN_PROCESS = h("sdrgpu_chan_process",
         FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, ADDRESS, JAVA_LONG, JAVA_INT, JAVA_INT, ADDRESS));
     static final MethodHandle CHAN_BLOCKS_FOR = h("sdrgpu_chan_blocks_for", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT));

@@ -687,10 +687,9 @@ struct sdrgpu_channelizer {
 
 namespace {
 
-sdrgpu_status upload_selection(sdrgpu_channelizer *h)
+// the filter bank's rows and gains for the output stage's rows `r`, and the store paths they allow
+sdrgpu_status upload_rows(sdrgpu_channelizer *h, const OutputRows &r)
 {
-    OutputRows r;
-    SDRGPU_TRY(outputs_select(h->outputs, h->channels, h->M, h->sample_rate, h->max_blocks, &r));
     const int n = (int)h->channels.size(), rows = (int)r.sel.size();
     std::vector<float> gf(rows);
     int exact = 1;
@@ -720,6 +719,13 @@ sdrgpu_status upload_selection(sdrgpu_channelizer *h)
         if (r.sel[i] != i || gf[i] != gf[0]) h->identity = 0;
     h->gain_uniform = n > 0 ? gf[0] : 0.0f;
     return SDRGPU_OK;
+}
+
+sdrgpu_status upload_selection(sdrgpu_channelizer *h)
+{
+    OutputRows r;
+    SDRGPU_TRY(outputs_select(h->outputs, h->channels, h->M, h->sample_rate, h->max_blocks, &r));
+    return upload_rows(h, r);
 }
 
 template <int M, int R1, int R2, int NB, int TT, int NT, int MINB, bool RAW, bool ROUTED>
@@ -1263,6 +1269,39 @@ sdrgpu_status sdrgpu_chan_select(sdrgpu_channelizer *h, const sdrgpu_output_chan
     SDRGPU_CUDA(cudaStreamSynchronize(h->stream));
     h->channels.assign(channels, channels + n_channels);
     return upload_selection(h);
+}
+
+sdrgpu_status sdrgpu_chan_set_frequency_offsets(sdrgpu_channelizer *h, const int *channels, const long long *offsets_hz, int n)
+{
+    if (!h || !channels || !offsets_hz || n <= 0) return fail(SDRGPU_ERR_INVALID_ARG, "NULL / empty argument");
+    const int n_sel = (int)h->channels.size();
+    std::vector<char> seen((size_t)n_sel, 0);
+    bool any_offset = false;
+    for (int i = 0; i < n; i++) {
+        if (channels[i] < 0 || channels[i] >= n_sel)
+            return fail(SDRGPU_ERR_INVALID_ARG, "channel %d is not in the selection of %d channels", channels[i], n_sel);
+        if (seen[(size_t)channels[i]]) return fail(SDRGPU_ERR_INVALID_ARG, "channel %d is listed twice", channels[i]);
+        seen[(size_t)channels[i]] = 1;
+        any_offset |= offsets_hz[i] != 0;
+    }
+    if (any_offset && !(h->sample_rate > 0.0))
+        return fail(SDRGPU_ERR_BAD_STATE, "frequency-corrected channels need sdrgpu_chan_set_sample_rate first");
+    // a repeat of a channel's offset changes nothing (Oscillator.update computes the same angle)
+    std::vector<sdrgpu_output_channel> next = h->channels;
+    std::vector<int> changed;
+    for (int i = 0; i < n; i++)
+        if (next[(size_t)channels[i]].frequency_offset_hz != offsets_hz[i]) {
+            next[(size_t)channels[i]].frequency_offset_hz = offsets_hz[i];
+            changed.push_back(channels[i]);
+        }
+    if (changed.empty()) return SDRGPU_OK;
+    SDRGPU_CUDA(cudaSetDevice(h->device));
+    OutputRows r;
+    bool rows_changed = false;
+    h->channels = next;
+    SDRGPU_TRY(outputs_set_offsets(h->outputs, h->channels, changed, h->M, h->sample_rate, h->stream, &r, &rows_changed));
+    if (rows_changed) SDRGPU_TRY(upload_rows(h, r));
+    return SDRGPU_OK;
 }
 
 int sdrgpu_chan_blocks_for(const sdrgpu_channelizer *h, int n_floats)

@@ -2,6 +2,7 @@
 // a frequency offset (osc_produce_kernel + osc_mix_kernel, or pfb2_kernel mixing the oscillators in where it stores).
 // The filter bank leaves their rows at gain 1 (bin values after the 1/M of the inverse FFT); this stage finishes them in
 // place on the channelizer's stream.
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <vector>
@@ -123,16 +124,10 @@ __global__ void __launch_bounds__(32) post_channel_kernel(float *out, long long 
 // (AbstractOscillator.mixComplex, J/dsp/mixer/AbstractOscillator.java:102-116: sample * current, then rotate();
 // Oscillator.rotate + Complex.fastNormalize, J/dsp/mixer/Oscillator.java:42-68.)
 // ---------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(32) osc_produce_kernel(const MixChannel *__restrict__ chans, float2 *__restrict__ state,
-                                                           float2 *__restrict__ ring, int ring_len, long long start, int count,
-                                                           int n_mix)
+// The `count` oscillator values from `cur` on into ring slots pos, pos + 1, ... (wrapping at ring_len); leaves cur at the
+// value after them
+__device__ __forceinline__ void osc_fill(float2 *r, int ring_len, int pos, int count, float2 &cur, float2 angle)
 {
-    const int ch = blockIdx.x * blockDim.x + threadIdx.x;
-    if (ch >= n_mix) return;
-    const float2 angle = make_float2(chans[ch].angle_i, chans[ch].angle_q);
-    float2 cur = state[ch];
-    float2 *r = ring + (size_t)ch * ring_len;
-    int pos = (int)(start % ring_len);
     int k = 0;
     while (k < count) {
         if ((pos & 1) == 0 && k + 8 <= count && pos + 8 <= ring_len) {
@@ -160,7 +155,80 @@ __global__ void __launch_bounds__(32) osc_produce_kernel(const MixChannel *__res
         }
         if (pos >= ring_len) pos = 0;
     }
+}
+
+__global__ void __launch_bounds__(32) osc_produce_kernel(const MixChannel *__restrict__ chans, float2 *__restrict__ state,
+                                                           float2 *__restrict__ ring, int ring_len, long long start, int count,
+                                                           int n_mix)
+{
+    const int ch = blockIdx.x * blockDim.x + threadIdx.x;
+    if (ch >= n_mix) return;
+    const float2 angle = make_float2(chans[ch].angle_i, chans[ch].angle_q);
+    float2 cur = state[ch];
+    float2 *r = ring + (size_t)ch * ring_len;
+    const int pos = (int)(start % ring_len);
+    osc_fill(r, ring_len, pos, count, cur, angle);
     state[ch] = cur;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// A new frequency offset for running one-bin channels (ChannelOutputProcessor.setFrequencyOffset -> Oscillator.update:
+// only the angle changes).  The rings hold the values of blocks start .. start + count - 1 (slot k % ring_len: the phasor
+// that multiplies block k), produced with the old angle.  Slot `start` stays: the next block is mixed with the phasor the
+// old angle produced.  Slots start + 1 .. start + count - 1 and the producer's state are rewritten from it with the new
+// angle, one thread per changed channel, with the producer's arithmetic.  A channel that starts mixing (held_row >= 0)
+// starts from the phasor it held, which also goes into slot `start`.  Calls still in flight read slots below `start`
+// only, and ring_len = 2 max_blocks + 9 > count, so no slot they read is rewritten.
+// ---------------------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(32) osc_reproduce_kernel(MixChannel *__restrict__ chans, float2 *__restrict__ state,
+                                                             float2 *__restrict__ ring, int ring_len, long long start, int count,
+                                                             const float2 *__restrict__ held,
+                                                             const __grid_constant__ OffsetChanges changes)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= changes.n) return;
+    const OffsetChange c = changes.c[i];
+    const float2 angle = make_float2(c.angle_i, c.angle_q);
+    // the producer's angle from here on (it runs on this kernel's stream)
+    chans[c.index].angle_i = c.angle_i;
+    chans[c.index].angle_q = c.angle_q;
+    float2 *r = ring + (size_t)c.index * ring_len;
+    const int pos = (int)(start % ring_len);
+    float2 cur = c.held_row >= 0 ? held[c.held_row] : (count > 0 ? r[pos] : state[c.index]);
+    if (count > 0) {
+        if (c.held_row >= 0) r[pos] = cur;
+        cur = osc_rotate(cur, angle);
+        osc_fill(r, ring_len, pos + 1 == ring_len ? 0 : pos + 1, count - 1, cur, angle);
+    }
+    state[c.index] = cur;
+}
+
+// two-bin channels: the synthesizer's Oscillator takes the new angle, on the channelizer's stream
+__global__ void post_angle_kernel(PostChannel *chans, const __grid_constant__ OffsetChanges changes)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= changes.n) return;
+    chans[changes.c[i].index].angle_i = changes.c[i].angle_i;
+    chans[changes.c[i].index].angle_q = changes.c[i].angle_q;
+}
+
+// The mix set changes (a one-bin channel starts or stops mixing): one block per old mix channel m.  A kept channel's
+// live ring window (blocks start .. start + count - 1) and producer state move to its new row dst[m]; a channel that
+// stops mixing holds the phasor its next block would have used.
+__global__ void osc_carry_kernel(const MixChannel *old_chans, const float2 *old_state, const float2 *old_ring, const int *dst,
+                                 float2 *state, float2 *ring, float2 *held, int ring_len, long long start, int count)
+{
+    const int m = blockIdx.x, d = dst[m];
+    const float2 *src = old_ring + (size_t)m * ring_len;
+    if (d < 0) {
+        if (threadIdx.x == 0) held[old_chans[m].row] = count > 0 ? src[start % ring_len] : old_state[m];
+        return;
+    }
+    for (int k = threadIdx.x; k < count; k += blockDim.x) {
+        const int pos = (int)((start + k) % ring_len);
+        ring[(size_t)d * ring_len + pos] = src[pos];
+    }
+    if (threadIdx.x == 0) state[d] = old_state[m];
 }
 
 // grid (ceil(n / 256), n_mix): row[k] = (float)((double)(row[k] * osc[start + k]) * gain)
@@ -237,6 +305,7 @@ cudaError_t free_buffers(ChanOutputs &o)
     release(o.d_mix);
     release(o.d_mix_state);
     release(o.d_osc);
+    release(o.d_held);
     o.osc_produced = o.osc_consumed = o.osc_safe = 0;
     o.osc_pending = false;
     return e;
@@ -250,19 +319,31 @@ sdrgpu_status upload(T **d, const std::vector<T> &v)
     return SDRGPU_OK;
 }
 
-}  // namespace
+// Oscillator.update: anglePerSample = (float)(2 pi f / fs) at the channel rate; Complex.fromAngle(float) -> (float)cos, (float)sin
+void osc_angle(long long offset_hz, int M, double sample_rate, float *angle_i, float *angle_q)
+{
+    const double channel_rate = 2.0 * sample_rate / (double)M;
+    const float angle = (float)(2.0 * 3.14159265358979323846 * (double)offset_hz / channel_rate);
+    *angle_i = (float)cos((double)angle);
+    *angle_q = (float)sin((double)angle);
+}
 
-sdrgpu_status sdrgpu::outputs_select(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &channels, int M,
-                                     double sample_rate, int max_blocks, OutputRows *rows)
+// The stage's tables for a selection: the filter bank's rows, the two-bin (post) and one-bin + offset (mix) channels, and
+// each selected channel's row in those tables (post_of / mix_of, -1: none)
+void plan_outputs(const std::vector<sdrgpu_output_channel> &channels, int M, double sample_rate, OutputRows *rows,
+                  std::vector<PostChannel> *post, std::vector<MixChannel> *mix, std::vector<int> *post_of,
+                  std::vector<int> *mix_of, int *n_two)
 {
     const int n = (int)channels.size();
     std::vector<int> &sel = rows->sel;
     std::vector<double> &gd = rows->gain;
     sel.clear();
     gd.clear();
-    std::vector<PostChannel> post;
-    std::vector<MixChannel> mix;
-    int n_two = 0;
+    post->clear();
+    mix->clear();
+    post_of->assign(n, -1);
+    mix_of->assign(n, -1);
+    *n_two = 0;
     for (int i = 0; i < n; i++) {
         const sdrgpu_output_channel &c = channels[i];
         const bool special = c.bin2 >= 0 || c.frequency_offset_hz != 0;
@@ -272,17 +353,18 @@ sdrgpu_status sdrgpu::outputs_select(ChanOutputs &o, const std::vector<sdrgpu_ou
         if (special) {
             PostChannel pc{};
             pc.row = i;
-            pc.row2 = c.bin2 >= 0 ? n_two++ : -1;
+            pc.row2 = c.bin2 >= 0 ? (*n_two)++ : -1;
             // TwoChannelOutputProcessor mixes unconditionally, OneChannelOutputProcessor only with an offset
             pc.mix = 1;
-            // Oscillator.update: anglePerSample = (float)(2 pi f / fs); Complex.fromAngle(float) -> (float)cos, (float)sin
-            const double channel_rate = 2.0 * sample_rate / (double)M;
-            const float angle = (float)(2.0 * 3.14159265358979323846 * (double)c.frequency_offset_hz / channel_rate);
-            pc.angle_i = (float)cos((double)angle);
-            pc.angle_q = (float)sin((double)angle);
+            osc_angle(c.frequency_offset_hz, M, sample_rate, &pc.angle_i, &pc.angle_q);
             pc.gain = c.gain;
-            if (c.bin2 >= 0) post.push_back(pc);                                        // two-bin: post_channel_kernel
-            else mix.push_back(MixChannel{pc.row, pc.angle_i, pc.angle_q, pc.gain});    // one bin + offset: look-ahead
+            if (c.bin2 >= 0) {   // two-bin: post_channel_kernel
+                (*post_of)[i] = (int)post->size();
+                post->push_back(pc);
+            } else {             // one bin + offset: look-ahead
+                (*mix_of)[i] = (int)mix->size();
+                mix->push_back(MixChannel{pc.row, pc.angle_i, pc.angle_q, pc.gain});
+            }
         }
     }
     for (int i = 0; i < n; i++)
@@ -290,16 +372,101 @@ sdrgpu_status sdrgpu::outputs_select(ChanOutputs &o, const std::vector<sdrgpu_ou
             sel.push_back(channels[i].bin2);
             gd.push_back(1.0);
         }
-    rows->mix_identity = (int)mix.size() == n && n == M && (int)sel.size() == n;
-    for (size_t m = 0; m < mix.size() && rows->mix_identity; m++)
-        if (mix[m].row != (int)m || sel[m] != (int)m || mix[m].gain != mix[0].gain || (double)(float)mix[m].gain != mix[m].gain)
+    rows->mix_identity = (int)mix->size() == n && n == M && (int)sel.size() == n;
+    for (size_t m = 0; m < mix->size() && rows->mix_identity; m++) {
+        const MixChannel &x = (*mix)[m];
+        if (x.row != (int)m || sel[m] != (int)m || x.gain != (*mix)[0].gain || (double)(float)x.gain != x.gain)
             rows->mix_identity = false;
-    rows->mix_gain = mix.empty() ? 0.0f : (float)mix[0].gain;
+    }
+    rows->mix_gain = mix->empty() ? 0.0f : (float)(*mix)[0].gain;
+}
+
+sdrgpu_status ensure_osc_stream(ChanOutputs &o)
+{
+    if (o.osc_stream) return SDRGPU_OK;
+    SDRGPU_CUDA(cudaStreamCreateWithFlags(&o.osc_stream, cudaStreamNonBlocking));
+    SDRGPU_CUDA(cudaEventCreateWithFlags(&o.ev_mix, cudaEventDisableTiming));
+    SDRGPU_CUDA(cudaEventCreateWithFlags(&o.ev_osc, cudaEventDisableTiming));
+    return SDRGPU_OK;
+}
+
+// the OffsetChanges launches of a change list, kMaxOffsetChanges at a time
+template <class Launch>
+sdrgpu_status launch_changes(const std::vector<OffsetChange> &list, Launch launch)
+{
+    for (size_t first = 0; first < list.size(); first += kMaxOffsetChanges) {
+        OffsetChanges c;
+        c.n = (int)std::min(list.size() - first, (size_t)kMaxOffsetChanges);
+        std::memcpy(c.c, list.data() + first, sizeof(OffsetChange) * (size_t)c.n);
+        launch(c);
+        count_launch();
+        SDRGPU_CUDA(cudaGetLastError());
+    }
+    return SDRGPU_OK;
+}
+
+// The mix set changes: new tables `mix` (mix_of: each selected channel's row in them), every kept channel's ring window
+// and state carried over, the phasors of channels that stop mixing held.  The caller has waited for the work in flight.
+sdrgpu_status rebuild_mix(ChanOutputs &o, const std::vector<MixChannel> &mix, const std::vector<int> &mix_of)
+{
+    const int n_old = o.n_mix, n_new = (int)mix.size();
+    if (n_old == 0) o.osc_produced = o.osc_consumed;   // no ring: nothing ahead
+    const long long start = o.osc_consumed;
+    const int count = (int)(o.osc_produced - o.osc_consumed);
+    if (n_new > 0) {
+        SDRGPU_TRY(ensure_osc_stream(o));
+        o.osc_ring_len = (2 * o.max_blocks + 8 + 1) & ~1;   // as outputs_select
+    }
+    MixChannel *d_mix = nullptr;
+    float2 *d_state = nullptr, *d_osc = nullptr;
+    if (n_new > 0) {
+        SDRGPU_TRY(upload(&d_mix, mix));
+        SDRGPU_CUDA(cudaMalloc(&d_state, sizeof(float2) * (size_t)n_new));
+        SDRGPU_CUDA(cudaMalloc(&d_osc, sizeof(float2) * (size_t)n_new * (size_t)o.osc_ring_len));
+    }
+    if (n_old > 0) {
+        std::vector<int> dst(n_old, -1);
+        for (size_t i = 0; i < o.mix_of.size(); i++)
+            if (o.mix_of[i] >= 0) dst[o.mix_of[i]] = mix_of[i];
+        int *d_dst = nullptr;
+        SDRGPU_TRY(upload(&d_dst, dst));
+        osc_carry_kernel<<<n_old, 128, 0, o.osc_stream>>>(o.d_mix, o.d_mix_state, o.d_osc, d_dst, d_state, d_osc, o.d_held,
+                                                          o.osc_ring_len, start, count);
+        count_launch();
+        const cudaError_t e = cudaGetLastError();
+        const cudaError_t s = cudaStreamSynchronize(o.osc_stream);
+        cudaFree(d_dst);
+        SDRGPU_CUDA(e);
+        SDRGPU_CUDA(s);
+    }
+    release(o.d_mix);
+    release(o.d_mix_state);
+    release(o.d_osc);
+    o.d_mix = d_mix;
+    o.d_mix_state = d_state;
+    o.d_osc = d_osc;
+    o.n_mix = n_new;
+    o.mix_of = mix_of;
+    return SDRGPU_OK;
+}
+
+}  // namespace
+
+sdrgpu_status sdrgpu::outputs_select(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &channels, int M,
+                                     double sample_rate, int max_blocks, OutputRows *rows)
+{
+    std::vector<PostChannel> post;
+    std::vector<MixChannel> mix;
+    std::vector<int> post_of, mix_of;
+    int n_two = 0;
+    plan_outputs(channels, M, sample_rate, rows, &post, &mix, &post_of, &mix_of, &n_two);
 
     SDRGPU_CUDA(free_buffers(o));
     o.max_blocks = max_blocks;
     o.n_post = 0;
     o.n_mix = 0;
+    // every channel holds the Oscillator's starting phasor until it first mixes (Oscillator.java:24)
+    SDRGPU_TRY(upload(&o.d_held, std::vector<float2>(channels.size(), make_float2(0.0f, -1.0f))));
     if (!post.empty()) {
         std::vector<PostState> init(post.size());
         std::memset(init.data(), 0, sizeof(PostState) * init.size());
@@ -313,11 +480,7 @@ sdrgpu_status sdrgpu::outputs_select(ChanOutputs &o, const std::vector<sdrgpu_ou
         SDRGPU_CUDA(cudaMalloc(&o.d_out2, sizeof(float) * 2 * (size_t)max_blocks * (size_t)n_two));
     }
     if (!mix.empty()) {
-        if (!o.osc_stream) {
-            SDRGPU_CUDA(cudaStreamCreateWithFlags(&o.osc_stream, cudaStreamNonBlocking));
-            SDRGPU_CUDA(cudaEventCreateWithFlags(&o.ev_mix, cudaEventDisableTiming));
-            SDRGPU_CUDA(cudaEventCreateWithFlags(&o.ev_osc, cudaEventDisableTiming));
-        }
+        SDRGPU_TRY(ensure_osc_stream(o));
         // two calls' worth: a pipeline tops the ring up at the START of a call, for the call after it (outputs_ahead)
         o.osc_ring_len = (2 * max_blocks + 8 + 1) & ~1;   // even: the producer stores pairs
         SDRGPU_TRY(upload(&o.d_mix, mix));
@@ -326,6 +489,66 @@ sdrgpu_status sdrgpu::outputs_select(ChanOutputs &o, const std::vector<sdrgpu_ou
     }
     o.n_post = (int)post.size();
     o.n_mix = (int)mix.size();
+    o.post_of = post_of;
+    o.mix_of = mix_of;
+    return SDRGPU_OK;
+}
+
+sdrgpu_status sdrgpu::outputs_set_offsets(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &channels,
+                                          const std::vector<int> &changed, int M, double sample_rate, cudaStream_t stream,
+                                          OutputRows *rows, bool *rows_changed)
+{
+    *rows_changed = false;
+    bool transition = false;
+    for (int i : changed)
+        if (channels[i].bin2 < 0 && (o.mix_of[i] >= 0) != (channels[i].frequency_offset_hz != 0)) transition = true;
+    std::vector<char> starts(channels.size(), 0);   // one-bin channels that start mixing
+    if (transition) {
+        // Rare (typically once per channel, at its first correction): the rows of the filter bank change, so the work in
+        // flight is waited for and the mix tables are rebuilt
+        SDRGPU_CUDA(cudaStreamSynchronize(stream));
+        if (o.osc_stream) SDRGPU_CUDA(cudaStreamSynchronize(o.osc_stream));
+        std::vector<PostChannel> post;
+        std::vector<MixChannel> mix;
+        std::vector<int> post_of, mix_of;
+        int n_two = 0;
+        plan_outputs(channels, M, sample_rate, rows, &post, &mix, &post_of, &mix_of, &n_two);
+        for (int i : changed)
+            if (channels[i].bin2 < 0 && o.mix_of[i] < 0 && mix_of[i] >= 0) starts[i] = 1;
+        SDRGPU_TRY(rebuild_mix(o, mix, mix_of));
+        *rows_changed = true;
+    }
+    std::vector<OffsetChange> post_list, mix_list;
+    for (int i : changed) {
+        OffsetChange c{};
+        c.held_row = -1;
+        osc_angle(channels[i].frequency_offset_hz, M, sample_rate, &c.angle_i, &c.angle_q);
+        if (o.post_of[i] >= 0) {
+            c.index = o.post_of[i];
+            post_list.push_back(c);
+        } else if (o.mix_of[i] >= 0) {
+            c.index = o.mix_of[i];
+            if (starts[i]) c.held_row = i;
+            mix_list.push_back(c);
+        }
+    }
+    // two-bin channels: behind the calls already enqueued on the channelizer's stream, which read the old angles
+    SDRGPU_TRY(launch_changes(post_list, [&](const OffsetChanges &c) {
+        post_angle_kernel<<<(c.n + 127) / 128, 128, 0, stream>>>(o.d_post, c);
+    }));
+    if (!mix_list.empty()) {
+        // on the side stream behind the producer in flight and the last kernel that read the rings; the next call waits
+        // for it (osc_safe below osc_consumed + its blocks)
+        if (o.mix_recorded) SDRGPU_CUDA(cudaStreamWaitEvent(o.osc_stream, o.ev_mix, 0));
+        const int count = (int)(o.osc_produced - o.osc_consumed);
+        SDRGPU_TRY(launch_changes(mix_list, [&](const OffsetChanges &c) {
+            osc_reproduce_kernel<<<(c.n + 31) / 32, 32, 0, o.osc_stream>>>(o.d_mix, o.d_mix_state, o.d_osc, o.osc_ring_len,
+                                                                           o.osc_consumed, count, o.d_held, c);
+        }));
+        SDRGPU_CUDA(cudaEventRecord(o.ev_osc, o.osc_stream));
+        o.osc_pending = true;
+        o.osc_safe = o.osc_consumed;
+    }
     return SDRGPU_OK;
 }
 

@@ -36,6 +36,19 @@ struct MixChannel {
     double gain;
 };
 
+// sdrgpu_chan_set_frequency_offsets: new angles for rows of the d_post / d_mix tables, passed by value to the kernels that
+// apply them (so nothing on the host has to outlive a launch queued behind calls in flight)
+constexpr int kMaxOffsetChanges = 1024;
+struct OffsetChange {
+    int index;              // row of d_post / d_mix
+    int held_row;           // a one-bin channel that starts mixing: its selection index (its phasor in d_held), else -1
+    float angle_i, angle_q;
+};
+struct OffsetChanges {
+    int n;
+    OffsetChange c[kMaxOffsetChanges];
+};
+
 // AbstractOscillator.mixComplex (J/dsp/mixer/AbstractOscillator.java:102-116): sample v times oscillator value z, every
 // product, difference and sum rounded on its own
 __device__ __forceinline__ float2 mix_complex(float2 v, float2 z)
@@ -73,6 +86,10 @@ struct ChanOutputs {
     cudaEvent_t ev_mix = nullptr, ev_osc = nullptr;
     bool osc_pending = false;
     bool mix_recorded = false;      // ev_mix marks the end of the last kernel that read the rings
+    // per selected channel: its row of d_post / d_mix (-1: none), and the phasor a one-bin channel holds while it does not
+    // mix (OneChannelOutputProcessor keeps its Oscillator when the offset goes to 0)
+    std::vector<int> post_of, mix_of;
+    float2 *d_held = nullptr;
 };
 
 // What the filter bank writes for a selection: the rows (each channel's first bin, then the second bins of two-bin
@@ -88,6 +105,14 @@ struct OutputRows {
 // Rebuilds the stage for a selection at this sample rate and channel count; restarts every oscillator and synthesizer.
 sdrgpu_status outputs_select(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &channels, int M, double sample_rate,
                              int max_blocks, OutputRows *rows);
+// New frequency offsets for the selected channels `changed` (channels holds every channel with its new offset), from the
+// next call on; calls already enqueued keep the old ones.  Two-bin channels and one-bin channels that keep mixing change
+// their angle in stream order and keep their oscillator, synthesizer and look-ahead (osc_reproduce_kernel).  A one-bin
+// channel that starts or stops mixing changes the filter bank's rows: the stage waits for the work in flight, rebuilds
+// the mix tables and returns the new rows in *rows (*rows_changed); otherwise *rows is untouched.
+sdrgpu_status outputs_set_offsets(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &channels,
+                                  const std::vector<int> &changed, int M, double sample_rate, cudaStream_t stream,
+                                  OutputRows *rows, bool *rows_changed);
 // Before a filter bank that mixes the oscillators in: makes the rings hold n_blocks values from osc_consumed on (on
 // `stream`) and gives the rings ([n_mix][osc_ring_len]) and the slot of the first value.
 sdrgpu_status outputs_before(ChanOutputs &o, int n_blocks, cudaStream_t stream, const float2 **osc, int *osc_start);

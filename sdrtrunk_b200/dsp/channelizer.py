@@ -180,6 +180,22 @@ class ComplexPolyphaseChannelizerM2:
         native.check(native.lib().sdrgpu_chan_select(self._h, arr, len(channels), filt, n_filt))
         self._n_selected = len(channels)
 
+    def setFrequencyOffsets(self, offsets):
+        """ChannelOutputProcessor.setFrequencyOffset for running channels: `offsets` maps an index into the current
+        selection (setOutputChannels / setChannels order) to its new frequency offset in Hz.  Takes effect from the next
+        call that runs this channelizer (receiveChannels or a pipeline call); only the oscillators' angles change, as in
+        the reference, and every other channel is untouched (sdrgpu_chan_set_frequency_offsets)."""
+        items = [(int(k), int(v)) for k, v in dict(offsets).items()]
+        if not items:
+            return
+        idx = (C.c_int * len(items))(*[k for k, _ in items])
+        hz = (C.c_longlong * len(items))(*[v for _, v in items])
+        native.check(native.lib().sdrgpu_chan_set_frequency_offsets(self._h, idx, hz, len(items)))
+
+    def setFrequencyOffset(self, index, frequencyOffset):
+        """the one-channel form of setFrequencyOffsets"""
+        self.setFrequencyOffsets({index: frequencyOffset})
+
     def receiveChannels(self, samples, samples_mem=native.HOST, out=None, out_mem=native.HOST, out_stride_floats=None):
         """Returns float32 [n_selected, 2*n_blocks]: each row one channel's interleaved I/Q stream."""
         return self._process(samples, samples_mem, out, out_mem, native.LAYOUT_CHANNELS, out_stride_floats)
