@@ -54,7 +54,7 @@ inline sdrgpu_status fail(sdrgpu_status code, const char *fmt, ...)
 
 // number of output rows the channelizer currently selects (channelizer.cu)
 int chan_selected_count(const sdrgpu_channelizer *h);
-// channelizer internals the fused pipeline (bank.cu) drives directly.  chan_enqueue writes channel-layout row c to
+// channelizer internals the fused pipeline (pipeline.cu) drives directly.  chan_enqueue writes channel-layout row c to
 // d_out + c * stride, or, given a row table (a pipeline routing the rows to several banks), to rows[c] + col (floats)
 sdrgpu_status chan_enqueue(sdrgpu_channelizer *h, const float2 *d_in, int n_in, float *d_out, long long stride, int layout,
                            int *n_blocks_out, float *const *rows = nullptr, long long col = 0);

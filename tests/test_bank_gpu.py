@@ -1060,6 +1060,47 @@ def test_asynchronous_pipeline_calls_equal_the_synchronous_sequence(gpu, fmt):
     pipe2.wait()
 
 
+def test_refused_asynchronous_call_changes_nothing(gpu):
+    """A submit the channelizers would take but the bank refuses (more samples per channel than its
+    max_samples_per_call) fails with OVERFLOW before anything is staged: the staging pairs keep alternating, so the next
+    submit does not overwrite the input of the call in flight, and both calls' dibits and counts equal the synchronous
+    sequence without the refused call."""
+    from sdrtrunk_b200.dsp import Bank, ComplexPolyphaseChannelizerM2, Pipeline
+    m, n_ch = 96, 30 * 1024
+    rng = np.random.default_rng(211)
+    bins = [[3, 40], [7, 88]]
+    xs = [_tuner_stream(rng, m, n_ch, b) for b in bins]
+    taps, fir = oracle.sinc_m2_channelizer(25000.0, m, 9), c4fm_taps()
+    unit = m * 1024          # input values per assembler buffer of every channel
+    a, c, d = ([x[i * 8 * unit:(i + 1) * 8 * unit] for x in xs] for i in range(3))
+    refused = [x[:12 * unit] for x in xs]
+
+    def pipeline():
+        chans = []
+        for k in range(2):
+            ch = ComplexPolyphaseChannelizerM2(taps, 2400000, m, maxInputFloats=16 * unit)
+            ch.setChannels(bins[k])
+            chans.append(ch)
+        pipe = Pipeline(chans, Bank.preset(gpu.PRESET_P25_C4FM, 4, 50000.0, fir, max_samples_per_call=9 * 1024))
+        pipe.setDeviceChunks(2)
+        return pipe
+
+    sync = pipeline()
+    want = [sync.process(seg) for seg in (a, c, d)]
+    assert all(w.size > 100 for w in want[0])
+    pipe = pipeline()
+    pipe.submit([x.copy() for x in a])
+    with pytest.raises(gpu.OverflowError_):
+        pipe.submit(refused)
+    pipe.submit([x.copy() for x in c])
+    got = [pipe.wait(), pipe.wait()]
+    pipe.submit([x.copy() for x in d])      # the pipeline still takes calls
+    got.append(pipe.wait())
+    for i in range(3):
+        for r in range(4):
+            assert np.array_equal(got[i][r], want[i][r]), (i, r)
+
+
 def test_asynchronous_pipeline_random_call_sizes(gpu):
     """a longer stream through submit / wait with random call sizes (whole buffers, ragged, shorter than a chunk, empty),
     waits taken late or early (one or two calls in flight), 8-bit tuner samples: every call's dibits equal the synchronous
