@@ -180,7 +180,8 @@ typedef struct {
  * TwoChannelSynthesizerM2 + FS4DownConverter + the frequency-correction Oscillator (always, as
  * TwoChannelOutputProcessor.java:113 does); one-bin channels run the Oscillator only with a non-zero offset
  * (OneChannelOutputProcessor.java:92-95).  Selecting resets the oscillators and synthesizer histories: to change only
- * the frequency offsets of selected channels without that reset, use sdrgpu_chan_set_frequency_offsets. */
+ * the frequency offsets of selected channels without that reset, use sdrgpu_chan_set_frequency_offsets; to add, remove
+ * or move channels without resetting the others, use sdrgpu_chan_update_selection. */
 sdrgpu_status sdrgpu_chan_select(sdrgpu_channelizer *h, const sdrgpu_output_channel *channels, int n_channels,
                                  const float *synthesis_filter, int n_synthesis_taps);
 
@@ -197,6 +198,32 @@ sdrgpu_status sdrgpu_chan_select(sdrgpu_channelizer *h, const sdrgpu_output_chan
  * before sdrgpu_chan_set_sample_rate; a refused call changes nothing. */
 sdrgpu_status sdrgpu_chan_set_frequency_offsets(sdrgpu_channelizer *h, const int *channels, const long long *offsets_hz,
                                                 int n);
+
+/* Edits the selection of a running channelizer.  channels[i] is entry i of the new selection. previous[i] is the index
+ * in the current selection that entry i continues, or -1 for a new channel.  This is what PolyphaseChannelManager does
+ * when it adds or removes an output processor, or moves one with setPolyphaseChannelIndices: the other channels'
+ * processors carry on untouched.
+ *   - A kept entry (previous[i] >= 0) keeps its output processor's state: its oscillator phasor (also the one it holds
+ *     while its offset is 0), its look-ahead of oscillator values, and for a two-bin channel its synthesizer history,
+ *     top-block flag and FS/4 position.  It may move to other bins of the same count (one bin to one bin, two to two),
+ *     and it may change its offset, which behaves as sdrgpu_chan_set_frequency_offsets.  It must keep its gain and its
+ *     bin count: in the reference either needs a new processor (SDRGPU_ERR_INVALID_ARG).
+ *   - A new entry (-1) starts as after sdrgpu_chan_select: the oscillator at (0, -1), a two-bin channel's synthesizer
+ *     empty with the top block first.
+ *   - Every current channel that no entry continues is removed; the rows after it move up.
+ * synthesis_filter == NULL keeps the current filter.  A new filter is refused while a kept entry is a two-bin channel
+ * (it would restart them: use sdrgpu_chan_select); new two-bin entries need a filter, the current one or a new one.
+ * The edit takes effect from the first output block of the next call that runs this channelizer (sdrgpu_chan_process
+ * or any pipeline call, including the next submit); calls already enqueued keep the old selection.  The call waits for
+ * the channelizer's work in flight.  An edit that keeps the number of channels leaves a pipeline built on this
+ * channelizer usable: its rows are indexed by row and now carry the new channels.  One that changes the number gets
+ * SDRGPU_ERR_BAD_STATE at the pipeline's next call.  SDRGPU_ERR_INVALID_ARG for NULL arguments, n_channels <= 0, a bin
+ * out of range, a previous index out of range or named twice, a kept entry whose bin count or gain changed, or a
+ * filter as above; SDRGPU_ERR_BAD_STATE for a two-bin or frequency-corrected channel before
+ * sdrgpu_chan_set_sample_rate.  Every check runs before any device work; a refused call changes nothing. */
+sdrgpu_status sdrgpu_chan_update_selection(sdrgpu_channelizer *h, const sdrgpu_output_channel *channels,
+                                           const int *previous, int n_channels,
+                                           const float *synthesis_filter, int n_synthesis_taps);
 
 enum {
     SDRGPU_LAYOUT_RESULTS = 0, /* [n_blocks][2*M] floats: ReusableChannelResultsBuffer, all bins, no gain */

@@ -38,6 +38,10 @@ public class GpuPolyphaseChannelizer extends AbstractComplexPolyphaseChannelizer
     private int mMaxInputFloats;
     private int mMaxBlocks;
     private boolean mSelectionChanged = true;
+    //the processors as of the last selection (and whether each had two bins then), and the synthesis filter it carried
+    private final List<GpuChannelOutputProcessor> mSelected = new ArrayList<>();
+    private final List<Boolean> mSelectedTwoBin = new ArrayList<>();
+    private float[] mSelectedFilter;
     private final ConcurrentLinkedQueue<GpuChannelOutputProcessor> mOffsetsChanged = new ConcurrentLinkedQueue<>();
 
     /**
@@ -156,7 +160,12 @@ public class GpuPolyphaseChannelizer extends AbstractComplexPolyphaseChannelizer
         }
     }
 
-    /** sdrgpu_chan_select: one sdrgpu_output_channel per registered processor, in registration order */
+    /**
+     * One sdrgpu_output_channel per registered processor, in registration order.  sdrgpu_chan_update_selection with each
+     * processor's index in the last selection (-1 for a new one), so that processors carry on across additions, removals
+     * and setPolyphaseChannelIndices as in PolyphaseChannelManager; sdrgpu_chan_select only for the first selection and
+     * for a new synthesis filter while two-bin processors are kept, which restarts them.
+     */
     private void updateSelection() throws Throwable
     {
         List<GpuChannelOutputProcessor> processors = mProcessors;
@@ -170,7 +179,9 @@ public class GpuPolyphaseChannelizer extends AbstractComplexPolyphaseChannelizer
         try(Arena arena = Arena.ofConfined())
         {
             MemorySegment channels = arena.allocate(SdrGpu.OUTPUT_CHANNEL, n);
+            MemorySegment previous = arena.allocate(JAVA_INT, n);
             float[] synthesis = null;
+            boolean keptTwoBin = false;
 
             for(int i = 0; i < n; i++)
             {
@@ -185,10 +196,49 @@ public class GpuPolyphaseChannelizer extends AbstractComplexPolyphaseChannelizer
                 {
                     synthesis = p.getSynthesisFilter();
                 }
+
+                //a processor moved to a different bin count continues as a new channel
+                int index = mSelected.indexOf(p);
+                boolean twoBin = p.getSecondIndex() >= 0;
+
+                if(index >= 0 && mSelectedTwoBin.get(index) != twoBin)
+                {
+                    index = -1;
+                }
+
+                keptTwoBin |= index >= 0 && twoBin;
+                previous.setAtIndex(JAVA_INT, i, index);
             }
 
-            MemorySegment filter = synthesis != null ? arena.allocateFrom(JAVA_FLOAT, synthesis) : MemorySegment.NULL;
-            SdrGpu.check((int)SdrGpu.CHAN_SELECT.invokeExact(mHandle, channels, n, filter, synthesis != null ? synthesis.length : 0));
+            boolean newFilter = synthesis != null && synthesis != mSelectedFilter;
+            boolean select = mSelected.isEmpty() || (newFilter && keptTwoBin);
+            //sdrgpu_chan_select takes the filter every time, an update only when it changed (NULL keeps the current one)
+            boolean passFilter = synthesis != null && (select || newFilter);
+            MemorySegment filter = passFilter ? arena.allocateFrom(JAVA_FLOAT, synthesis) : MemorySegment.NULL;
+            int filterLength = passFilter ? synthesis.length : 0;
+
+            if(select)
+            {
+                SdrGpu.check((int)SdrGpu.CHAN_SELECT.invokeExact(mHandle, channels, n, filter, filterLength));
+            }
+            else
+            {
+                SdrGpu.check((int)SdrGpu.CHAN_UPDATE_SELECTION.invokeExact(mHandle, channels, previous, n, filter, filterLength));
+            }
+
+            mSelected.clear();
+            mSelectedTwoBin.clear();
+
+            for(GpuChannelOutputProcessor p : processors)
+            {
+                mSelected.add(p);
+                mSelectedTwoBin.add(p.getSecondIndex() >= 0);
+            }
+
+            if(synthesis != null)
+            {
+                mSelectedFilter = synthesis;
+            }
         }
 
         long outBytes = 8L * mMaxBlocks * n;
@@ -213,7 +263,7 @@ public class GpuPolyphaseChannelizer extends AbstractComplexPolyphaseChannelizer
         {
             if(mSelectionChanged)
             {
-                mOffsetsChanged.clear();   //the selection carries every processor's current offset
+                mOffsetsChanged.clear();   //the selection update carries every processor's current offset
                 updateSelection();
             }
             else

@@ -80,6 +80,10 @@ public final class SdrGpu
      *  channels, from the next process call on; only the oscillator angles change */
     static final MethodHandle CHAN_SET_FREQUENCY_OFFSETS = h("sdrgpu_chan_set_frequency_offsets",
         FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_INT));
+    /** (channelizer, sdrgpu_output_channel[] channels, int[] previous, n, float[] synthesis filter or NULL, taps): edits
+     *  the selection; previous[i] is the index in the current selection that entry i continues, -1 for a new channel */
+    static final MethodHandle CHAN_UPDATE_SELECTION = h("sdrgpu_chan_update_selection",
+        FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_INT, ADDRESS, JAVA_INT));
     static final MethodHandle CHAN_PROCESS = h("sdrgpu_chan_process",
         FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT, ADDRESS, JAVA_LONG, JAVA_INT, JAVA_INT, ADDRESS));
     static final MethodHandle CHAN_BLOCKS_FOR = h("sdrgpu_chan_blocks_for", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT));

@@ -1234,41 +1234,101 @@ sdrgpu_status sdrgpu_chan_set_sample_rate(sdrgpu_channelizer *h, double sample_r
     return SDRGPU_OK;
 }
 
-sdrgpu_status sdrgpu_chan_select(sdrgpu_channelizer *h, const sdrgpu_output_channel *channels, int n_channels,
-                                 const float *synthesis_filter, int n_synthesis_taps)
+namespace {
+
+// the bins of a selection are in range; two-bin and frequency-corrected channels need the sample rate
+sdrgpu_status check_channels(const sdrgpu_channelizer *h, const sdrgpu_output_channel *channels, int n_channels,
+                             bool *any_two)
 {
-    if (!h || !channels || n_channels <= 0) return fail(SDRGPU_ERR_INVALID_ARG, "NULL / empty selection");
-    bool any_two = false, any_special = false;
+    bool any_special = false;
+    *any_two = false;
     for (int i = 0; i < n_channels; i++) {
         if (channels[i].bin1 < 0 || channels[i].bin1 >= h->M)
             return fail(SDRGPU_ERR_INVALID_ARG, "Channel [%d] is not valid -- max channel is %d", channels[i].bin1, h->M);
         if (channels[i].bin2 >= h->M)
             return fail(SDRGPU_ERR_INVALID_ARG, "Channel [%d] is not valid -- max channel is %d", channels[i].bin2, h->M);
-        any_two |= channels[i].bin2 >= 0;
+        *any_two |= channels[i].bin2 >= 0;
         any_special |= channels[i].bin2 >= 0 || channels[i].frequency_offset_hz != 0;
     }
     if (any_special && !(h->sample_rate > 0.0))
         return fail(SDRGPU_ERR_BAD_STATE, "two-bin / frequency-corrected channels need sdrgpu_chan_set_sample_rate first");
-    if (any_two) {
-        if (!synthesis_filter || n_synthesis_taps < 2)
-            return fail(SDRGPU_ERR_INVALID_ARG, "two-bin channels need the synthesis filter (getSincM2Synthesizer)");
-        // TwoChannelSynthesizerM2.init (:74-88): tapsPerChannel = ceil(filter.length / 2) with integer division; the
-        // I/Q-duplicated filter has 2 * tapsPerChannel * 2 entries
-        const int entries = n_synthesis_taps / 2;
-        if (entries > kMaxSynthEntries)
-            return fail(SDRGPU_ERR_INVALID_ARG, "synthesis filter longer than %d taps", 2 * kMaxSynthEntries);
-        SynthFilter &synth = h->outputs.synth;
-        std::memset(&synth, 0, sizeof(synth));
-        synth.entries = entries;
-        int fp = 0;
-        for (int cp = 0; cp < n_synthesis_taps && fp + 1 < 4 * entries; cp++) {
-            synth.f[fp++] = synthesis_filter[cp];
-            synth.f[fp++] = synthesis_filter[cp];
-        }
+    return SDRGPU_OK;
+}
+
+sdrgpu_status parse_synthesis_filter(const float *synthesis_filter, int n_synthesis_taps, SynthFilter *synth)
+{
+    if (!synthesis_filter || n_synthesis_taps < 2)
+        return fail(SDRGPU_ERR_INVALID_ARG, "two-bin channels need the synthesis filter (getSincM2Synthesizer)");
+    // TwoChannelSynthesizerM2.init (:74-88): tapsPerChannel = ceil(filter.length / 2) with integer division; the
+    // I/Q-duplicated filter has 2 * tapsPerChannel * 2 entries
+    const int entries = n_synthesis_taps / 2;
+    if (entries > kMaxSynthEntries)
+        return fail(SDRGPU_ERR_INVALID_ARG, "synthesis filter longer than %d taps", 2 * kMaxSynthEntries);
+    std::memset(synth, 0, sizeof(*synth));
+    synth->entries = entries;
+    int fp = 0;
+    for (int cp = 0; cp < n_synthesis_taps && fp + 1 < 4 * entries; cp++) {
+        synth->f[fp++] = synthesis_filter[cp];
+        synth->f[fp++] = synthesis_filter[cp];
     }
+    return SDRGPU_OK;
+}
+
+}  // namespace
+
+sdrgpu_status sdrgpu_chan_select(sdrgpu_channelizer *h, const sdrgpu_output_channel *channels, int n_channels,
+                                 const float *synthesis_filter, int n_synthesis_taps)
+{
+    if (!h || !channels || n_channels <= 0) return fail(SDRGPU_ERR_INVALID_ARG, "NULL / empty selection");
+    bool any_two = false;
+    SDRGPU_TRY(check_channels(h, channels, n_channels, &any_two));
+    if (any_two) SDRGPU_TRY(parse_synthesis_filter(synthesis_filter, n_synthesis_taps, &h->outputs.synth));
     SDRGPU_CUDA(cudaStreamSynchronize(h->stream));
     h->channels.assign(channels, channels + n_channels);
     return upload_selection(h);
+}
+
+sdrgpu_status sdrgpu_chan_update_selection(sdrgpu_channelizer *h, const sdrgpu_output_channel *channels,
+                                           const int *previous, int n_channels, const float *synthesis_filter,
+                                           int n_synthesis_taps)
+{
+    if (!h || !channels || !previous || n_channels <= 0) return fail(SDRGPU_ERR_INVALID_ARG, "NULL / empty selection");
+    bool any_two = false, kept_two = false;
+    SDRGPU_TRY(check_channels(h, channels, n_channels, &any_two));
+    const int n_old = (int)h->channels.size();
+    std::vector<char> named((size_t)n_old, 0);
+    for (int i = 0; i < n_channels; i++) {
+        const int p = previous[i];
+        if (p < -1 || p >= n_old)
+            return fail(SDRGPU_ERR_INVALID_ARG, "entry %d continues channel %d of a selection of %d channels", i, p, n_old);
+        if (p < 0) continue;
+        if (named[(size_t)p]) return fail(SDRGPU_ERR_INVALID_ARG, "channel %d is continued twice", p);
+        named[(size_t)p] = 1;
+        // OneChannelOutputProcessor / TwoChannelOutputProcessor take the gain and the bin count at creation
+        const sdrgpu_output_channel &was = h->channels[(size_t)p];
+        if ((was.bin2 >= 0) != (channels[i].bin2 >= 0))
+            return fail(SDRGPU_ERR_INVALID_ARG, "entry %d changes the bin count of channel %d: make it a new channel", i, p);
+        if (was.gain != channels[i].gain)
+            return fail(SDRGPU_ERR_INVALID_ARG, "entry %d changes the gain of channel %d: make it a new channel", i, p);
+        kept_two |= was.bin2 >= 0;
+    }
+    SynthFilter synth = h->outputs.synth;
+    if (synthesis_filter) {
+        if (kept_two)
+            return fail(SDRGPU_ERR_INVALID_ARG, "a new synthesis filter restarts the two-bin channels: sdrgpu_chan_select");
+        SDRGPU_TRY(parse_synthesis_filter(synthesis_filter, n_synthesis_taps, &synth));
+    } else if (any_two && synth.entries == 0) {
+        return fail(SDRGPU_ERR_INVALID_ARG, "two-bin channels need the synthesis filter (getSincM2Synthesizer)");
+    }
+    SDRGPU_CUDA(cudaSetDevice(h->device));
+    const std::vector<sdrgpu_output_channel> next(channels, channels + n_channels);
+    OutputRows r;
+    // outputs_update waits for the calls in flight, which read the current filter, before anything changes
+    SDRGPU_TRY(outputs_update(h->outputs, h->channels, next, std::vector<int>(previous, previous + n_channels), h->M,
+                              h->sample_rate, h->stream, &r));
+    h->outputs.synth = synth;
+    h->channels = next;
+    return upload_rows(h, r);
 }
 
 sdrgpu_status sdrgpu_chan_set_frequency_offsets(sdrgpu_channelizer *h, const int *channels, const long long *offsets_hz, int n)
@@ -1298,8 +1358,9 @@ sdrgpu_status sdrgpu_chan_set_frequency_offsets(sdrgpu_channelizer *h, const int
     SDRGPU_CUDA(cudaSetDevice(h->device));
     OutputRows r;
     bool rows_changed = false;
+    SDRGPU_TRY(outputs_set_offsets(h->outputs, h->channels, next, changed, h->M, h->sample_rate, h->stream, &r,
+                                   &rows_changed));
     h->channels = next;
-    SDRGPU_TRY(outputs_set_offsets(h->outputs, h->channels, changed, h->M, h->sample_rate, h->stream, &r, &rows_changed));
     if (rows_changed) SDRGPU_TRY(upload_rows(h, r));
     return SDRGPU_OK;
 }

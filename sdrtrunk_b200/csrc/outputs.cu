@@ -212,16 +212,17 @@ __global__ void post_angle_kernel(PostChannel *chans, const __grid_constant__ Of
     chans[changes.c[i].index].angle_q = changes.c[i].angle_q;
 }
 
-// The mix set changes (a one-bin channel starts or stops mixing): one block per old mix channel m.  A kept channel's
-// live ring window (blocks start .. start + count - 1) and producer state move to its new row dst[m]; a channel that
-// stops mixing holds the phasor its next block would have used.
-__global__ void osc_carry_kernel(const MixChannel *old_chans, const float2 *old_state, const float2 *old_ring, const int *dst,
-                                 float2 *state, float2 *ring, float2 *held, int ring_len, long long start, int count)
+// The mix set changes (outputs_update): one block per old mix channel m.  A kept channel that keeps mixing moves its live
+// ring window (blocks start .. start + count - 1) and producer state to its new row to[m].x; one that stops mixing
+// (to[m].x < 0) holds, at its new selection index to[m].y, the phasor its next block would have used; a removed one
+// (both -1) is dropped.
+__global__ void osc_carry_kernel(const float2 *old_state, const float2 *old_ring, const int2 *to, float2 *state,
+                                 float2 *ring, float2 *held, int ring_len, long long start, int count)
 {
-    const int m = blockIdx.x, d = dst[m];
+    const int m = blockIdx.x, d = to[m].x;
     const float2 *src = old_ring + (size_t)m * ring_len;
     if (d < 0) {
-        if (threadIdx.x == 0) held[old_chans[m].row] = count > 0 ? src[start % ring_len] : old_state[m];
+        if (threadIdx.x == 0 && to[m].y >= 0) held[to[m].y] = count > 0 ? src[start % ring_len] : old_state[m];
         return;
     }
     for (int k = threadIdx.x; k < count; k += blockDim.x) {
@@ -229,6 +230,16 @@ __global__ void osc_carry_kernel(const MixChannel *old_chans, const float2 *old_
         ring[(size_t)d * ring_len + pos] = src[pos];
     }
     if (threadIdx.x == 0) state[d] = old_state[m];
+}
+
+// A table indexed by row follows a selection edit: entry i of the new table is entry from[i] of the old one, or `init`
+// for a new channel (from[i] < 0).  Two-bin channels' PostState (phasor, top_block, fs4, synthesizer history) and the
+// phasors d_held keeps per selected channel.
+template <class T>
+__global__ void gather_kernel(const T *src, const int *from, T *dst, int n, const __grid_constant__ T init)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) dst[i] = from[i] >= 0 ? src[from[i]] : init;
 }
 
 // grid (ceil(n / 256), n_mix): row[k] = (float)((double)(row[k] * osc[start + k]) * gain)
@@ -295,10 +306,8 @@ void release(T *&d)
     d = nullptr;
 }
 
-// the stage's buffers, once the producer is done with them; the rings restart empty
-cudaError_t free_buffers(ChanOutputs &o)
+void release_tables(ChanOutputs &o)
 {
-    const cudaError_t e = o.osc_stream ? cudaStreamSynchronize(o.osc_stream) : cudaSuccess;
     release(o.d_post);
     release(o.d_post_state);
     release(o.d_out2);
@@ -306,6 +315,13 @@ cudaError_t free_buffers(ChanOutputs &o)
     release(o.d_mix_state);
     release(o.d_osc);
     release(o.d_held);
+}
+
+// the stage's buffers, once the producer is done with them; the rings restart empty
+cudaError_t free_buffers(ChanOutputs &o)
+{
+    const cudaError_t e = o.osc_stream ? cudaStreamSynchronize(o.osc_stream) : cudaSuccess;
+    release_tables(o);
     o.osc_produced = o.osc_consumed = o.osc_safe = 0;
     o.osc_pending = false;
     return e;
@@ -405,48 +421,32 @@ sdrgpu_status launch_changes(const std::vector<OffsetChange> &list, Launch launc
     return SDRGPU_OK;
 }
 
-// The mix set changes: new tables `mix` (mix_of: each selected channel's row in them), every kept channel's ring window
-// and state carried over, the phasors of channels that stop mixing held.  The caller has waited for the work in flight.
-sdrgpu_status rebuild_mix(ChanOutputs &o, const std::vector<MixChannel> &mix, const std::vector<int> &mix_of)
+// TwoChannelOutputProcessor's state at creation
+PostState post_init()
 {
-    const int n_old = o.n_mix, n_new = (int)mix.size();
-    if (n_old == 0) o.osc_produced = o.osc_consumed;   // no ring: nothing ahead
-    const long long start = o.osc_consumed;
+    PostState st;
+    std::memset(&st, 0, sizeof(st));
+    st.cur_i = 0.0f;   // Oscillator.java:24: mCurrentAngle = new Complex(0.0f, -1.0f)
+    st.cur_q = -1.0f;
+    st.top_block = 1;  // TwoChannelSynthesizerM2: mTopBlockIndicator = true
+    return st;
+}
+
+// New angles for mix rows (a held_row starts the row from that held phasor): the look-ahead from osc_consumed on is
+// rewritten on the side stream, behind the producer in flight and the last kernel that read the rings; the next call
+// waits for it (osc_safe below osc_consumed + its blocks)
+sdrgpu_status reproduce(ChanOutputs &o, const std::vector<OffsetChange> &list)
+{
+    if (list.empty()) return SDRGPU_OK;
+    if (o.mix_recorded) SDRGPU_CUDA(cudaStreamWaitEvent(o.osc_stream, o.ev_mix, 0));
     const int count = (int)(o.osc_produced - o.osc_consumed);
-    if (n_new > 0) {
-        SDRGPU_TRY(ensure_osc_stream(o));
-        o.osc_ring_len = (2 * o.max_blocks + 8 + 1) & ~1;   // as outputs_select
-    }
-    MixChannel *d_mix = nullptr;
-    float2 *d_state = nullptr, *d_osc = nullptr;
-    if (n_new > 0) {
-        SDRGPU_TRY(upload(&d_mix, mix));
-        SDRGPU_CUDA(cudaMalloc(&d_state, sizeof(float2) * (size_t)n_new));
-        SDRGPU_CUDA(cudaMalloc(&d_osc, sizeof(float2) * (size_t)n_new * (size_t)o.osc_ring_len));
-    }
-    if (n_old > 0) {
-        std::vector<int> dst(n_old, -1);
-        for (size_t i = 0; i < o.mix_of.size(); i++)
-            if (o.mix_of[i] >= 0) dst[o.mix_of[i]] = mix_of[i];
-        int *d_dst = nullptr;
-        SDRGPU_TRY(upload(&d_dst, dst));
-        osc_carry_kernel<<<n_old, 128, 0, o.osc_stream>>>(o.d_mix, o.d_mix_state, o.d_osc, d_dst, d_state, d_osc, o.d_held,
-                                                          o.osc_ring_len, start, count);
-        count_launch();
-        const cudaError_t e = cudaGetLastError();
-        const cudaError_t s = cudaStreamSynchronize(o.osc_stream);
-        cudaFree(d_dst);
-        SDRGPU_CUDA(e);
-        SDRGPU_CUDA(s);
-    }
-    release(o.d_mix);
-    release(o.d_mix_state);
-    release(o.d_osc);
-    o.d_mix = d_mix;
-    o.d_mix_state = d_state;
-    o.d_osc = d_osc;
-    o.n_mix = n_new;
-    o.mix_of = mix_of;
+    SDRGPU_TRY(launch_changes(list, [&](const OffsetChanges &c) {
+        osc_reproduce_kernel<<<(c.n + 31) / 32, 32, 0, o.osc_stream>>>(o.d_mix, o.d_mix_state, o.d_osc, o.osc_ring_len,
+                                                                       o.osc_consumed, count, o.d_held, c);
+    }));
+    SDRGPU_CUDA(cudaEventRecord(o.ev_osc, o.osc_stream));
+    o.osc_pending = true;
+    o.osc_safe = o.osc_consumed;
     return SDRGPU_OK;
 }
 
@@ -468,15 +468,8 @@ sdrgpu_status sdrgpu::outputs_select(ChanOutputs &o, const std::vector<sdrgpu_ou
     // every channel holds the Oscillator's starting phasor until it first mixes (Oscillator.java:24)
     SDRGPU_TRY(upload(&o.d_held, std::vector<float2>(channels.size(), make_float2(0.0f, -1.0f))));
     if (!post.empty()) {
-        std::vector<PostState> init(post.size());
-        std::memset(init.data(), 0, sizeof(PostState) * init.size());
-        for (auto &st : init) {
-            st.cur_i = 0.0f;   // Oscillator.java:24: mCurrentAngle = new Complex(0.0f, -1.0f)
-            st.cur_q = -1.0f;
-            st.top_block = 1;  // TwoChannelSynthesizerM2: mTopBlockIndicator = true
-        }
         SDRGPU_TRY(upload(&o.d_post, post));
-        SDRGPU_TRY(upload(&o.d_post_state, init));
+        SDRGPU_TRY(upload(&o.d_post_state, std::vector<PostState>(post.size(), post_init())));
         SDRGPU_CUDA(cudaMalloc(&o.d_out2, sizeof(float) * 2 * (size_t)max_blocks * (size_t)n_two));
     }
     if (!mix.empty()) {
@@ -494,7 +487,108 @@ sdrgpu_status sdrgpu::outputs_select(ChanOutputs &o, const std::vector<sdrgpu_ou
     return SDRGPU_OK;
 }
 
-sdrgpu_status sdrgpu::outputs_set_offsets(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &channels,
+sdrgpu_status sdrgpu::outputs_update(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &old,
+                                     const std::vector<sdrgpu_output_channel> &channels, const std::vector<int> &previous,
+                                     int M, double sample_rate, cudaStream_t stream, OutputRows *rows)
+{
+    std::vector<PostChannel> post;
+    std::vector<MixChannel> mix;
+    std::vector<int> post_of, mix_of;
+    int n_two = 0;
+    plan_outputs(channels, M, sample_rate, rows, &post, &mix, &post_of, &mix_of, &n_two);
+    const int n = (int)channels.size(), n_old_mix = o.n_mix, n_post = (int)post.size(), n_mix = (int)mix.size();
+    // held_from / post_from: each new row's old row (-1: new); mix_to: each old mix row's new mix row and selection index
+    std::vector<int> held_from(previous), post_from(n_post, -1);
+    std::vector<int2> mix_to(n_old_mix, make_int2(-1, -1));
+    std::vector<OffsetChange> restart;   // mix rows whose look-ahead is rewritten from their phasor (osc_reproduce_kernel)
+    for (int i = 0; i < n; i++) {
+        const int p = previous[i];
+        const bool was_mixing = p >= 0 && o.mix_of[p] >= 0;
+        if (post_of[i] >= 0 && p >= 0) post_from[post_of[i]] = o.post_of[p];
+        if (was_mixing) mix_to[o.mix_of[p]] = make_int2(mix_of[i], i);
+        // a channel that starts mixing (a new one included) resumes from its held phasor; one that keeps mixing at a new
+        // offset mixes its next block with the phasor the old angle produced
+        if (mix_of[i] >= 0 && (!was_mixing || old[p].frequency_offset_hz != channels[i].frequency_offset_hz)) {
+            OffsetChange c{};
+            c.index = mix_of[i];
+            c.held_row = was_mixing ? -1 : i;
+            c.angle_i = mix[mix_of[i]].angle_i;
+            c.angle_q = mix[mix_of[i]].angle_q;
+            restart.push_back(c);
+        }
+    }
+
+    // the calls in flight read the old tables
+    SDRGPU_CUDA(cudaStreamSynchronize(stream));
+    if (o.osc_stream) SDRGPU_CUDA(cudaStreamSynchronize(o.osc_stream));
+    if (n_old_mix == 0) o.osc_produced = o.osc_consumed;   // no ring: nothing ahead
+    if (n_mix > 0) {
+        SDRGPU_TRY(ensure_osc_stream(o));
+        o.osc_ring_len = (2 * o.max_blocks + 8 + 1) & ~1;   // as outputs_select
+    }
+    // the new tables in `next`; o keeps the old ones until the carry is done
+    ChanOutputs next = o;
+    next.d_post = nullptr;
+    next.d_post_state = nullptr;
+    next.d_out2 = nullptr;
+    next.d_mix = nullptr;
+    next.d_mix_state = nullptr;
+    next.d_osc = nullptr;
+    next.d_held = nullptr;
+    int *d_held_from = nullptr, *d_post_from = nullptr;
+    int2 *d_mix_to = nullptr;
+    const auto launch_carry = [&]() -> sdrgpu_status {
+        SDRGPU_CUDA(cudaMalloc(&next.d_held, sizeof(float2) * (size_t)n));
+        SDRGPU_TRY(upload(&d_held_from, held_from));
+        gather_kernel<float2><<<(n + 127) / 128, 128, 0, stream>>>(o.d_held, d_held_from, next.d_held, n,
+                                                                    make_float2(0.0f, -1.0f));   // Oscillator.java:24
+        count_launch();
+        if (n_post > 0) {
+            SDRGPU_TRY(upload(&next.d_post, post));
+            SDRGPU_TRY(upload(&d_post_from, post_from));
+            SDRGPU_CUDA(cudaMalloc(&next.d_post_state, sizeof(PostState) * (size_t)n_post));
+            SDRGPU_CUDA(cudaMalloc(&next.d_out2, sizeof(float) * 2 * (size_t)o.max_blocks * (size_t)n_two));
+            gather_kernel<PostState><<<(n_post + 127) / 128, 128, 0, stream>>>(o.d_post_state, d_post_from,
+                                                                                next.d_post_state, n_post, post_init());
+            count_launch();
+        }
+        if (n_mix > 0) {
+            SDRGPU_TRY(upload(&next.d_mix, mix));
+            SDRGPU_CUDA(cudaMalloc(&next.d_mix_state, sizeof(float2) * (size_t)n_mix));
+            SDRGPU_CUDA(cudaMalloc(&next.d_osc, sizeof(float2) * (size_t)n_mix * (size_t)o.osc_ring_len));
+        }
+        if (n_old_mix > 0) {
+            SDRGPU_TRY(upload(&d_mix_to, mix_to));
+            osc_carry_kernel<<<n_old_mix, 128, 0, stream>>>(o.d_mix_state, o.d_osc, d_mix_to, next.d_mix_state, next.d_osc,
+                                                            next.d_held, o.osc_ring_len, o.osc_consumed,
+                                                            (int)(o.osc_produced - o.osc_consumed));
+            count_launch();
+        }
+        SDRGPU_CUDA(cudaGetLastError());
+        return SDRGPU_OK;
+    };
+    sdrgpu_status st = launch_carry();
+    if (st == SDRGPU_OK) {
+        const cudaError_t e = cudaStreamSynchronize(stream);
+        if (e != cudaSuccess) st = fail(SDRGPU_ERR_CUDA, "selection update failed: %s", cudaGetErrorString(e));
+    }
+    cudaFree(d_held_from);
+    cudaFree(d_post_from);
+    cudaFree(d_mix_to);
+    release_tables(st == SDRGPU_OK ? o : next);
+    if (st != SDRGPU_OK) return st;
+    next.n_post = n_post;
+    next.n_mix = n_mix;
+    next.post_of = post_of;
+    next.mix_of = mix_of;
+    next.osc_pending = false;
+    next.osc_safe = next.osc_produced;
+    o = next;
+    return reproduce(o, restart);
+}
+
+sdrgpu_status sdrgpu::outputs_set_offsets(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &old,
+                                          const std::vector<sdrgpu_output_channel> &channels,
                                           const std::vector<int> &changed, int M, double sample_rate, cudaStream_t stream,
                                           OutputRows *rows, bool *rows_changed)
 {
@@ -502,21 +596,13 @@ sdrgpu_status sdrgpu::outputs_set_offsets(ChanOutputs &o, const std::vector<sdrg
     bool transition = false;
     for (int i : changed)
         if (channels[i].bin2 < 0 && (o.mix_of[i] >= 0) != (channels[i].frequency_offset_hz != 0)) transition = true;
-    std::vector<char> starts(channels.size(), 0);   // one-bin channels that start mixing
     if (transition) {
-        // Rare (typically once per channel, at its first correction): the rows of the filter bank change, so the work in
-        // flight is waited for and the mix tables are rebuilt
-        SDRGPU_CUDA(cudaStreamSynchronize(stream));
-        if (o.osc_stream) SDRGPU_CUDA(cudaStreamSynchronize(o.osc_stream));
-        std::vector<PostChannel> post;
-        std::vector<MixChannel> mix;
-        std::vector<int> post_of, mix_of;
-        int n_two = 0;
-        plan_outputs(channels, M, sample_rate, rows, &post, &mix, &post_of, &mix_of, &n_two);
-        for (int i : changed)
-            if (channels[i].bin2 < 0 && o.mix_of[i] < 0 && mix_of[i] >= 0) starts[i] = 1;
-        SDRGPU_TRY(rebuild_mix(o, mix, mix_of));
+        // Rare (typically once per channel, at its first correction): the rows of the filter bank change.  This is a
+        // selection update that keeps every channel at its own index.
+        std::vector<int> same(channels.size());
+        for (size_t i = 0; i < same.size(); i++) same[i] = (int)i;
         *rows_changed = true;
+        return outputs_update(o, old, channels, same, M, sample_rate, stream, rows);
     }
     std::vector<OffsetChange> post_list, mix_list;
     for (int i : changed) {
@@ -528,7 +614,6 @@ sdrgpu_status sdrgpu::outputs_set_offsets(ChanOutputs &o, const std::vector<sdrg
             post_list.push_back(c);
         } else if (o.mix_of[i] >= 0) {
             c.index = o.mix_of[i];
-            if (starts[i]) c.held_row = i;
             mix_list.push_back(c);
         }
     }
@@ -536,20 +621,7 @@ sdrgpu_status sdrgpu::outputs_set_offsets(ChanOutputs &o, const std::vector<sdrg
     SDRGPU_TRY(launch_changes(post_list, [&](const OffsetChanges &c) {
         post_angle_kernel<<<(c.n + 127) / 128, 128, 0, stream>>>(o.d_post, c);
     }));
-    if (!mix_list.empty()) {
-        // on the side stream behind the producer in flight and the last kernel that read the rings; the next call waits
-        // for it (osc_safe below osc_consumed + its blocks)
-        if (o.mix_recorded) SDRGPU_CUDA(cudaStreamWaitEvent(o.osc_stream, o.ev_mix, 0));
-        const int count = (int)(o.osc_produced - o.osc_consumed);
-        SDRGPU_TRY(launch_changes(mix_list, [&](const OffsetChanges &c) {
-            osc_reproduce_kernel<<<(c.n + 31) / 32, 32, 0, o.osc_stream>>>(o.d_mix, o.d_mix_state, o.d_osc, o.osc_ring_len,
-                                                                           o.osc_consumed, count, o.d_held, c);
-        }));
-        SDRGPU_CUDA(cudaEventRecord(o.ev_osc, o.osc_stream));
-        o.osc_pending = true;
-        o.osc_safe = o.osc_consumed;
-    }
-    return SDRGPU_OK;
+    return reproduce(o, mix_list);
 }
 
 sdrgpu_status sdrgpu::outputs_before(ChanOutputs &o, int n_blocks, cudaStream_t stream, const float2 **osc, int *osc_start)

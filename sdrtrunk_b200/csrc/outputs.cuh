@@ -71,7 +71,7 @@ __device__ __forceinline__ float *channel_row(float *out, long long stride, floa
 
 struct ChanOutputs {
     int max_blocks = 0;             // blocks one channelizer call can produce: scratch rows and rings are sized for it
-    SynthFilter synth{};            // two-bin channels' synthesis filter (sdrgpu_chan_select)
+    SynthFilter synth{};            // two-bin channels' synthesis filter (sdrgpu_chan_select / _update_selection)
     int n_post = 0;                 // two-bin channels
     PostChannel *d_post = nullptr;
     PostState *d_post_state = nullptr;
@@ -105,14 +105,24 @@ struct OutputRows {
 // Rebuilds the stage for a selection at this sample rate and channel count; restarts every oscillator and synthesizer.
 sdrgpu_status outputs_select(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &channels, int M, double sample_rate,
                              int max_blocks, OutputRows *rows);
-// New frequency offsets for the selected channels `changed` (channels holds every channel with its new offset), from the
-// next call on; calls already enqueued keep the old ones.  Two-bin channels and one-bin channels that keep mixing change
-// their angle in stream order and keep their oscillator, synthesizer and look-ahead (osc_reproduce_kernel).  A one-bin
-// channel that starts or stops mixing changes the filter bank's rows: the stage waits for the work in flight, rebuilds
-// the mix tables and returns the new rows in *rows (*rows_changed); otherwise *rows is untouched.
-sdrgpu_status outputs_set_offsets(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &channels,
-                                  const std::vector<int> &changed, int M, double sample_rate, cudaStream_t stream,
-                                  OutputRows *rows, bool *rows_changed);
+// A new selection `channels` (the current one is `old`) whose entry i continues the channel at index previous[i] of the
+// current selection, or is a new channel (-1).  Waits for the work in flight, then builds the tables for the new
+// selection and carries every kept channel's state to its new rows: a two-bin channel's PostState, a one-bin channel's
+// held phasor, look-ahead window and producer state.  New channels start as after outputs_select; a kept channel at a
+// new offset changes only its angle, as outputs_set_offsets does.  The caller has checked that kept entries keep their
+// class (one or two bins) and gain.  Returns the filter bank's rows in *rows.
+sdrgpu_status outputs_update(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &old,
+                             const std::vector<sdrgpu_output_channel> &channels, const std::vector<int> &previous, int M,
+                             double sample_rate, cudaStream_t stream, OutputRows *rows);
+// New frequency offsets for the selected channels `changed` (old: the selection with the current offsets, channels: with
+// the new ones), from the next call on; calls already enqueued keep the old ones.  Two-bin channels and one-bin channels
+// that keep mixing change their angle in stream order and keep their oscillator, synthesizer and look-ahead
+// (osc_reproduce_kernel).  A one-bin channel that starts or stops mixing changes the filter bank's rows: that is an
+// outputs_update keeping every channel at its index, returning the new rows in *rows (*rows_changed); otherwise *rows is
+// untouched.
+sdrgpu_status outputs_set_offsets(ChanOutputs &o, const std::vector<sdrgpu_output_channel> &old,
+                                  const std::vector<sdrgpu_output_channel> &channels, const std::vector<int> &changed,
+                                  int M, double sample_rate, cudaStream_t stream, OutputRows *rows, bool *rows_changed);
 // Before a filter bank that mixes the oscillators in: makes the rings hold n_blocks values from osc_consumed on (on
 // `stream`) and gives the rings ([n_mix][osc_ring_len]) and the slot of the first value.
 sdrgpu_status outputs_before(ChanOutputs &o, int n_blocks, cudaStream_t stream, const float2 **osc, int *osc_start);

@@ -159,6 +159,32 @@ class ComplexPolyphaseChannelizerM2:
         2-element list ChannelCalculator.getChannelIndexes returns (PolyphaseChannelManager.getOutputProcessor,
         :198-222: One/TwoChannelOutputProcessor, gain = channel count).  The two-channel synthesis filter defaults to
         getSincM2Synthesizer(channelSampleRate, channelBandwidth, 2, 9) (getOutputProcessorFilter, :491-504)."""
+        arr, any_two = self._output_channels(channels)
+        filt, n_filt = None, 0
+        if any_two:
+            if synthesisFilter is None:
+                synthesisFilter = FilterFactory.getSincM2Synthesizer(self.getChannelSampleRate(),
+                                                                     self.mSampleRate / self.mChannelCount, 2,
+                                                                     self.POLYPHASE_SYNTHESIZER_TAPS_PER_CHANNEL)
+            filt, n_filt = self._synthesis_filter(synthesisFilter)
+        native.check(native.lib().sdrgpu_chan_select(self._h, arr, len(channels), filt, n_filt))
+        self._n_selected = len(channels)
+
+    def updateOutputChannels(self, channels, previous, synthesisFilter=None):
+        """Edits the running selection without resetting the channels it keeps (sdrgpu_chan_update_selection):
+        `channels` as for setOutputChannels, previous[i] the index in the current selection that entry i continues (its
+        output processor carries on, as after setPolyphaseChannelIndices / setFrequencyOffset) or -1 for a new channel.
+        Channels no entry continues are removed.  A kept entry keeps its bin count and gain.  synthesisFilter=None keeps
+        the current two-bin synthesis filter.  Takes effect from the next call that runs this channelizer."""
+        if len(previous) != len(channels):
+            raise native.IllegalArgumentException("one previous index per channel")
+        arr, _ = self._output_channels(channels)
+        prev = (C.c_int * len(channels))(*[int(p) for p in previous])
+        filt, n_filt = (None, 0) if synthesisFilter is None else self._synthesis_filter(synthesisFilter)
+        native.check(native.lib().sdrgpu_chan_update_selection(self._h, arr, prev, len(channels), filt, n_filt))
+        self._n_selected = len(channels)
+
+    def _output_channels(self, channels):
         arr = (native.OutputChannel * len(channels))()
         any_two = False
         for i, ch in enumerate(channels):
@@ -169,16 +195,11 @@ class ComplexPolyphaseChannelizerM2:
                     "Request to create an output processor for unexpected channel index size:%d" % len(indexes))
             any_two |= len(indexes) == 2
             arr[i] = native.OutputChannel(int(indexes[0]), int(indexes[1]) if len(indexes) == 2 else -1, int(offset), gain)
-        filt, n_filt = None, 0
-        if any_two:
-            if synthesisFilter is None:
-                synthesisFilter = FilterFactory.getSincM2Synthesizer(self.getChannelSampleRate(),
-                                                                     self.mSampleRate / self.mChannelCount, 2,
-                                                                     self.POLYPHASE_SYNTHESIZER_TAPS_PER_CHANNEL)
-            self._synth = native.f32(synthesisFilter)
-            filt, n_filt = self._synth.ctypes.data_as(C.POINTER(C.c_float)), self._synth.size
-        native.check(native.lib().sdrgpu_chan_select(self._h, arr, len(channels), filt, n_filt))
-        self._n_selected = len(channels)
+        return arr, any_two
+
+    def _synthesis_filter(self, synthesisFilter):
+        self._synth = native.f32(synthesisFilter)
+        return self._synth.ctypes.data_as(C.POINTER(C.c_float)), self._synth.size
 
     def setFrequencyOffsets(self, offsets):
         """ChannelOutputProcessor.setFrequencyOffset for running channels: `offsets` maps an index into the current

@@ -113,6 +113,7 @@ PROTOTYPES = {
     "sdrgpu_chan_set_sample_rate": (C.c_int, [_vp, C.c_double]),
     "sdrgpu_chan_select": (C.c_int, [_vp, C.POINTER(OutputChannel), C.c_int, _f32p, C.c_int]),
     "sdrgpu_chan_set_frequency_offsets": (C.c_int, [_vp, _i32p, C.POINTER(C.c_longlong), C.c_int]),
+    "sdrgpu_chan_update_selection": (C.c_int, [_vp, C.POINTER(OutputChannel), _i32p, C.c_int, _f32p, C.c_int]),
     "sdrgpu_chan_process": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp, C.c_longlong, C.c_int, C.c_int, _i32p]),
     "sdrgpu_chan_blocks_for": (C.c_int, [_vp, C.c_int]),
     "sdrgpu_chan_enable_timing": (C.c_int, [_vp, C.c_int]),
